@@ -17,6 +17,9 @@ on the device (`e2e_device_pipeline`); at N > 1, where N host copies of 512 MB p
 the two legs is reported as `e2e` and the other next to it (`e2e_host_frames` / `e2e_device_pipeline`).  `roofline`: the dominant kernel class (implicit-GEMM convolutions),
 algorithmic FLOPs / CUDA-event time measured in an instrumented pass after the timed region.
 `cpu_baseline`: the CPU oracle port timed on this box's host cores on a bounded sample.
+
+`--dump-outputs DIR` writes what the last step of the `value` region computed (rank 0) as float32 .npy files, so that
+two builds can be compared output for output: the same arguments give the same inputs and initial weights.
 """
 import argparse
 import json
@@ -36,6 +39,7 @@ METRIC_OF = {"CREMAD": METRIC, "KineticSound": "DGL train samples/sec (Kinetics-
              "VGGSound": "DGL train samples/sec (VGGSound shape)"}
 UNIT = "samples/s"
 TRAIN_GFLOP_PER_SAMPLE = {"CREMAD": 42.57, "KineticSound": 50.56, "VGGSound": 50.56}  # BASELINE.md §3
+DUMP_SAMPLE = 1 << 21  # elements of the ~22 M parameters / gradients that --dump-outputs writes (8 MB each)
 
 
 def measured_peaks():
@@ -294,6 +298,8 @@ def run_gpu(a):
     ms, wall_ms = timed(a.steps, e2e=False)
     say("timed region done")
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, step, model, torch)
     for _ in range(2):
         step.prefetch(spec_h, image_h, label_h)
         step.step()
@@ -376,6 +382,26 @@ def run_gpu(a):
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, step, model, torch):
+    """What the step returns to its caller after its last run: the 7 statistics of read_stats(), the three logit sets,
+    the updated parameters and their (clipped) gradients, and the BatchNorm running statistics.  Parameters and
+    gradients are concatenated in arena order (head | audio | visual) and sampled at DUMP_SAMPLE fixed, seeded
+    positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    params = torch.cat([p.detach().reshape(-1) for p in step.arena.params])
+    grads = torch.cat([p.grad.reshape(-1) for p in step.arena.params])
+    n = params.numel()
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:min(n, DUMP_SAMPLE)].sort().values
+    idx = idx.to(params.device)
+    bn = [t.reshape(-1) for m in model.modules() if isinstance(m, torch.nn.BatchNorm2d)
+          for t in (m.running_mean, m.running_var)]
+    out = {"stats": torch.tensor(step.read_stats()), "logits": step.logits, "params_sample": params[idx],
+           "grads_sample": grads[idx], "bn_running_stats": torch.cat(bn)}
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def roofline_pass(step, torch, ops, B):
@@ -461,12 +487,16 @@ def main():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-device-pipeline", action="store_true", help="skip the e2e leg with the GPU visual transform")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "gdl_b200":
+        ap.error("--dump-outputs applies to --impl gdl_b200")
     if a.impl == "cudnn_sidebar":
         run_cudnn_sidebar(a)
     elif a.impl == "reference":
-        if a.steps > 3:
-            a.steps = 3          # bounded sample: each CPU step is several seconds
         a.warmup = min(a.warmup, 1)
         run_reference(a)
     else:

@@ -3,9 +3,9 @@ bit-exact"; SURVEY.md §8d).  The reference's dataset classes (dataset/CramedDat
 dataset/KSDataset.py:136-201) are run UNMODIFIED with only their file I/O mocked by the seeded stand-ins of
 gdl_b200.synthetic (librosa.load -> synth_wave, librosa.stft -> stft, Image.open -> synth_image); under the same
 torch / numpy / python seeds the synthetic classes must return bit-identical spectrograms and image tensors
-(crop offsets, flips, audio offsets) and leave all three RNGs in the same state.  Where /root/reference is absent
-(the GPU box) the same outputs are compared with the committed digests tests/golden/sampling_golden.json
-(written by this file when run with GDL_WRITE_GOLDEN=1 here)."""
+(crop offsets, flips, audio offsets) and leave all three RNGs in the same state.  The outputs are always compared
+with the digests of the reference's outputs committed as tests/golden/sampling_golden.json.  With GDL_REFERENCE_DIR
+naming a checkout of the reference, its classes are also run live, and GDL_WRITE_GOLDEN=1 rewrites the digests."""
 import argparse
 import hashlib
 import json
@@ -18,7 +18,7 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("GDL_REFERENCE_DIR")
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "sampling_golden.json")
 IDXS = [0, 3, 7, 12]
 
@@ -125,7 +125,7 @@ def test_sampling_matches_reference_bit_exact(kind, mode, tmp_path):
     syn, syn_rng = _run(_synthetic(kind, mode), seed=1234)
     digests = [_digest(*s) for s in syn]
     key = "%s/%s" % (kind, mode)
-    if os.path.isdir(REF):
+    if REF:
         ref, ref_rng = _run(_reference(kind, mode, tmp_path), seed=1234)
         for (s0, i0, l0), (s1, i1, l1) in zip(syn, ref):
             assert np.array_equal(np.asarray(s0), np.asarray(s1)), "spectrogram / audio crop offset differs"
