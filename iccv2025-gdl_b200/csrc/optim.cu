@@ -1,9 +1,9 @@
-// optim.cu — gradient clipping statistics, DGL gradient diagnostics and SGD-momentum over
+// optim.cu — gradient clipping statistics, DGL gradient diagnostics and the parameter updates over
 // the flat fp32 parameter arena (reference main_dgl.py:129 clip_grad_norm_(40, L2),
-// :132-143 sum_p mean|grad_p| per encoder, :154/:249 torch.optim.SGD(momentum, weight_decay)).
-// One pass over the gradients produces the global L2 norm and both diagnostics; the clip
-// coefficient stays on the device and is folded into the SGD kernel, which also writes the
-// clipped gradient back (clip_grad_norm_ is in-place in the reference).
+// :132-143 sum_p mean|grad_p| per encoder, :154/:249-256 torch.optim.SGD(momentum, weight_decay),
+// Adagrad and Adam).  One pass over the gradients produces the global L2 norm and both diagnostics;
+// the clip coefficient stays on the device and is folded into the update kernel, which also writes
+// the clipped gradient back (clip_grad_norm_ is in-place in the reference).
 #include "common.cuh"
 #include "api_version.h"
 
@@ -142,6 +142,110 @@ __global__ void __launch_bounds__(256) sgd_momentum_kernel(float* __restrict__ p
   }
 }
 
+// ---- Adam / Adagrad (torch.optim.Adam / Adagrad, non-capturable single-tensor and foreach formulas) ----
+// The update runs inside a CUDA graph captured once per lr, so the step count cannot be a kernel argument: it lives
+// in step_state[0] on the device.  One thread advances it and writes the step's scalars into step_state[1..2]
+// before the element kernel reads them (stream order), so every block of the element kernel sees the same step.
+enum { kRuleAdam = 0, kRuleAdagrad = 1 };
+
+__global__ void optim_step_prologue_kernel(int32_t* __restrict__ step_state, int rule, double lr, double a,
+                                           double b) {
+  pdl_enter();
+  const int32_t step = step_state[0] + 1;
+  step_state[0] = step;
+  float* f = reinterpret_cast<float*>(step_state + 1);
+  const double s = (double)step;  // torch: the step is a Python float here
+  if (rule == kRuleAdam) {        // a = beta1, b = beta2
+    const double bc1 = 1.0 - pow(a, s), bc2 = 1.0 - pow(b, s);
+    f[0] = (float)(lr / bc1);  // step_size, cast where addcdiv_(value=-step_size) casts it
+    f[1] = (float)sqrt(bc2);   // bias_correction2_sqrt, cast where the tensor division casts it
+  } else {                     // a = lr_decay
+    f[0] = (float)(lr / (1.0 + (s - 1.0) * a));  // clr
+  }
+}
+
+__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, float* __restrict__ grad,
+                                                   float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq,
+                                                   int64_t n4, int64_t numel, float w1, float beta2, float w2,
+                                                   float eps, float wd, const float* __restrict__ stats,
+                                                   const int32_t* __restrict__ step_state) {
+  pdl_enter();
+  const float coef = stats ? stats[1] : 1.f;
+  const float* sc = reinterpret_cast<const float*>(step_state + 1);
+  const float step_size = sc[0], bc2s = sc[1];
+  // m = lerp(m, g, w1) (torch's small-weight branch), v = beta2*v + w2*g*g, p -= step_size * m / (sqrt(v)/bc2s + eps)
+  auto upd = [&](float& p, float& g, float& m, float& v) {
+    const float gc = g * coef;
+    g = gc;
+    const float d = fmaf(wd, p, gc);
+    m = fmaf(w1, d - m, m);
+    v = fmaf(w2, d * d, v * beta2);
+    const float denom = sqrtf(v) / bc2s + eps;
+    p = fmaf(-step_size, m / denom, p);
+  };
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    float4 p = reinterpret_cast<float4*>(param)[i];
+    float4 g = reinterpret_cast<float4*>(grad)[i];
+    float4 m = reinterpret_cast<float4*>(exp_avg)[i];
+    float4 v = reinterpret_cast<float4*>(exp_avg_sq)[i];
+    upd(p.x, g.x, m.x, v.x);
+    upd(p.y, g.y, m.y, v.y);
+    upd(p.z, g.z, m.z, v.z);
+    upd(p.w, g.w, m.w, v.w);
+    reinterpret_cast<float4*>(param)[i] = p;
+    reinterpret_cast<float4*>(grad)[i] = g;
+    reinterpret_cast<float4*>(exp_avg)[i] = m;
+    reinterpret_cast<float4*>(exp_avg_sq)[i] = v;
+  }
+  // tail (numel not a multiple of 4)
+  if (blockIdx.x == 0 && threadIdx.x < (numel & 3)) {
+    int64_t i = n4 * 4 + threadIdx.x;
+    upd(param[i], grad[i], exp_avg[i], exp_avg_sq[i]);
+  }
+}
+
+__global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ param, float* __restrict__ grad,
+                                                      float* __restrict__ sum, int64_t n4, int64_t numel, float eps,
+                                                      float wd, const float* __restrict__ stats,
+                                                      const int32_t* __restrict__ step_state) {
+  pdl_enter();
+  const float coef = stats ? stats[1] : 1.f;
+  const float clr = reinterpret_cast<const float*>(step_state + 1)[0];
+  // s += g*g, p -= clr * g / (sqrt(s) + eps)
+  auto upd = [&](float& p, float& g, float& s) {
+    const float gc = g * coef;
+    g = gc;
+    const float d = fmaf(wd, p, gc);
+    s = fmaf(d, d, s);
+    p = fmaf(-clr, d / (sqrtf(s) + eps), p);
+  };
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    float4 p = reinterpret_cast<float4*>(param)[i];
+    float4 g = reinterpret_cast<float4*>(grad)[i];
+    float4 s = reinterpret_cast<float4*>(sum)[i];
+    upd(p.x, g.x, s.x);
+    upd(p.y, g.y, s.y);
+    upd(p.z, g.z, s.z);
+    upd(p.w, g.w, s.w);
+    reinterpret_cast<float4*>(param)[i] = p;
+    reinterpret_cast<float4*>(grad)[i] = g;
+    reinterpret_cast<float4*>(sum)[i] = s;
+  }
+  if (blockIdx.x == 0 && threadIdx.x < (numel & 3)) {
+    int64_t i = n4 * 4 + threadIdx.x;
+    upd(param[i], grad[i], sum[i]);
+  }
+}
+
+static unsigned elementwise_blocks(int64_t numel) {
+  int64_t n4 = numel / 4;
+  int64_t blocks = ceil_div64(n4 > 0 ? n4 : 1, 256);
+  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
+  return (unsigned)blocks;
+}
+
 static char g_last_error[512] = "";
 
 void set_last_error(const char* msg) { snprintf(g_last_error, sizeof(g_last_error), "%s", msg); }
@@ -196,11 +300,37 @@ extern "C" int gdl_sgd_momentum(float* param, float* grad, float* momentum_buf, 
   GDL_REQUIRE(param && grad && momentum_buf && numel > 0, "gdl_sgd_momentum: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)momentum_buf) & 15) == 0,
               "gdl_sgd_momentum: arenas must be 16-byte aligned");
-  int64_t n4 = numel / 4;
-  int64_t blocks = ceil_div64(n4 > 0 ? n4 : 1, 256);
-  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-  launch_pdl(sgd_momentum_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)s, param, grad, momentum_buf, n4, numel,
-                                                                    lr, mu, wd, first_step, stats);
+  launch_pdl(sgd_momentum_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, momentum_buf,
+             numel / 4, numel, lr, mu, wd, first_step, stats);
   GDL_CHECK_LAUNCH("sgd_momentum_kernel");
+  return GDL_OK;
+}
+
+extern "C" int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
+                        int64_t numel, double lr, double beta1, double beta2, double eps, double wd,
+                        const float* stats, gdl_stream_t s) {
+  GDL_REQUIRE(param && grad && exp_avg && exp_avg_sq && step_state && numel > 0, "gdl_adam: bad arguments");
+  GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
+              "gdl_adam: arenas must be 16-byte aligned");
+  GDL_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0, "gdl_adam: betas must lie in [0, 1)");
+  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdam, lr, beta1, beta2);
+  GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
+  launch_pdl(adam_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, exp_avg, exp_avg_sq,
+             numel / 4, numel, (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)eps, (float)wd,
+             stats, (const int32_t*)step_state);
+  GDL_CHECK_LAUNCH("adam_kernel");
+  return GDL_OK;
+}
+
+extern "C" int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
+                           double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s) {
+  GDL_REQUIRE(param && grad && sum && step_state && numel > 0, "gdl_adagrad: bad arguments");
+  GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)sum) & 15) == 0,
+              "gdl_adagrad: arenas must be 16-byte aligned");
+  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdagrad, lr, lr_decay, 0.0);
+  GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
+  launch_pdl(adagrad_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, sum, numel / 4, numel,
+             (float)eps, (float)wd, stats, (const int32_t*)step_state);
+  GDL_CHECK_LAUNCH("adagrad_kernel");
   return GDL_OK;
 }

@@ -32,6 +32,7 @@ _p = C.c_void_p
 _i = C.c_int
 _l = C.c_int64
 _f = C.c_float
+_d = C.c_double
 _dp = C.POINTER(ConvDesc)
 
 # name -> (restype, argtypes); every symbol of include/gdl_b200.h
@@ -99,6 +100,8 @@ SIGNATURES = {
     "gdl_optim_scratch_floats": (_l, [_l, _i]),
     "gdl_grad_stats": (_i, [_p, _l, _p, _p, _p, _i, _f, _p, _p, _p]),
     "gdl_sgd_momentum": (_i, [_p, _p, _p, _l, _f, _f, _f, _i, _p, _p]),
+    "gdl_adam": (_i, [_p, _p, _p, _p, _p, _l, _d, _d, _d, _d, _d, _p, _p]),
+    "gdl_adagrad": (_i, [_p, _p, _p, _p, _l, _d, _d, _d, _d, _p, _p]),
     "gdl_check_conv_fwd": (_i, [_dp, _i, _p, _p, _p, _p]),
     "gdl_check_conv_dgrad": (_i, [_dp, _i, _p, _p, _p, _p, _p]),
     "gdl_check_conv_wgrad": (_i, [_dp, _i, _p, _p, _p, _p]),

@@ -497,6 +497,19 @@ def sgd_momentum(param, grad, buf, numel, lr, mu, wd, first_step, stats):
                                        int(first_step), _ptr(stats), _stream()), "gdl_sgd_momentum")
 
 
+# Adam / Adagrad: step_state is the int32 [3] device counter of include/gdl_b200.h (one launch advances it, one updates)
+@_op("adam", 2, lambda param, grad, m, v, step_state, numel, *a: ("bytes", 32.0 * numel))
+def adam(param, grad, exp_avg, exp_avg_sq, step_state, numel, lr, beta1, beta2, eps, wd, stats):
+    check(_lib.load().gdl_adam(_ptr(param), _ptr(grad), _ptr(exp_avg), _ptr(exp_avg_sq), _ptr(step_state), numel,
+                               lr, beta1, beta2, eps, wd, _ptr(stats), _stream()), "gdl_adam")
+
+
+@_op("adagrad", 2, lambda param, grad, s, step_state, numel, *a: ("bytes", 24.0 * numel))
+def adagrad(param, grad, state_sum, step_state, numel, lr, lr_decay, eps, wd, stats):
+    check(_lib.load().gdl_adagrad(_ptr(param), _ptr(grad), _ptr(state_sum), _ptr(step_state), numel, lr, lr_decay,
+                                  eps, wd, _ptr(stats), _stream()), "gdl_adagrad")
+
+
 # ---------------------------------------------------------------------------------- data pipeline
 @_op("crop_resize_normalize", 2,
      lambda store, n, Hs, Ws, params, frames, T, S, mean, std, out, table: ("bytes", frames * 3.0 * S * S * 4.0))

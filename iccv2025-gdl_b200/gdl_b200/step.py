@@ -3,7 +3,8 @@
 One call = reference main_dgl.py:93-158 for one batch: H2D of (spec, image, label), both
 ResNet-18 encoders forward, global average pooling, the fused DGL head (three logit sets,
 three cross-entropies, truncated gradients), both encoder backwards, [gradient all-reduce],
-clip_grad_norm_(40), the audio/visual gradient diagnostics, SGD-momentum, and the refresh of
+clip_grad_norm_(40), the audio/visual gradient diagnostics, the optimizer update (SGD-momentum, Adam or Adagrad:
+gdl_b200.optim.UpdateRule), and the refresh of
 the bf16 weight shadows — as a fixed sequence of libgdl_b200.so kernels on two CUDA streams
 (audio || visual), optionally captured into one CUDA graph.  The only device->host traffic is
 one 7-float read (3 losses + norm, clip coefficient, 2 diagnostics) when the caller asks.
@@ -23,6 +24,7 @@ from . import ops, parallel
 from .autograd import to_nhwc8  # noqa: F401  (re-export for callers)
 from .basic_model import AVClassifier_DGL
 from .fusion_modules import ConcatFusion_DGL, FiLM_DGL, GatedFusion_DGL, SumFusion_DGL
+from .optim import UpdateRule
 
 _SEG_ALIGN = 64  # floats; keeps every tensor 256-byte aligned inside the arenas
 
@@ -55,11 +57,13 @@ def head_trainable(fm):
 
 
 class ParamArena:
-    """Flat fp32 arenas (parameters, gradients, momentum) with the nn.Parameters re-pointed to
-    views, so clipping statistics, SGD and the gradient all-reduce are single passes.
-    Order: head | audio_net | visual_net  (groups 2, 0, 1 for the diagnostics)."""
+    """Flat fp32 arenas (parameters, gradients, optimizer state) with the nn.Parameters re-pointed to
+    views, so clipping statistics, the update and the gradient all-reduce are single passes.
+    Order: head | audio_net | visual_net  (groups 2, 0, 1 for the diagnostics).
+    The optimizer state is that of `rule.kind` only (default SGD): `momentum`; Adam `exp_avg`, `exp_avg_sq`;
+    Adagrad `sum`.  `state_buffers` pairs each with its key in torch's `optimizer.state[p]`."""
 
-    def __init__(self, model, device):
+    def __init__(self, model, device, rule=None):
         groups = [(2, head_trainable(model.fusion_module)),
                   (0, list(model.audio_net.parameters())),
                   (1, list(model.visual_net.parameters()))]
@@ -81,7 +85,24 @@ class ParamArena:
         self.extra = 64  # tail slots all-reduced together with the gradients (3 losses)
         self.param = torch.zeros(off, device=device)
         self.grad = torch.zeros(off + self.extra, device=device)
-        self.momentum = torch.zeros(off, device=device)
+        self.kind = rule.kind if rule is not None else "sgd"
+        if self.kind == "sgd":
+            self.momentum = torch.zeros(off, device=device)
+            self.state_buffers = [("momentum_buffer", self.momentum)]
+        elif self.kind == "adam":
+            self.exp_avg = torch.zeros(off, device=device)
+            self.exp_avg_sq = torch.zeros(off, device=device)
+            self.state_buffers = [("exp_avg", self.exp_avg), ("exp_avg_sq", self.exp_avg_sq)]
+        else:
+            self.sum = torch.full((off,), rule.initial_accumulator_value, device=device)
+            self.state_buffers = [("sum", self.sum)]
+        # Adam / Adagrad step count t (torch's state['step']): one count for the whole arena, so every DGLStep on it
+        # (an epoch's short tail batch has its own) continues it.  step_state[0] is the copy the update kernels advance
+        # on the device (also under CUDA-graph replay), `steps` the host's, advanced by DGLStep.step; `step_tensors`
+        # are the CPU tensors train.adopt_momentum put into optimizer.state[p]['step'], refreshed by sync_step_tensors.
+        self.step_state = torch.zeros(3, device=device, dtype=torch.int32)
+        self.steps = 0
+        self.step_tensors = {}
         for p, o in zip(self.params, self.offsets):
             n = p.numel()
             self.param[o:o + n].copy_(p.data.reshape(-1))
@@ -104,6 +125,16 @@ class ParamArena:
         base = self.param.data_ptr()
         return all(p is q and p.data.data_ptr() == base + 4 * o for p, q, o in zip(groups, self.params, self.offsets))
 
+    def set_steps(self, t):
+        """Continue from step count t (a restored checkpoint)."""
+        self.steps = int(t)
+        self.step_state[0] = self.steps
+
+    def sync_step_tensors(self):
+        """Write the step count into the optimizer's state['step'] tensors, so optimizer.state_dict() carries it."""
+        for t in self.step_tensors.values():
+            t.fill_(float(self.steps))
+
     def late_split(self, gid, late_params):
         """Offset where the `late_params` of group gid start, checked to be exactly the tail of the group
         (module registration order: conv1, bn1, layer1 .. layer4)."""
@@ -117,9 +148,12 @@ class ParamArena:
 
 class DGLStep:
     def __init__(self, model, batch_size, spec_hw, image_thw, alpha=4.0, lr=0.001, momentum=0.9,
-                 weight_decay=1e-4, max_norm=40.0, world_size=1, process_group=None, use_graph=True, check_fp32=None):
+                 weight_decay=1e-4, max_norm=40.0, world_size=1, process_group=None, use_graph=True, check_fp32=None,
+                 rule=None):
         """model: AVClassifier_DGL on a CUDA device (possibly wrapped: `.module` is unwrapped).
         batch_size: LOCAL batch on this GPU; losses are means over batch_size*world_size.
+        rule: the update (gdl_b200.optim.UpdateRule, e.g. update_rule(torch_optimizer)); its lr, weight decay and
+        momentum replace the three arguments of the same names.  Default: SGD with lr, momentum, weight_decay.
         check_fp32 (default: env GDL_CHECK_FP32): the FP32 check mode — the encoders store fp32 activations and run
         the CUDA-core fp64-accumulating kernels of csrc/check_fp32.cu (gdl_b200/check.py) instead of the bf16
         tcgen05 engine; head, truncation, clipping, SGD and the all-reduce are the product code.  For parity
@@ -136,7 +170,10 @@ class DGLStep:
         self.B = batch_size
         self.F_, self.Tt = spec_hw
         self.T, self.H, self.W = image_thw
-        self.alpha, self.lr, self.mu, self.wd, self.max_norm = alpha, lr, momentum, weight_decay, max_norm
+        if rule is None:
+            rule = UpdateRule("sgd", lr, weight_decay, momentum=momentum)
+        self.rule = rule
+        self.alpha, self.lr, self.mu, self.wd, self.max_norm = alpha, rule.lr, rule.momentum, rule.weight_decay, max_norm
         self.world_size, self.pg = world_size, process_group
         self.inv_batch = 1.0 / (batch_size * world_size)
         self.n = model.n_classes
@@ -144,10 +181,10 @@ class DGLStep:
         B, T = self.B, self.T
 
         # ONE arena per model: a second DGLStep of another batch geometry (an epoch's short tail batch) shares the
-        # parameters, gradients and momentum of the first instead of re-allocating and copying them
+        # parameters, gradients and optimizer state of the first instead of re-allocating and copying them
         arena = getattr(model, "_gdl_arena", None)
-        if arena is None or not arena.owns(model, dev):
-            arena = ParamArena(model, dev)
+        if arena is None or not arena.owns(model, dev) or arena.kind != rule.kind:
+            arena = ParamArena(model, dev, rule)
             model._gdl_arena = arena
         self.arena = arena
         if check_fp32 is None:
@@ -348,12 +385,19 @@ class DGLStep:
         parallel.allreduce_finish(works, self._buckets["early"], self.pg)
 
     def _enqueue_update(self, lr, first):
-        """Clip statistics + diagnostics + SGD + bf16 shadow refresh (after the all-reduce)."""
-        ar = self.arena
+        """Clip statistics + diagnostics + optimizer update + bf16 shadow refresh (after the all-reduce)."""
+        ar, r = self.arena, self.rule
         ops.grad_stats(ar.grad, ar.numel, ar.seg_end, ar.seg_group, ar.seg_inv, ar.nseg, self.max_norm,
                        ar.scratch, self.stats[4:8])
-        ops.sgd_momentum(ar.param, ar.grad, ar.momentum, ar.numel, lr, self.mu, self.wd,
-                         first and not self.momentum_loaded, self.stats[4:8])
+        if r.kind == "sgd":
+            ops.sgd_momentum(ar.param, ar.grad, ar.momentum, ar.numel, lr, self.mu, self.wd,
+                             first and not self.momentum_loaded, self.stats[4:8])
+        elif r.kind == "adam":
+            ops.adam(ar.param, ar.grad, ar.exp_avg, ar.exp_avg_sq, ar.step_state, ar.numel, lr, r.betas[0], r.betas[1],
+                     r.eps, self.wd, self.stats[4:8])
+        else:
+            ops.adagrad(ar.param, ar.grad, ar.sum, ar.step_state, ar.numel, lr, r.lr_decay, r.eps, self.wd,
+                        self.stats[4:8])
         self.enc_a.repack()
         self.enc_v.repack()
         if self.film is not None:
@@ -460,6 +504,7 @@ class DGLStep:
                 self._allreduce()
                 self._graph_update.replay()
         self.steps_done += 1
+        self.arena.steps += 1
         return self.stats
 
     def read_stats(self):

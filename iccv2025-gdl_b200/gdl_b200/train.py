@@ -4,14 +4,16 @@ the same signatures, return values, prints and CSV side effects, running on the 
 Differences that are invisible to the caller: the 123 per-step host syncs of the reference
 (120 `.item()` for the diagnostics + 3 losses) become one 8-float D2H per LOG_EVERY steps
 (the per-step values are kept in a device ring and flushed in order), and the optimizer passed
-in is only read for its hyper-parameters / lr schedule — the update itself is the fused
-SGD-momentum kernel over the parameter arena (its momentum is exposed through
-`optimizer.state[p]['momentum_buffer']` so reference-format checkpoints still carry it).
+in is only read for its update rule, hyper-parameters and lr schedule (gdl_b200.optim.update_rule: SGD-momentum,
+Adam or Adagrad; anything else raises) — the update itself is a fused kernel over the parameter arena (its state is
+exposed through `optimizer.state[p]` — `momentum_buffer`, `exp_avg` / `exp_avg_sq` / `step`, `sum` / `step` — so
+reference-format checkpoints still carry it).
 """
 import csv
 
 import torch
 
+from .optim import update_rule
 from .step import DGLStep
 
 LOG_EVERY = 100  # the reference prints every 100 steps (main_dgl.py:125,144)
@@ -50,12 +52,11 @@ def _get_step(args, model, optimizer, spec, image, pipeline=None, audio_pipeline
             st.momentum_loaded = True  # the momentum arena is live: never torch's first-step `buf = g` again
         inner._gdl_step, inner._gdl_step_key = st, key
         return st
-    g = optimizer.param_groups[0]
+    rule = update_rule(optimizer)
     world = torch.distributed.get_world_size() if torch.distributed.is_available() and \
         torch.distributed.is_initialized() else 1
     trained = any(s.steps_done > 0 for s in steps.values())
-    st = DGLStep(inner, B, spec_hw, thw, alpha=args.alpha, lr=g['lr'],
-                 momentum=g.get('momentum', 0.9), weight_decay=g.get('weight_decay', 1e-4), max_norm=40.0,
+    st = DGLStep(inner, B, spec_hw, thw, alpha=args.alpha, rule=rule, max_norm=40.0,
                  world_size=world, process_group=torch.distributed.group.WORLD if world > 1 else None)
     adopt_momentum(st.arena, optimizer, st)
     if trained:
@@ -69,19 +70,38 @@ def _get_step(args, model, optimizer, spec, image, pipeline=None, audio_pipeline
 
 def adopt_momentum(arena, optimizer, step=None):
     """Checkpoint compatibility in both directions (reference main_dgl.py:396-412 saves `optimizer.state_dict()`):
-    momentum buffers already present in `optimizer.state` — loaded from a checkpoint by
-    `optimizer.load_state_dict`, or left by a previous DGLStep of another batch geometry — are copied INTO the
-    arena, then `optimizer.state[p]['momentum_buffer']` is re-pointed at the arena views so the next
-    `optimizer.state_dict()` carries what the fused SGD kernel maintains.  When anything was adopted the
-    step's first update must use `mu * buf + g` instead of torch's first-step `buf = g`."""
-    loaded = False
+    optimizer state already present in `optimizer.state` — loaded from a checkpoint by `optimizer.load_state_dict`,
+    created by torch's Adagrad at construction (`sum` = initial_accumulator_value), or left by a previous DGLStep of
+    another batch geometry — is copied INTO the arena buffers of the rule in use (SGD `momentum_buffer`, Adam
+    `exp_avg` / `exp_avg_sq`, Adagrad `sum`), then `optimizer.state[p]` is re-pointed at the arena views so the next
+    `optimizer.state_dict()` carries what the fused kernels maintain.  Returns whether anything was copied.
+    SGD: when anything was adopted the step's first update must use `mu * buf + g` instead of torch's first-step
+    `buf = g`.
+    Adam / Adagrad: a `state['step']` the arena did not put there sets the arena's step count, which must then be
+    the same for every arena parameter (ValueError otherwise; a parameter without state counts 0).  It is replaced by
+    a CPU float tensor of the arena's, which `ParamArena.sync_step_tensors` (end of train_epoch) keeps current.
+    Parameters outside the arena (never trained, e.g. concat's fc_auxi) keep whatever state torch gave them."""
+    loaded, counts = False, set()
     for p, o in zip(arena.params, arena.offsets):
-        view = arena.momentum[o:o + p.numel()].view(p.shape)
-        buf = optimizer.state.get(p, {}).get('momentum_buffer')
-        if buf is not None and buf.data_ptr() != view.data_ptr():
-            view.copy_(buf)
-            loaded = True
-        optimizer.state[p]['momentum_buffer'] = view
+        state = optimizer.state[p]
+        for key, buf in arena.state_buffers:
+            view = buf[o:o + p.numel()].view(p.shape)
+            old = state.get(key)
+            if old is not None and old.data_ptr() != view.data_ptr():
+                view.copy_(old)
+                loaded = True
+            state[key] = view
+        if arena.kind != "sgd":
+            t, own = state.get('step'), arena.step_tensors.get(id(p))
+            if own is None or t is not own:
+                counts.add(0 if t is None else int(t))
+    if len(counts) > 1:
+        raise ValueError("optimizer state holds different step counts {} for the parameters of one update; the fused "
+                         "{} step keeps one count for all of them".format(sorted(counts), arena.kind))
+    if counts:
+        arena.set_steps(counts.pop())
+        for p in arena.params:
+            arena.step_tensors[id(p)] = optimizer.state[p]['step'] = torch.tensor(float(arena.steps))
     if loaded and step is not None:
         step.momentum_loaded = True
     return loaded
@@ -151,6 +171,8 @@ def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, wr
         if len(pending) == LOG_EVERY:
             flush()
     flush()
+    if st is not None:
+        st.arena.sync_step_tensors()  # optimizer.state[p]['step'] for the checkpoint main_dgl.py writes next
     n = max(len(dataloader), 1) if hasattr(dataloader, "__len__") else max(nsteps, 1)
     return totals[0] / n, totals[1] / n, totals[2] / n, 0.0, 0.0, 0.0, 0.0
 

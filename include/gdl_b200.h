@@ -354,6 +354,21 @@ int gdl_grad_stats(const float* grad, int64_t numel, const int64_t* seg_end,
  * p -= lr*buf.  coef is read from stats[1] on the device (may be NULL => 1). */
 int gdl_sgd_momentum(float* param, float* grad, float* momentum_buf, int64_t numel, float lr,
                      float mu, float wd, int first_step, const float* stats, gdl_stream_t s);
+/* Adam and Adagrad (torch.optim.Adam / Adagrad semantics, main_dgl.py:251-256; no amsgrad, maximize or decoupled
+ * weight decay).  step_state int32 [3], device memory owned by the caller: [0] is the step count t (0 before the
+ * first update, torch's state['step']), [1..2] scratch.  Each call launches a one-thread kernel that advances
+ * t by one and derives the step's scalars from it in double precision, then the element kernel, so the count
+ * advances on every replay of a captured graph and lr is the only host-side argument that changes the result.
+ * Adam (32 bytes per element):
+ *   g = grad*coef (written back); g += wd*p; m = lerp(m, g, 1-beta1); v = beta2*v + (1-beta2)*g*g;
+ *   p -= (lr/(1-beta1^t)) * m / (sqrt(v)/sqrt(1-beta2^t) + eps).
+ * Adagrad (24 bytes per element):
+ *   g = grad*coef (written back); g += wd*p; s += g*g; p -= lr/(1+(t-1)*lr_decay) * g / (sqrt(s) + eps).
+ * coef is read from stats[1] on the device (may be NULL => 1).  All arenas 16-byte aligned. */
+int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state, int64_t numel,
+             double lr, double beta1, double beta2, double eps, double wd, const float* stats, gdl_stream_t s);
+int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
+                double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s);
 
 /* ---- visual data pipeline (reference dataset/CramedDataset.py:76-89,96-101; KSDataset.py:160-173,183-190) ---
  * RandomResizedCrop(S) | Resize((S,S)) -> RandomHorizontalFlip -> ToTensor -> Normalize for `frames` frames,

@@ -1,8 +1,7 @@
 #!/usr/bin/env python
 """CLI-compatible entry point for the reference's main_dgl.py (same flags, same defaults,
 same prints / csv / checkpoint file names, same evaluation-mode checkpoint loading), running the B200-native DGL step.
-Deviations: --optimizer AdaGrad / Adam raise NotImplementedError (the fused update is SGD-momentum, the reference
-default); no TensorBoard branch; `--resume` and `--synthetic_len` are additions.
+Deviations: no TensorBoard branch; `--resume` and `--synthetic_len` are additions.
 
     python main_dgl.py --train --ckpt_path ckpt --dataset CREMAD --fusion_method concat \
         --fps 3 --alpha 4 --batch_size 64 --audio_path synthetic
@@ -96,11 +95,10 @@ def main(argv=None):
 
     if args.optimizer == 'sgd':
         optimizer = optim.SGD(model.parameters(), lr=args.learning_rate, momentum=0.9, weight_decay=1e-4)
-    elif args.optimizer in ('AdaGrad', 'Adam'):
-        # accepted by the reference (main_dgl.py:251-256); every shipped script uses sgd and the fused update
-        # kernel implements SGD-momentum only
-        raise NotImplementedError('optimizer {}: the B200 DGL step implements the reference default (sgd) only'
-                                  .format(args.optimizer))
+    elif args.optimizer == 'AdaGrad':  # reference main_dgl.py:251-256 (OGM-GE lineage arguments)
+        optimizer = optim.Adagrad(model.parameters(), lr=args.learning_rate)
+    elif args.optimizer == 'Adam':
+        optimizer = optim.Adam(model.parameters(), lr=args.learning_rate, betas=(0.9, 0.999), eps=1e-08)
     else:
         raise ValueError('Incorrect optimizer: {}'.format(args.optimizer))  # reference main_dgl.py:259
     scheduler = optim.lr_scheduler.MultiStepLR(optimizer, eval(args.lr_decay_step), args.lr_decay_ratio)
@@ -145,7 +143,8 @@ def main(argv=None):
     start_epoch, best_acc = 0, 0.0
     if args.resume and args.train:
         # the reference saves {'saved_epoch', 'model' (module.-prefixed keys), 'optimizer', 'scheduler', ...} but has
-        # no way to load it back; the momentum buffers are adopted by the fused optimizer on the first batch
+        # no way to load it back; the optimizer state (momentum, Adam moments, Adagrad sums, step count) is adopted by
+        # the fused update on the first batch
         ckpt = torch.load(args.resume, map_location=device)
         model.load_state_dict(ckpt['model'])
         optimizer.load_state_dict(ckpt['optimizer'])
