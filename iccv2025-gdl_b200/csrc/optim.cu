@@ -239,6 +239,26 @@ __global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ param,
   }
 }
 
+// dst = src or dst = dst + src: the gradient sum over replicas run one after another (DGLStep replicas > 1)
+__global__ void __launch_bounds__(256) grad_accumulate_kernel(float* __restrict__ dst, const float* __restrict__ src,
+                                                              int64_t n4, int64_t numel, int accumulate) {
+  pdl_enter();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    float4 s = reinterpret_cast<const float4*>(src)[i];
+    if (accumulate) {
+      const float4 d = reinterpret_cast<const float4*>(dst)[i];
+      s.x = d.x + s.x; s.y = d.y + s.y; s.z = d.z + s.z; s.w = d.w + s.w;
+    }
+    reinterpret_cast<float4*>(dst)[i] = s;
+  }
+  // tail (numel not a multiple of 4)
+  if (blockIdx.x == 0 && threadIdx.x < (numel & 3)) {
+    int64_t i = n4 * 4 + threadIdx.x;
+    dst[i] = accumulate ? dst[i] + src[i] : src[i];
+  }
+}
+
 static unsigned elementwise_blocks(int64_t numel) {
   int64_t n4 = numel / 4;
   int64_t blocks = ceil_div64(n4 > 0 ? n4 : 1, 256);
@@ -332,5 +352,14 @@ extern "C" int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_
   launch_pdl(adagrad_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, sum, numel / 4, numel,
              (float)eps, (float)wd, stats, (const int32_t*)step_state);
   GDL_CHECK_LAUNCH("adagrad_kernel");
+  return GDL_OK;
+}
+
+extern "C" int gdl_grad_accumulate(float* dst, const float* src, int64_t numel, int accumulate, gdl_stream_t s) {
+  GDL_REQUIRE(dst && src && numel > 0, "gdl_grad_accumulate: bad arguments");
+  GDL_REQUIRE((((uintptr_t)dst | (uintptr_t)src) & 15) == 0, "gdl_grad_accumulate: arenas must be 16-byte aligned");
+  launch_pdl(grad_accumulate_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, dst, src, numel / 4, numel,
+             accumulate);
+  GDL_CHECK_LAUNCH("grad_accumulate_kernel");
   return GDL_OK;
 }

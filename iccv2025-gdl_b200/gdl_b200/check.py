@@ -41,12 +41,14 @@ class _Unit:
         self.y = torch.empty_like(self.x)                               # [relu](bn(x) [+ res])
         self.mean, self.invstd = torch.empty(Co, device=dev), torch.empty(Co, device=dev)
 
-    def forward(self, inp, res=None, training=True):
+    def forward(self, inp, res=None, training=True, running=None):
+        """running: the (mean, var) pair a training-mode forward updates (default: the module's own)."""
         lib, bn = _lib.load(), self.bn
+        rm, rv = running if running is not None else (bn.running_mean, bn.running_var)
         check(lib.gdl_check_conv_fwd(C.byref(self.d), self.ci, _p(inp), _p(self.conv.weight.data), _p(self.x), _s()),
               "gdl_check_conv_fwd")
         check(lib.gdl_check_bn_fwd(_p(self.x), _p(res), _p(self.y), self.N, self.C, self.HW, _p(bn.weight.data),
-                                   _p(bn.bias.data), bn.eps, bn.momentum, _p(bn.running_mean), _p(bn.running_var),
+                                   _p(bn.bias.data), bn.eps, bn.momentum, _p(rm), _p(rv),
                                    _p(self.mean), _p(self.invstd), int(self.relu), int(training), _s()),
               "gdl_check_bn_fwd")
         _count(2)
@@ -102,6 +104,7 @@ class CheckEncoder:
         self.Hf, self.Wf, self.Cf = h, w, 512
         self.g_feat = torch.empty(N, 512, h, w, device=device)
         self.folded = torch.empty(N, cin, H, W, device=device)  # private copy: the staging set may be refilled
+        self.stats_sink = (torch.zeros(512, device=device), torch.zeros(512, device=device))  # see EncoderEngine
 
     # ---- interface shared with engine.EncoderEngine ------------------------------------------------------
     def repack(self):
@@ -136,18 +139,19 @@ class CheckEncoder:
         _count()
         self.x_in = self.folded
 
-    def forward(self, x_unused=None, training=True):
+    def forward(self, x_unused=None, training=True, own_stats=True):
         lib = _lib.load()
+        run = None if own_stats else self.stats_sink
         s = self.stem
-        y0 = s.forward(self.x_in, training=training)
+        y0 = s.forward(self.x_in, training=training, running=run)
         check(lib.gdl_check_maxpool_fwd(_p(y0), _p(self.pool_y), _p(self.pool_idx), self.N * 64, s.d.Ho, s.d.Wo, self.Hp,
                                         self.Wp, _s()), "gdl_check_maxpool_fwd")
         _count()
         u = self.pool_y
         for (u1, u2, ud) in self.blocks:
-            y1 = u1.forward(u, training=training)
-            ident = u if ud is None else ud.forward(u, training=training)
-            u = u2.forward(y1, res=ident, training=training)
+            y1 = u1.forward(u, training=training, running=run)
+            ident = u if ud is None else ud.forward(u, training=training, running=run)
+            u = u2.forward(y1, res=ident, training=training, running=run)
         return u
 
     def gap_fwd(self, feat, out, B):

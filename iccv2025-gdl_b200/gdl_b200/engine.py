@@ -93,14 +93,13 @@ class _ConvBN:
         ops.sweep(c)
         rows = ops.conv_fwd_stats(self.d, inp, self.wp, self.x, eng.bn_partial, self.ci_real)
         ops.sweep((not c) if SWEEP else 0)
+        rm, rv = eng.running(bn)
         if rows:
             ops.bn_stats_finalize(eng.bn_partial, rows, self.P, self.C, bn.weight.data, bn.bias.data, bn.eps,
-                                  bn.momentum, bn.running_mean, bn.running_var, self.mean, self.invstd,
-                                  self.scale, self.shift)
+                                  bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
         else:
             ops.bn_stats(self.x, self.P, self.C, eng.bn_partial, bn.weight.data, bn.bias.data, bn.eps,
-                         bn.momentum, bn.running_mean, bn.running_var, self.mean, self.invstd,
-                         self.scale, self.shift)
+                         bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
         # with the statistics out of the conv epilogue the apply pass is the FIRST pass over x after the convolution: it
         # walks against the convolution's direction (starts on the tail that is still in L2) and leaves the head of y,
         # where the next convolution starts, in L2.  GDL_APPLY_SWEEP=0: the round-1 order (same direction).
@@ -135,18 +134,17 @@ class _StemBN(_ConvBN):
 
     def forward(self, eng, x16, res=None):
         bn = self.bn
+        rm, rv = eng.running(bn)
         if STEM_STATS:  # batch statistics out of the stem's epilogue: no separate pass over the largest activation
             rows = ops.stem_fwd_stats(x16, self.wp, self.x, self.N, self.H, self.W, self.ci_real, eng.bn_partial)
             ops.bn_stats_finalize(eng.bn_partial, rows, self.P, self.C, bn.weight.data, bn.bias.data, bn.eps,
-                                  bn.momentum, bn.running_mean, bn.running_var, self.mean, self.invstd,
-                                  self.scale, self.shift)
+                                  bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
             ops.sweep(1 if SWEEP else 0)
         else:
             ops.stem_fwd(x16, self.wp, self.x, self.N, self.H, self.W, self.ci_real)
             ops.sweep(1 if SWEEP else 0)
             ops.bn_stats(self.x, self.P, self.C, eng.bn_partial, bn.weight.data, bn.bias.data, bn.eps,
-                         bn.momentum, bn.running_mean, bn.running_var, self.mean, self.invstd,
-                         self.scale, self.shift)
+                         bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
         # BN-apply + ReLU + MaxPool(3,2,1) in one pass (reference backbone.py:104-106)
         ops.bn_relu_maxpool_fwd(self.x, self.scale, self.shift, eng.pool_y, eng.pool_idx, eng.pool_xmax,
                                 self.N, self.Ho, self.Wo, 64, eng.Hp, eng.Wp)
@@ -192,6 +190,10 @@ class EncoderEngine:
         self.wgrad_ws = torch.empty(max(self.max_wgrad_ws, 16) // 4, device=device, dtype=torch.float32)
         self.bn_partial = torch.empty(self.max_bn_partial, device=device, dtype=torch.float32)
         self.wgrad_stream = torch.cuda.Stream(device) if USE_WGRAD_STREAM else None
+        # running-statistics sink of a forward that must leave the modules' running buffers untouched (a replica
+        # other than the first of a DGLStep with replicas > 1): the finalize kernels update this pair instead
+        self.stats_sink = (torch.zeros(512, device=device), torch.zeros(512, device=device))
+        self.own_stats = True
         self._readers = {}
         self._manual_version = 0
         self._eval_key_folded = None
@@ -275,11 +277,18 @@ class EncoderEngine:
         return u
 
     # ------------------------------------------------------------------ forward
-    def forward(self, x16, training=True):
+    def running(self, bn):
+        """The running-statistics pair a training-mode forward updates: the module's own, or the sink."""
+        return (bn.running_mean, bn.running_var) if self.own_stats else self.stats_sink
+
+    def forward(self, x16, training=True, own_stats=True):
         """x16: bf16 space-to-depth input [N,Hp,Wp,16] -> bf16 [N,Hf,Wf,512] (the layer4 map,
-        reference backbone.py:175-181).  training=False: eval mode, BatchNorm folded into the convolutions."""
+        reference backbone.py:175-181).  training=False: eval mode, BatchNorm folded into the convolutions.
+        own_stats=False: batch statistics as usual, but the BatchNorm running buffers stay bit-identical (the
+        choice is fixed into a CUDA graph that captures the call)."""
         if not training:
             return self.forward_eval(x16)
+        self.own_stats = own_stats
         s = self.stem
         u = s.forward(self, x16)  # stem conv + BN + ReLU + max-pool -> pool_y
         for (u1, u2, ud) in self.blocks:

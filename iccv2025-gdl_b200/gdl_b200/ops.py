@@ -510,6 +510,13 @@ def adagrad(param, grad, state_sum, step_state, numel, lr, lr_decay, eps, wd, st
                                   eps, wd, _ptr(stats), _stream()), "gdl_adagrad")
 
 
+@_op("grad_accumulate", 1, lambda dst, src, numel, accumulate: ("bytes", (12.0 if accumulate else 8.0) * numel))
+def grad_accumulate(dst, src, numel, accumulate):
+    """dst[:numel] = src[:numel] (accumulate False) or dst[:numel] += src[:numel]."""
+    check(_lib.load().gdl_grad_accumulate(_ptr(dst), _ptr(src), numel, int(accumulate), _stream()),
+          "gdl_grad_accumulate")
+
+
 # ---------------------------------------------------------------------------------- data pipeline
 @_op("crop_resize_normalize", 2,
      lambda store, n, Hs, Ws, params, frames, T, S, mean, std, out, table: ("bytes", frames * 3.0 * S * S * 4.0))

@@ -14,6 +14,17 @@ def shard_range(rank, world, batch):
     return lo, min(lo + per, batch)
 
 
+def replicas_per_rank(global_batch, replicas, world):
+    """Data-parallel replicas each of `world` processes runs one after another: `replicas` (R) replicas of
+    global_batch / R rows in torch.chunk order, R / world of them per process (rank r runs replicas
+    r*R/world .. (r+1)*R/world - 1).  ValueError unless R divides the global batch and world divides R."""
+    G, R, W = int(global_batch), int(replicas), int(world)
+    if G < 1 or R < 1 or W < 1 or G % R or R % W:
+        raise ValueError("batch_size {} must split into {} data-parallel replicas of equal size, and the replicas "
+                         "evenly over {} processes".format(G, R, W))
+    return R // W
+
+
 def allreduce_sum_(flat, group=None):
     """In-place SUM all-reduce of a flat gradient arena (NCCL on GPUs, gloo in CPU tests)."""
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:

@@ -109,6 +109,7 @@ class ParamArena:
             p.data = self.param[o:o + n].view(p.shape)
             p.grad = self.grad[o:o + n].view(p.shape)
         self.offset_of = {id(p): o for p, o in zip(self.params, self.offsets)}
+        self.acc = None  # gradient sum of the earlier replicas of a step (DGLStep replicas > 1), see accumulator()
         self.nseg = len(seg_end)
         self.seg_end = torch.tensor(seg_end, device=device, dtype=torch.int64)
         self.seg_group = torch.tensor(seg_group, device=device, dtype=torch.int32)
@@ -124,6 +125,13 @@ class ParamArena:
             return False
         base = self.param.data_ptr()
         return all(p is q and p.data.data_ptr() == base + 4 * o for p, q, o in zip(groups, self.params, self.offsets))
+
+    def accumulator(self):
+        """The fp32 arena (shape of `grad`, loss tail included) that sums the gradients of a step's replicas before
+        the last one; allocated on first use, so a step with one replica per process costs no memory for it."""
+        if self.acc is None:
+            self.acc = torch.zeros_like(self.grad)
+        return self.acc
 
     def set_steps(self, t):
         """Continue from step count t (a restored checkpoint)."""
@@ -149,9 +157,14 @@ class ParamArena:
 class DGLStep:
     def __init__(self, model, batch_size, spec_hw, image_thw, alpha=4.0, lr=0.001, momentum=0.9,
                  weight_decay=1e-4, max_norm=40.0, world_size=1, process_group=None, use_graph=True, check_fp32=None,
-                 rule=None):
+                 rule=None, replicas=1):
         """model: AVClassifier_DGL on a CUDA device (possibly wrapped: `.module` is unwrapped).
-        batch_size: LOCAL batch on this GPU; losses are means over batch_size*world_size.
+        batch_size: rows of ONE replica (the BatchNorm batch); losses are means over batch_size*replicas*world_size.
+        replicas: data-parallel replicas run one after another on this GPU per step (nn.DataParallel over
+        replicas*world_size devices, reference main_dgl.py:244).  A step then takes replicas*batch_size rows; replica k
+        trains on rows [k*batch_size, (k+1)*batch_size) with its own BatchNorm batch statistics, the gradients (and
+        losses) of the replicas are summed on the device before the all-reduce, the clip and the update, and only
+        replica 0 updates the BatchNorm running statistics (DataParallel's replica 0 aliases the module's buffers).
         rule: the update (gdl_b200.optim.UpdateRule, e.g. update_rule(torch_optimizer)); its lr, weight decay and
         momentum replace the three arguments of the same names.  Default: SGD with lr, momentum, weight_decay.
         check_fp32 (default: env GDL_CHECK_FP32): the FP32 check mode — the encoders store fp32 activations and run
@@ -175,7 +188,11 @@ class DGLStep:
         self.rule = rule
         self.alpha, self.lr, self.mu, self.wd, self.max_norm = alpha, rule.lr, rule.momentum, rule.weight_decay, max_norm
         self.world_size, self.pg = world_size, process_group
-        self.inv_batch = 1.0 / (batch_size * world_size)
+        if replicas < 1:
+            raise ValueError("replicas must be >= 1, got {}".format(replicas))
+        self.replicas = R = replicas
+        self.rows = R * batch_size  # rows of this process's share of a global batch
+        self.inv_batch = 1.0 / (batch_size * R * world_size)
         self.n = model.n_classes
         self.use_graph = use_graph
         B, T = self.B, self.T
@@ -187,6 +204,7 @@ class DGLStep:
             arena = ParamArena(model, dev, rule)
             model._gdl_arena = arena
         self.arena = arena
+        self.acc = arena.accumulator() if R > 1 else None
         if check_fp32 is None:
             check_fp32 = os.environ.get("GDL_CHECK_FP32", "0") != "0"
         self.check_fp32 = bool(check_fp32)
@@ -201,8 +219,9 @@ class DGLStep:
         # Inputs: two staging sets (fp32 batch as the reference's DataLoader delivers it).  The layout kernels
         # read the current set OUTSIDE the captured graph and write the fixed-address bf16 stem inputs a8/v8, so
         # the next batch can be copied H2D on a side stream into the other set while this step computes.
-        self._stage = [(torch.zeros(B, self.F_, self.Tt, device=dev), torch.zeros(B, 3, T, self.H, self.W, device=dev),
-                        torch.zeros(B, device=dev, dtype=torch.int64)) for _ in range(2)]
+        rows = self.rows
+        self._stage = [(torch.zeros(rows, self.F_, self.Tt, device=dev), torch.zeros(rows, 3, T, self.H, self.W, device=dev),
+                        torch.zeros(rows, device=dev, dtype=torch.int64)) for _ in range(2)]
         self._cur, self._pending = 0, None
         self._crop_params = None  # device copies of the crop-box tables (prefetch with a VisualPipeline)
         self._audio_params = None  # device copies of the {clip, start} tables (prefetch with an AudioPipeline)
@@ -234,6 +253,8 @@ class DGLStep:
         self._graph = None
         self._graph_b = None
         self._graph_update = None
+        self._graph_first = None  # replicas > 1: replica 0 (owns the running statistics), then acc <- grad
+        self._graph_mid = None    # replicas > 2: replicas 1 .. R-2, acc += grad
         self._graph_lr = None
         self.launches_per_step = None
         # gradient buckets (views of the gradient arena; arena order: head | audio | visual)
@@ -244,6 +265,14 @@ class DGLStep:
             cut_a = ar.late_split(0, self.enc_a.late_parameters())
             cut_v = ar.late_split(1, self.enc_v.late_parameters())
             self._buckets = parallel.gradient_buckets(ar.grad, cut_a, ar.group_ranges[0][1], cut_v)
+        # the ranges grad += acc covers after the last replica (the arena + the 3 losses): all at once, or per bucket
+        # just before that bucket's all-reduce
+        end = self.arena.numel + 3
+        if self.overlap:
+            ea = self.arena.group_ranges[0][1]
+            self._acc_ranges = {"late": [(cut_a, ea), (cut_v, end)], "early": [(0, cut_a), (ea, cut_v)]}
+        else:
+            self._acc_ranges = {"all": [(0, end)]}
 
     # ------------------------------------------------------------------ heads
     def _init_head(self):
@@ -293,16 +322,16 @@ class DGLStep:
     def image_in(self):
         return self._stage[self._cur][1]
 
-    def _enqueue_inputs(self):
-        """Eager, outside the graph: consume the prefetched batch if there is one, then the per-frame
+    def _enqueue_inputs(self, k=0):
+        """Eager, outside the graph: consume the prefetched batch if there is one (k = 0), then the per-frame
         reshape + fp32->bf16 space-to-depth layout of both modalities (reference backbone.py:162-164,
-        main_dgl.py:100) from the current staging set into the fixed-address stem inputs."""
+        main_dgl.py:100) of replica k's rows of the current staging set into the fixed-address stem inputs."""
         B, T = self.B, self.T
         main = torch.cuda.current_stream()
-        if self._pending is not None:
+        if k == 0 and self._pending is not None:
             main.wait_event(self._stage_ready[self._pending])
             self._cur, self._pending = self._pending, None
-        spec, image, label = self._stage[self._cur]
+        spec, image, label = (t[k * B:(k + 1) * B] for t in self._stage[self._cur])
         if self.check_fp32:
             self.enc_a.stage_input(spec, B)
             self.enc_v.stage_input(image, B)
@@ -310,23 +339,42 @@ class DGLStep:
             ops.stem_layout(spec, self.a8, B, 1, 1, self.F_, self.Tt)
             ops.stem_layout(image, self.v8, B, 3, T, self.H, self.W)
         self.label_in.copy_(label, non_blocking=True)
-        self._stage_free[self._cur].record(main)
+        if k == self.replicas - 1:
+            self._stage_free[self._cur].record(main)
 
     def _enqueue(self, lr, first):
+        """The last replica of the step (with replicas == 1 its only one), the all-reduce and the update."""
         if self.overlap:
-            self._enqueue_compute(part=0)
+            self._enqueue_last(part=0)
             works = self._allreduce_late()
-            self._enqueue_compute(part=1)
+            self._enqueue_last(part=1)
             self._allreduce_finish(works)
         else:
-            self._enqueue_compute()
+            self._enqueue_last()
             if self.world_size > 1:
                 self._allreduce()
         self._enqueue_update(lr, first)
 
-    def _enqueue_compute(self, part=None):
+    def _enqueue_last(self, part=None):
+        """Compute of the last replica; with replicas > 1 then grad += acc over the part's range (part 0: the late
+        bucket, so its all-reduce carries the sum over the replicas)."""
+        self._enqueue_compute(part, own_stats=self.replicas == 1)
+        if self.replicas > 1:
+            key = "all" if part is None else ("late", "early")[part]
+            for a, b in self._acc_ranges[key]:
+                ops.grad_accumulate(self.arena.grad[a:b], self.acc[a:b], b - a, True)
+
+    def _enqueue_replica(self, k):
+        """Replica k < replicas - 1: compute, then acc <- grad (k = 0) or acc += grad, over the arena + 3 losses.
+        Only replica 0 updates the BatchNorm running statistics."""
+        self._enqueue_compute(own_stats=k == 0)
+        n = self.arena.numel + 3
+        ops.grad_accumulate(self.acc, self.arena.grad, n, k > 0)
+
+    def _enqueue_compute(self, part=None, own_stats=True):
         """Forward + head + backward on the current stream (+ the two encoder streams).
-        part=0: forward, head and the backward of layer4 + layer3; part=1: the rest of the backward."""
+        part=0: forward, head and the backward of layer4 + layer3; part=1: the rest of the backward.
+        own_stats=False: the forward leaves the BatchNorm running statistics untouched."""
         B, T = self.B, self.T
         main = torch.cuda.current_stream()
         sa, sv = self.stream_a, self.stream_v
@@ -334,10 +382,10 @@ class DGLStep:
             sa.wait_stream(main)
             sv.wait_stream(main)
             with torch.cuda.stream(sa):
-                fa = self.enc_a.forward(self.a8)
+                fa = self.enc_a.forward(self.a8, own_stats=own_stats)
                 self._gap_fwd(self.enc_a, fa, self.a_feat, 1)
             with torch.cuda.stream(sv):
-                fv = self.enc_v.forward(self.v8)
+                fv = self.enc_v.forward(self.v8, own_stats=own_stats)
                 self._gap_fwd(self.enc_v, fv, self.v_feat, T)
             main.wait_stream(sa)
             main.wait_stream(sv)
@@ -443,14 +491,15 @@ class DGLStep:
                 s_spec.copy_(spec, non_blocking=True)
             else:
                 if self._audio_params is None:
-                    self._audio_params = [torch.empty(self.B, 2, device=self.device, dtype=torch.int32) for _ in range(2)]
+                    self._audio_params = [torch.empty(self.rows, 2, device=self.device, dtype=torch.int32)
+                                          for _ in range(2)]
                 self._audio_params[nxt].copy_(spec, non_blocking=True)
                 audio_pipeline(self._audio_params[nxt], out=s_spec)
             if pipeline is None:
                 s_image.copy_(image, non_blocking=True)
             else:
                 if self._crop_params is None:
-                    self._crop_params = [torch.empty(self.B * self.T, 6, device=self.device, dtype=torch.int32)
+                    self._crop_params = [torch.empty(self.rows * self.T, 6, device=self.device, dtype=torch.int32)
                                          for _ in range(2)]
                 self._crop_params[nxt].copy_(image, non_blocking=True)
                 pipeline(self._crop_params[nxt], out=s_image)
@@ -467,8 +516,11 @@ class DGLStep:
         n0 = ops.LAUNCHES
         self._enqueue_inputs()
         if first or not self.use_graph:
+            for k in range(1, self.replicas):
+                self._enqueue_replica(k - 1)
+                self._enqueue_inputs(k)
             self._enqueue(self.lr, first)
-            self.launches_per_step = ops.LAUNCHES - n0  # kernels of libgdl_b200.so per step
+            self.launches_per_step = ops.LAUNCHES - n0  # kernels of libgdl_b200.so per (global) step
         else:
             if self._graph is None or self._graph_lr != self.lr:
                 torch.cuda.synchronize()
@@ -483,17 +535,31 @@ class DGLStep:
                     # NCCL bucket 2 -> graph(update)
                     self._graph = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(self._graph, capture_error_mode=_CAPTURE_MODE):
-                        self._enqueue_compute(part=0 if self.overlap else None)
+                        self._enqueue_last(part=0 if self.overlap else None)
                     self._graph_b = None
                     if self.overlap:
                         self._graph_b = torch.cuda.CUDAGraph()
                         with torch.cuda.graph(self._graph_b, capture_error_mode=_CAPTURE_MODE):
-                            self._enqueue_compute(part=1)
+                            self._enqueue_last(part=1)
                     self._graph_update = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(self._graph_update, capture_error_mode=_CAPTURE_MODE):
                         self._enqueue_update(self.lr, False)
+                # replicas before the last: one graph for replica 0, one shared by replicas 1 .. R-2 (the eager
+                # input layout of the next replica runs between the replays)
+                self._graph_first = self._graph_mid = None
+                for k in range(min(self.replicas - 1, 2)):
+                    g = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(g, capture_error_mode=_CAPTURE_MODE):
+                        self._enqueue_replica(k)
+                    if k == 0:
+                        self._graph_first = g
+                    else:
+                        self._graph_mid = g
                 self._graph_lr = self.lr
-                # capture does not execute: the replay below runs this step
+                # capture does not execute: the replays below run this step
+            for k in range(1, self.replicas):
+                (self._graph_first if k == 1 else self._graph_mid).replay()
+                self._enqueue_inputs(k)
             self._graph.replay()
             if self._graph_b is not None:
                 works = self._allreduce_late()

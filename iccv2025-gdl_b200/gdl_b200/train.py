@@ -14,6 +14,7 @@ import csv
 import torch
 
 from .optim import update_rule
+from .parallel import replicas_per_rank
 from .step import DGLStep
 
 LOG_EVERY = 100  # the reference prints every 100 steps (main_dgl.py:125,144)
@@ -37,7 +38,18 @@ def _get_step(args, model, optimizer, spec, image, pipeline=None, audio_pipeline
     B = spec.shape[0]
     thw = (pipeline.T, pipeline.S, pipeline.S) if pipeline is not None else tuple(image.shape[2:])
     spec_hw = (audio_pipeline.F, audio_pipeline.frames) if audio_pipeline is not None else tuple(spec.shape[1:])
-    key = (B, spec_hw, thw)
+    world = torch.distributed.get_world_size() if torch.distributed.is_available() and \
+        torch.distributed.is_initialized() else 1
+    # args.dp_replicas (main_dgl.py --dp_replicas; 0 = one replica per process): R data-parallel replicas of
+    # batch_size / R rows, R / world of them run one after another by each process (DGLStep replicas)
+    replicas = getattr(args, 'dp_replicas', 0) or 0
+    local = 1
+    if replicas:
+        local = replicas_per_rank(getattr(args, 'batch_size', B * world), replicas, world)
+        if B % local:
+            raise ValueError("a batch of {} rows does not split into {} replicas of equal size (a short last batch: "
+                             "drop it, as the reference's loaders do)".format(B, local))
+    key = (B, spec_hw, thw, local)
     # per-geometry cache (two entries: the full batch and an epoch's short tail batch when the loader does not drop it).
     # The steps share ONE parameter / gradient / momentum arena (DGLStep), so switching costs a weight-shadow refresh,
     # not a re-allocation, a momentum copy and a graph re-capture.
@@ -53,11 +65,10 @@ def _get_step(args, model, optimizer, spec, image, pipeline=None, audio_pipeline
         inner._gdl_step, inner._gdl_step_key = st, key
         return st
     rule = update_rule(optimizer)
-    world = torch.distributed.get_world_size() if torch.distributed.is_available() and \
-        torch.distributed.is_initialized() else 1
     trained = any(s.steps_done > 0 for s in steps.values())
-    st = DGLStep(inner, B, spec_hw, thw, alpha=args.alpha, rule=rule, max_norm=40.0,
-                 world_size=world, process_group=torch.distributed.group.WORLD if world > 1 else None)
+    st = DGLStep(inner, B // local, spec_hw, thw, alpha=args.alpha, rule=rule, max_norm=40.0,
+                 world_size=world, process_group=torch.distributed.group.WORLD if world > 1 else None,
+                 replicas=local)
     adopt_momentum(st.arena, optimizer, st)
     if trained:
         st.momentum_loaded = True

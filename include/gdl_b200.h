@@ -369,6 +369,10 @@ int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32
              double lr, double beta1, double beta2, double eps, double wd, const float* stats, gdl_stream_t s);
 int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
                 double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s);
+/* Gradient accumulation over several replicas run one after another on one GPU (DGLStep replicas > 1):
+ * dst = src (accumulate == 0, 8 bytes per element) or dst = dst + src (accumulate != 0, 12 bytes per element),
+ * fp32, element-wise.  dst and src 16-byte aligned, numel > 0 (any value: a scalar tail covers numel % 4). */
+int gdl_grad_accumulate(float* dst, const float* src, int64_t numel, int accumulate, gdl_stream_t s);
 
 /* ---- visual data pipeline (reference dataset/CramedDataset.py:76-89,96-101; KSDataset.py:160-173,183-190) ---
  * RandomResizedCrop(S) | Resize((S,S)) -> RandomHorizontalFlip -> ToTensor -> Normalize for `frames` frames,

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """CLI-compatible entry point for the reference's main_dgl.py (same flags, same defaults,
 same prints / csv / checkpoint file names, same evaluation-mode checkpoint loading), running the B200-native DGL step.
-Deviations: no TensorBoard branch; `--resume` and `--synthetic_len` are additions.
+Deviations: no TensorBoard branch; `--resume`, `--synthetic_len` and `--dp_replicas` are additions.
 
     python main_dgl.py --train --ckpt_path ckpt --dataset CREMAD --fusion_method concat \
         --fps 3 --alpha 4 --batch_size 64 --audio_path synthetic
@@ -25,6 +25,7 @@ import torch.optim as optim  # noqa: E402
 from torch.utils.data import DataLoader  # noqa: E402
 
 from gdl_b200 import AVClassifier_DGL, setup_seed, weight_init  # noqa: E402
+from gdl_b200.parallel import replicas_per_rank  # noqa: E402
 from gdl_b200.synthetic import SyntheticAV  # noqa: E402
 from gdl_b200.train import train_epoch, valid  # noqa: E402
 
@@ -63,6 +64,9 @@ def get_arguments(argv=None):
     parser.add_argument('--synthetic_len', default=0, type=int, help='synthetic dataset length (0 = CREMA-D sizes)')
     parser.add_argument('--resume', default=None, type=str,
                         help='checkpoint written by this script or by the reference (main_dgl.py:396-412) to continue from')
+    parser.add_argument('--dp_replicas', default=0, type=int,
+                        help='data-parallel replicas R (0 = one per process): batch_size / R rows per BatchNorm batch, '
+                             'R / processes of them run one after another on each GPU, like nn.DataParallel over R GPUs')
     return parser.parse_args(argv)
 
 
@@ -74,6 +78,8 @@ def main(argv=None):
     if args.backbone != 'resnet':
         raise EOFError  # reference main_dgl.py:236-240
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dp_replicas and args.train:
+        replicas_per_rank(args.batch_size, args.dp_replicas, world)  # ValueError before any device or data work
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     device = torch.device('cuda', local)
