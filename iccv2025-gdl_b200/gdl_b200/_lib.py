@@ -95,6 +95,8 @@ SIGNATURES = {
     "gdl_gated_head_scratch_floats": (_l, [_i, _i]),
     "gdl_dgl_head_gated": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _f, _f, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p]),
     "gdl_softmax_ce": (_i, [_p, _p, _f, _f, _p, _p, _p, _i, _i, _p]),
+    "gdl_eval_head": (_i, [_i, _p, _i, _p, _i, _p, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p]),
+    "gdl_eval_count": (_i, [_p, _p, _p, _i, _i, _p]),
     "gdl_gated_fwd": (_i, [_p, _p, _p, _p, _p, _l, _p]),
     "gdl_gated_bwd": (_i, [_p, _p, _p, _p, _p, _p, _l, _p]),
     "gdl_optim_scratch_floats": (_l, [_l, _i]),

@@ -102,11 +102,14 @@ def to_nhwc8(net, x):
 def encoder_map(net, x):
     x8, (N, H, W) = to_nhwc8(net, x)
     eng = net.engine(N, H, W)
-    eng.repack()
-    if not net.training or not torch.is_grad_enabled():
-        # eval / no-grad: BN uses the running statistics when the module is in eval mode
+    if not net.training:
+        # eval: BatchNorm folded into the weights from the running statistics (re-folded only when they changed)
         with torch.no_grad():
-            feat = eng.forward(x8, training=net.training)
+            return eng.forward(x8, training=False).permute(0, 3, 1, 2).float()
+    eng.repack()
+    if not torch.is_grad_enabled():
+        with torch.no_grad():
+            feat = eng.forward(x8)
             return feat.permute(0, 3, 1, 2).float()
     params = eng.parameters()
     out = _EncoderMapFn.apply(net, x8, eng, *params)

@@ -42,6 +42,11 @@ class AVClassifier_DGL(nn.Module):
         self.n_classes = n_classes
 
     def forward(self, audio, visual):
+        if not self.training:
+            # eval mode: the EvalStep valid() runs (folded BatchNorm, fused pooling + head), so the logits of
+            # model(...) and of valid() come from one arithmetic; no autograd graph is recorded
+            from .step import eval_forward
+            return eval_forward(self, audio, visual)
         a = self.audio_net(audio)    # [B,512,h,w]
         v = self.visual_net(visual)  # [B*T,512,7,7]
         (_, C, H, W) = v.size()

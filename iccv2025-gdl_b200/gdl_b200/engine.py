@@ -36,6 +36,17 @@ APPLY_SWEEP = int(os.environ.get("GDL_APPLY_SWEEP", "1"))
 STEM_STATS = int(os.environ.get("GDL_STEM_STATS", "1"))  # BatchNorm statistics of the stem from its epilogue
 
 
+def note_writes(module):
+    """Record that kernels changed `module`'s parameters or buffers behind torch's version counters (an optimizer
+    update over the parameter arena, the BatchNorm running statistics of a training forward, a weight refresh).
+    The eval-mode fold (EncoderEngine.fold_eval) and the FiLM eval shadow re-derive themselves when this count moves."""
+    module._gdl_writes = getattr(module, "_gdl_writes", 0) + 1
+
+
+def kernel_writes(module):
+    return getattr(module, "_gdl_writes", 0)
+
+
 class _Pool:
     """Static buffer planner: buffers are requested/released while the plan is built; a released
     buffer of the same size is reused by a later request (backward temporaries)."""
@@ -195,7 +206,6 @@ class EncoderEngine:
         self.stats_sink = (torch.zeros(512, device=device), torch.zeros(512, device=device))
         self.own_stats = True
         self._readers = {}
-        self._manual_version = 0
         self._eval_key_folded = None
         self._plan_backward()
         self.repack()
@@ -209,7 +219,7 @@ class EncoderEngine:
     def repack(self):
         """Refresh the bf16 shadows from the fp32 masters (after every optimizer step): one multi-tensor
         launch for the 19 block convolutions + the stem's own packer."""
-        self._manual_version += 1  # parameters / running statistics changed behind torch's version counters
+        note_writes(self.net)  # parameters / running statistics changed behind torch's version counters
         convs = [u for u in self.units if u is not self.stem]
         key = tuple(u.conv.weight.data_ptr() for u in convs)
         if getattr(self, "_pack_key", None) != key:  # the parameters moved (e.g. into the step's arena)
@@ -221,7 +231,7 @@ class EncoderEngine:
 
     # ------------------------------------------------------------------ eval mode: BatchNorm folded into the conv
     def _eval_key(self):
-        v = self._manual_version
+        v = kernel_writes(self.net)
         for u in self.units:
             bn = u.bn
             v += (u.conv.weight._version + bn.weight._version + bn.bias._version + bn.running_mean._version
@@ -234,7 +244,8 @@ class EncoderEngine:
         separate bf16 shadows (w' = w * scale, one multi-tensor pack launch with gdl_pack_entry.scale), and
         shift = beta - running_mean * scale becomes the bias of the conv epilogue (gdl_conv_fwd_bias_act), together
         with the residual add and the ReLU: an eval unit is ONE kernel, no BatchNorm pass.  Re-folded only when a
-        parameter / buffer changed (torch version counters + the engine's own counter for kernel-side updates)."""
+        parameter / buffer changed (torch version counters + the module's count of kernel-side writes, note_writes).
+        Runs outside any CUDA graph: a graph that captured forward_eval reads the fold's fixed-address buffers."""
         key = self._eval_key()
         if self._eval_key_folded == key:
             return

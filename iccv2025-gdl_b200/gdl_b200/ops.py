@@ -381,6 +381,33 @@ def dgl_head_gated(a, v, Wx, bx, Wy, by, Wo, bo, labels, alpha, inv_batch, logit
                                          _ptr(dWo), _ptr(dbo), _ptr(scratch), B, D, n, _stream()), "gdl_dgl_head_gated")
 
 
+EVAL_KINDS = {"concat": 0, "sum": 1, "gated": 2, "pool": 3}
+
+
+def _eval_head_bytes(kind, fa, Ga, fv, Gv, Wx, Wy, ldw, bx, by, Wo, bo, x_gate, labels, a_out, v_out, logits, counts,
+                     B, n):
+    """Map reads (the weights are re-read from L2 by every CTA: counted once) + pooled / logit writes."""
+    w = {0: n * 2 * 512, 1: n * 2 * 512, 2: 2 * 512 * 512 + n * 512, 3: 0}[kind]
+    return ("bytes", 2.0 * B * (Ga + Gv) * 512 + 4.0 * w + (8.0 * B * 512 if a_out is not None else 0.0)
+            + (12.0 * B * n if logits is not None else 0.0))
+
+
+@_op("eval_head", 1, _eval_head_bytes)
+def eval_head(kind, fa, Ga, fv, Gv, Wx, Wy, ldw, bx, by, Wo, bo, x_gate, labels, a_out, v_out, logits, counts, B, n):
+    """Eval-mode head from the bf16 NHWC layer-4 maps (include/gdl_b200.h gdl_eval_head): pooling, the three logit
+    sets of `kind` (EVAL_KINDS), their row arg-max, and `counts[h] += correct` when labels is given.
+    Wx / Wy are raw integer device addresses or tensors (concat's Wy points into the middle of fc_out.weight)."""
+    check(_lib.load().gdl_eval_head(kind, _ptr(fa), Ga, _ptr(fv), Gv, _addr(Wx), _addr(Wy), ldw, _ptr(bx), _ptr(by),
+                                    _ptr(Wo), _ptr(bo), int(x_gate), _ptr(labels), _ptr(a_out), _ptr(v_out),
+                                    _ptr(logits), _ptr(counts), B, n, _stream()), "gdl_eval_head")
+
+
+@_op("eval_count", 1, lambda logits, labels, counts, B, n: ("bytes", 12.0 * B * n + 8.0 * B))
+def eval_count(logits, labels, counts, B, n):
+    """counts[h] += #rows of logits[h] ([3, B, n]) whose arg-max equals the label."""
+    check(_lib.load().gdl_eval_count(_ptr(logits), _ptr(labels), _ptr(counts), B, n, _stream()), "gdl_eval_count")
+
+
 @_op("softmax_ce", 2)
 def softmax_ce(logits, labels, loss_scale, grad_scale, loss_out, dlogits, scratch, B, n):
     check(_lib.load().gdl_softmax_ce(_ptr(logits), _ptr(labels), loss_scale, grad_scale, _ptr(loss_out),

@@ -59,6 +59,20 @@ def allreduce_finish(works, tensors, group=None):
         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
 
 
+def broadcast_running_stats(model, group=None):
+    """Give every rank rank 0's BatchNorm running statistics (one broadcast of their concatenation).  This is what
+    nn.DataParallel evaluates with: its replicas are copies of device 0's module and keep no statistics of their own."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return
+    bufs = [b for m in model.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)
+            for b in (m.running_mean, m.running_var)]
+    flat = torch.cat([b.reshape(-1) for b in bufs])
+    dist.broadcast(flat, src=0, group=group)
+    if dist.get_rank(group) != 0:  # rank 0 keeps its buffers untouched (and its BatchNorm fold valid)
+        for b, v in zip(bufs, flat.split([b.numel() for b in bufs])):
+            b.copy_(v.view_as(b))
+
+
 class ChunkShardBatchSampler(torch.utils.data.Sampler):
     """Batch sampler for one rank of a data-parallel run that reproduces what nn.DataParallel does to the reference's
     DataLoader (main_dgl.py:244,284-288): ONE global sample order (any sampler — RandomSampler for shuffle=True,

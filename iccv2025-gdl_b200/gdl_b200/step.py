@@ -21,6 +21,7 @@ import os
 import torch
 
 from . import ops, parallel
+from .engine import kernel_writes, note_writes
 from .autograd import to_nhwc8  # noqa: F401  (re-export for callers)
 from .basic_model import AVClassifier_DGL
 from .fusion_modules import ConcatFusion_DGL, FiLM_DGL, GatedFusion_DGL, SumFusion_DGL
@@ -154,6 +155,73 @@ class ParamArena:
         return cut
 
 
+class InputStage:
+    """Two device staging sets for batches of `rows` rows of the reference contract (fp32 spectrograms [rows, F, Tt],
+    fp32 frames [rows, 3, T, H, W], int64 labels) and the copy stream that fills the set the running step does not
+    read, so the H2D copy (or the device data pipeline) of the next batch overlaps the current batch's kernels.
+    Shared by DGLStep (training) and EvalStep (validation)."""
+
+    def __init__(self, device, rows, spec_hw, image_thw):
+        F_, Tt = spec_hw
+        T, H, W = image_thw
+        self.device, self.rows, self.T = device, rows, T
+        self.sets = [(torch.zeros(rows, F_, Tt, device=device), torch.zeros(rows, 3, T, H, W, device=device),
+                      torch.zeros(rows, device=device, dtype=torch.int64)) for _ in range(2)]
+        self.cur, self.pending = 0, None
+        self.crop_params = None   # device copies of the crop-box tables (prefetch with a VisualPipeline)
+        self.audio_params = None  # device copies of the {clip, start} tables (prefetch with an AudioPipeline)
+        self.copy_stream = torch.cuda.Stream(device)
+        self.ready = [torch.cuda.Event() for _ in range(2)]
+        self.free = [torch.cuda.Event() for _ in range(2)]
+
+    def current(self):
+        return self.sets[self.cur]
+
+    def acquire(self, stream):
+        """Make `stream` wait for a prefetched batch and make it the current set."""
+        if self.pending is not None:
+            stream.wait_event(self.ready[self.pending])
+            self.cur, self.pending = self.pending, None
+
+    def release(self, stream):
+        """The kernels enqueued on `stream` so far are the last readers of the current set."""
+        self.free[self.cur].record(stream)
+
+    def load(self, spec, image, label):
+        """Copy a batch (host or device tensors) into the current set on the current stream."""
+        self.pending = None
+        for dst, src in zip(self.sets[self.cur], (spec, image, label)):
+            if src.data_ptr() != dst.data_ptr():
+                dst.copy_(src, non_blocking=True)
+
+    def prefetch(self, spec, image, label, pipeline=None, audio_pipeline=None):
+        """Start the copy of the next batch into the other set on the copy stream (see DGLStep.prefetch)."""
+        nxt = 1 - self.cur
+        cs = self.copy_stream
+        cs.wait_event(self.free[nxt])  # the layout kernels that last read this set have run
+        with torch.cuda.stream(cs):
+            s_spec, s_image, s_label = self.sets[nxt]
+            s_label.copy_(label, non_blocking=True)
+            if audio_pipeline is None:
+                s_spec.copy_(spec, non_blocking=True)
+            else:
+                if self.audio_params is None:
+                    self.audio_params = [torch.empty(self.rows, 2, device=self.device, dtype=torch.int32)
+                                         for _ in range(2)]
+                self.audio_params[nxt].copy_(spec, non_blocking=True)
+                audio_pipeline(self.audio_params[nxt], out=s_spec)
+            if pipeline is None:
+                s_image.copy_(image, non_blocking=True)
+            else:
+                if self.crop_params is None:
+                    self.crop_params = [torch.empty(self.rows * self.T, 6, device=self.device, dtype=torch.int32)
+                                        for _ in range(2)]
+                self.crop_params[nxt].copy_(image, non_blocking=True)
+                pipeline(self.crop_params[nxt], out=s_image)
+            self.ready[nxt].record(cs)
+        self.pending = nxt
+
+
 class DGLStep:
     def __init__(self, model, batch_size, spec_hw, image_thw, alpha=4.0, lr=0.001, momentum=0.9,
                  weight_decay=1e-4, max_norm=40.0, world_size=1, process_group=None, use_graph=True, check_fp32=None,
@@ -219,15 +287,8 @@ class DGLStep:
         # Inputs: two staging sets (fp32 batch as the reference's DataLoader delivers it).  The layout kernels
         # read the current set OUTSIDE the captured graph and write the fixed-address bf16 stem inputs a8/v8, so
         # the next batch can be copied H2D on a side stream into the other set while this step computes.
-        rows = self.rows
-        self._stage = [(torch.zeros(rows, self.F_, self.Tt, device=dev), torch.zeros(rows, 3, T, self.H, self.W, device=dev),
-                        torch.zeros(rows, device=dev, dtype=torch.int64)) for _ in range(2)]
-        self._cur, self._pending = 0, None
-        self._crop_params = None  # device copies of the crop-box tables (prefetch with a VisualPipeline)
-        self._audio_params = None  # device copies of the {clip, start} tables (prefetch with an AudioPipeline)
-        self.copy_stream = torch.cuda.Stream(dev)
-        self._stage_ready = [torch.cuda.Event() for _ in range(2)]
-        self._stage_free = [torch.cuda.Event() for _ in range(2)]
+        self.stage = InputStage(dev, self.rows, spec_hw, image_thw)
+        self.copy_stream = self.stage.copy_stream
         self.label_in = torch.zeros(B, device=dev, dtype=torch.int64)  # fixed address: read inside the graph
         self.a8 = self.v8 = None
         if not self.check_fp32:
@@ -316,11 +377,11 @@ class DGLStep:
     # ------------------------------------------------------------------ the step
     @property
     def spec_in(self):
-        return self._stage[self._cur][0]
+        return self.stage.current()[0]
 
     @property
     def image_in(self):
-        return self._stage[self._cur][1]
+        return self.stage.current()[1]
 
     def _enqueue_inputs(self, k=0):
         """Eager, outside the graph: consume the prefetched batch if there is one (k = 0), then the per-frame
@@ -328,10 +389,9 @@ class DGLStep:
         main_dgl.py:100) of replica k's rows of the current staging set into the fixed-address stem inputs."""
         B, T = self.B, self.T
         main = torch.cuda.current_stream()
-        if k == 0 and self._pending is not None:
-            main.wait_event(self._stage_ready[self._pending])
-            self._cur, self._pending = self._pending, None
-        spec, image, label = (t[k * B:(k + 1) * B] for t in self._stage[self._cur])
+        if k == 0:
+            self.stage.acquire(main)
+        spec, image, label = (t[k * B:(k + 1) * B] for t in self.stage.current())
         if self.check_fp32:
             self.enc_a.stage_input(spec, B)
             self.enc_v.stage_input(image, B)
@@ -340,7 +400,7 @@ class DGLStep:
             ops.stem_layout(image, self.v8, B, 3, T, self.H, self.W)
         self.label_in.copy_(label, non_blocking=True)
         if k == self.replicas - 1:
-            self._stage_free[self._cur].record(main)
+            self.stage.release(main)
 
     def _enqueue(self, lr, first):
         """The last replica of the step (with replicas == 1 its only one), the all-reduce and the update."""
@@ -464,10 +524,7 @@ class DGLStep:
     def load_inputs(self, spec, image, label):
         """Copy a batch (host or device tensors of the reference contract) into the current staging set,
         on the current stream (the synchronous path; see prefetch() for the overlapped one)."""
-        self._pending = None
-        for dst, src in zip(self._stage[self._cur], (spec, image, label)):
-            if src.data_ptr() != dst.data_ptr():
-                dst.copy_(src, non_blocking=True)
+        self.stage.load(spec, image, label)
 
     def prefetch(self, spec, image, label, pipeline=None, audio_pipeline=None):
         """Start the H2D copy of the NEXT batch (pinned host tensors) on the copy stream into the staging
@@ -481,30 +538,7 @@ class DGLStep:
         cross PCIe.
         audio_pipeline: a datapipe.AudioPipeline — `spec` is then the int32 [B, 2] table {clip index, start sample}
         and the log-STFT spectrograms are computed on the device from the resident waveforms (gdl_log_stft)."""
-        nxt = 1 - self._cur
-        cs = self.copy_stream
-        cs.wait_event(self._stage_free[nxt])  # the layout kernels that last read this set have run
-        with torch.cuda.stream(cs):
-            s_spec, s_image, s_label = self._stage[nxt]
-            s_label.copy_(label, non_blocking=True)
-            if audio_pipeline is None:
-                s_spec.copy_(spec, non_blocking=True)
-            else:
-                if self._audio_params is None:
-                    self._audio_params = [torch.empty(self.rows, 2, device=self.device, dtype=torch.int32)
-                                          for _ in range(2)]
-                self._audio_params[nxt].copy_(spec, non_blocking=True)
-                audio_pipeline(self._audio_params[nxt], out=s_spec)
-            if pipeline is None:
-                s_image.copy_(image, non_blocking=True)
-            else:
-                if self._crop_params is None:
-                    self._crop_params = [torch.empty(self.rows * self.T, 6, device=self.device, dtype=torch.int32)
-                                         for _ in range(2)]
-                self._crop_params[nxt].copy_(image, non_blocking=True)
-                pipeline(self._crop_params[nxt], out=s_image)
-            self._stage_ready[nxt].record(cs)
-        self._pending = nxt
+        self.stage.prefetch(spec, image, label, pipeline, audio_pipeline)
 
     def step(self, spec=None, image=None, label=None, lr=None):
         """Run one training step; returns the device tensor `stats` (8 floats, see __init__)."""
@@ -571,9 +605,220 @@ class DGLStep:
                 self._graph_update.replay()
         self.steps_done += 1
         self.arena.steps += 1
+        for m in (self.model.audio_net, self.model.visual_net, self.model.fusion_module):
+            note_writes(m)  # the update and the running statistics changed on the device (graph replays included)
         return self.stats
 
     def read_stats(self):
         """One D2H copy: (Lf, La, Lv, grad_norm, clip_coef, audio_grad_sum, visual_grad_sum)."""
         s = self.stats.tolist()
         return s[0], s[1], s[2], s[4], s[5], s[6], s[7]
+
+
+# ---------------------------------------------------------------------------------------------------- evaluation
+def _eval_resources(model, rows, spec_hw, image_thw):
+    """(b, audio engine, visual engine, training step or None) that an EvalStep of `rows` rows runs on.  When a
+    training step of this geometry has a per-replica batch b dividing `rows` (with --dp_replicas the step's rows are
+    R_local * b), evaluation runs in sub-batches of b on the training step's own engines, so nothing is evicted or
+    rebuilt and no second set of activation buffers is allocated.  Otherwise the modules' engine cache serves `rows`."""
+    steps = list(getattr(model, "_gdl_steps", {}).values())
+    cur = getattr(model, "_gdl_step", None)
+    if cur is not None and cur not in steps:
+        steps.append(cur)
+    for st in sorted(steps, key=lambda st: -st.B):
+        if (not st.check_fp32 and (st.F_, st.Tt) == tuple(spec_hw) and (st.T, st.H, st.W) == tuple(image_thw)
+                and rows % st.B == 0):
+            return st.B, st.enc_a, st.enc_v, st
+    (F_, Tt), (T, H, W) = spec_hw, image_thw
+    return rows, model.audio_net.engine(rows, F_, Tt), model.visual_net.engine(rows * T, H, W), None
+
+
+def eval_counts(model, device):
+    """The model's int64 [3] device counter of correct arg-maxes (out, out_a, out_v) that every EvalStep adds to."""
+    c = getattr(model, "_gdl_eval_counts", None)
+    if c is None or c.device != device:
+        c = model._gdl_eval_counts = torch.zeros(3, device=device, dtype=torch.int64)
+    return c
+
+
+class EvalStep:
+    """Eval-mode forward of AVClassifier_DGL for batches of `rows` rows (reference valid(), main_dgl.py:168-222, and
+    `model(...)` in eval mode): stem layout of each sub-batch of b rows, both encoders with BatchNorm folded
+    (EncoderEngine.forward_eval) on the audio and visual streams, then the eval head (gdl_eval_head: pooling, the
+    three logit sets, arg-max and correct counts into `counts`; FiLM: pooling, the FiLM forward GEMMs, fc_out and
+    gdl_eval_count).  Everything after the layout is one CUDA graph, captured on the second call and re-captured only
+    when a head parameter moves.  The BatchNorm fold and the FiLM weight shadow are refreshed outside the graph, and
+    only when a parameter or buffer changed.  The logits of the last sub-batch stay in `logits` [3, b, n]."""
+
+    def __init__(self, model, rows, spec_hw, image_thw, use_graph=True):
+        model = getattr(model, "module", model)
+        if not isinstance(model, AVClassifier_DGL):
+            raise TypeError("EvalStep needs a gdl_b200.AVClassifier_DGL")
+        dev = next(model.parameters()).device
+        if dev.type != "cuda":
+            raise RuntimeError("EvalStep runs on a B200 only (no CPU fallback)")
+        ops.init()
+        self.model, self.device, self.rows = model, dev, rows
+        self.F_, self.Tt = spec_hw
+        self.T, self.H, self.W = image_thw
+        self.n = model.n_classes
+        self.use_graph = use_graph
+        self.B, self.enc_a, self.enc_v, train_step = _eval_resources(model, rows, spec_hw, image_thw)
+        self.chunks = rows // self.B
+        B, dev_kw = self.B, dict(device=dev)
+        self.stage = InputStage(dev, rows, spec_hw, image_thw)
+        if train_step is not None:  # the fixed-address stem inputs of the training step: rewritten before every use
+            self.a8, self.v8 = train_step.a8, train_step.v8
+        else:
+            self.a8 = torch.empty(self.enc_a.input_shape, dtype=torch.bfloat16, **dev_kw)
+            self.v8 = torch.empty(self.enc_v.input_shape, dtype=torch.bfloat16, **dev_kw)
+        self.label_in = torch.full((B,), -1, dtype=torch.int64, **dev_kw)
+        self.logits = torch.empty(3, B, self.n, **dev_kw)
+        self.counts = eval_counts(model, dev)
+        fm = model.fusion_module
+        self.kind = "film" if isinstance(fm, FiLM_DGL) else "gated" if isinstance(fm, GatedFusion_DGL) else \
+            "sum" if isinstance(fm, SumFusion_DGL) else "concat" if isinstance(fm, ConcatFusion_DGL) else None
+        if self.kind is None:
+            raise NotImplementedError('Incorrect fusion method: {}!'.format(type(fm).__name__))
+        self.film, self._film_key = None, None
+        if self.kind == "film":
+            from .film import FilmChunkBuffers
+            self.a_feat, self.v_feat = torch.empty(B, 512, **dev_kw), torch.empty(B, 512, **dev_kw)
+            self.film = train_step.film.buf if train_step is not None and train_step.film is not None \
+                else FilmChunkBuffers(B, dev)
+        self.stream_a, self.stream_v = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
+        self.calls = 0
+        self._graph, self._graph_key = None, None
+
+    # ------------------------------------------------------------------ outside the graph
+    def refresh(self):
+        """Re-fold BatchNorm into the eval weight packs and re-derive the FiLM bf16 shadow, each only if its inputs
+        changed since the last call (torch version counters + engine.note_writes counts)."""
+        self.enc_a.fold_eval()
+        self.enc_v.fold_eval()
+        if self.film is not None:
+            w = self.model.fusion_module.fc.weight
+            key = (w.data_ptr(), w._version, kernel_writes(self.model.fusion_module))
+            if key != self._film_key:
+                self.film.refresh(w.data)
+                self._film_key = key
+
+    def _enqueue_inputs(self, k):
+        """Sub-batch k of the current staging set -> the fixed-address stem inputs and labels."""
+        B, T = self.B, self.T
+        main = torch.cuda.current_stream()
+        if k == 0:
+            self.stage.acquire(main)
+        spec, image, label = (t[k * B:(k + 1) * B] for t in self.stage.current())
+        ops.stem_layout(spec, self.a8, B, 1, 1, self.F_, self.Tt)
+        ops.stem_layout(image, self.v8, B, 3, T, self.H, self.W)
+        self.label_in.copy_(label, non_blocking=True)
+        if k == self.chunks - 1:
+            self.stage.release(main)
+
+    # ------------------------------------------------------------------ the captured part
+    def _enqueue(self):
+        main = torch.cuda.current_stream()
+        sa, sv = self.stream_a, self.stream_v
+        sa.wait_stream(main)
+        sv.wait_stream(main)
+        with torch.cuda.stream(sa):
+            fa = self.enc_a.forward_eval(self.a8)
+        with torch.cuda.stream(sv):
+            fv = self.enc_v.forward_eval(self.v8)
+        main.wait_stream(sa)
+        main.wait_stream(sv)
+        fm, B, n, D = self.model.fusion_module, self.B, self.n, 512
+        Ga, Gv = self.enc_a.Hf * self.enc_a.Wf, self.T * self.enc_v.Hf * self.enc_v.Wf
+        if self.kind == "concat":
+            W = fm.fc_out.weight
+            ops.eval_head(0, fa, Ga, fv, Gv, W.data_ptr(), W.data_ptr() + 4 * D, 2 * D, fm.fc_out.bias.data, None,
+                          None, None, 1, self.label_in, None, None, self.logits, self.counts, B, n)
+        elif self.kind == "sum":
+            ops.eval_head(1, fa, Ga, fv, Gv, fm.fc_x.weight.data_ptr(), fm.fc_y.weight.data_ptr(), D, fm.fc_x.bias.data,
+                          fm.fc_y.bias.data, None, None, 1, self.label_in, None, None, self.logits, self.counts, B, n)
+        elif self.kind == "gated":
+            ops.eval_head(2, fa, Ga, fv, Gv, fm.fc_x.weight.data_ptr(), fm.fc_y.weight.data_ptr(), D, fm.fc_x.bias.data,
+                          fm.fc_y.bias.data, fm.fc_out.weight.data, fm.fc_out.bias.data, fm.x_gate, self.label_in, None,
+                          None, self.logits, self.counts, B, n)
+        else:
+            from .film import CHUNK_I, FC
+            b = self.film
+            ops.eval_head(3, fa, Ga, fv, Gv, None, None, 0, None, None, None, None, 1, None, self.a_feat, self.v_feat,
+                          None, None, B, n)
+            # H = sum over chunks of Zt_c^T W1t_c + b1 (rows: [a (x) v | a (x) a | v (x) v]), as in FilmHead.run
+            for c in range(D // CHUNK_I):
+                ops.film_outer_chunk(self.a_feat, self.v_feat, b.Zt, B, D, b.ZB, 3, b.scratch, c * FC, FC)
+                if c == 0:
+                    ops.gemm_tn_f32(b.Zt, b.W1t[:FC], fm.fc.bias.data, b.H, b.ZB, D, FC, b.ws)
+                else:
+                    ops.gemm_tn_f32_acc(b.Zt, b.W1t[c * FC:(c + 1) * FC], b.H, b.ZB, D, FC, b.ws)
+            for i in range(3):
+                ops.linear_fwd(b.H[i * B:(i + 1) * B], fm.fc_out.weight.data, fm.fc_out.bias.data, self.logits[i],
+                               B, D, n)
+            ops.eval_count(self.logits, self.label_in, self.counts, B, n)
+
+    def _compute(self, k):
+        """Sub-batch k: eager the first time (and without graphs), a graph replay afterwards."""
+        if not self.use_graph or self.calls == 0:
+            self._enqueue()
+            return
+        key = tuple(p.data_ptr() for p in self.model.fusion_module.parameters()) + (self.counts.data_ptr(),)
+        if self._graph is None or self._graph_key != key:
+            torch.cuda.synchronize()
+            self._graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(self._graph, capture_error_mode=_CAPTURE_MODE):
+                self._enqueue()
+            self._graph_key = key
+        self._graph.replay()
+
+    def run(self, out=None):
+        """Evaluate the current (or just prefetched) batch: counts += correct arg-maxes of its rows.  out: optional
+        f32 [3, rows, n] that receives the logits (out, out_a, out_v) of every row."""
+        self.refresh()
+        for k in range(self.chunks):
+            self._enqueue_inputs(k)
+            self._compute(k)
+            if out is not None:
+                out[:, k * self.B:(k + 1) * self.B].copy_(self.logits)
+        self.calls += 1
+
+    def load_inputs(self, spec, image, label=None):
+        """Synchronous input path: spec [rows, F, Tt] (or [rows, 1, F, Tt]), image [rows, 3, T, H, W], label [rows] or
+        None (a label of -1 is never counted)."""
+        if label is None:
+            label = torch.full((self.rows,), -1, dtype=torch.int64, device=self.device)
+        self.stage.load(spec.reshape(self.rows, self.F_, self.Tt), image, label)
+
+    def prefetch(self, spec, image, label, pipeline=None, audio_pipeline=None):
+        """Start the copy of the next batch on the copy stream (DGLStep.prefetch); the next run() consumes it."""
+        self.stage.prefetch(spec, image, label, pipeline, audio_pipeline)
+
+
+def get_eval_step(model, rows, spec_hw, image_thw):
+    """The model's cached EvalStep for this geometry (two live entries: the full batch and a short tail batch).  The
+    cache key includes the engines it runs on, so a training step created later is picked up."""
+    model = getattr(model, "module", model)
+    cache = getattr(model, "_gdl_evals", None)
+    if cache is None:
+        cache = model._gdl_evals = {}
+    b, enc_a, enc_v, _ = _eval_resources(model, rows, spec_hw, image_thw)
+    key = (rows, tuple(spec_hw), tuple(image_thw), b, id(enc_a), id(enc_v))
+    ev = cache.pop(key, None)
+    if ev is None:
+        ev = EvalStep(model, rows, spec_hw, image_thw)
+        while len(cache) >= 2:
+            cache.pop(next(iter(cache)))
+    cache[key] = ev  # most recently used last
+    return ev
+
+
+def eval_forward(model, audio, visual):
+    """`model(audio, visual)` in eval mode: (out, a_out, v_out) of the EvalStep that valid() runs, bit for bit."""
+    B = audio.shape[0]
+    spec_hw, thw = tuple(audio.shape[-2:]), tuple(visual.shape[2:])
+    ev = get_eval_step(model, B, spec_hw, thw)
+    out = torch.empty(3, B, ev.n, device=ev.device)
+    ev.load_inputs(audio.float(), visual.float())
+    ev.run(out)
+    return out[0], out[1], out[2]

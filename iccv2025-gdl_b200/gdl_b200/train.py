@@ -14,8 +14,8 @@ import csv
 import torch
 
 from .optim import update_rule
-from .parallel import replicas_per_rank
-from .step import DGLStep
+from .parallel import ChunkShardBatchSampler, broadcast_running_stats, replicas_per_rank
+from .step import DGLStep, eval_counts, get_eval_step
 
 LOG_EVERY = 100  # the reference prints every 100 steps (main_dgl.py:125,144)
 GRAD_CSV = 'audio_visual_grad_vanilla.csv'  # main_dgl.py:148
@@ -33,13 +33,32 @@ def _audio_pipeline_of(dataloader):
     return getattr(getattr(dataloader, "dataset", None), "device_audio_pipeline", None)
 
 
+def _geometry(spec, image, pipeline=None, audio_pipeline=None):
+    """(spectrogram (F, Tt), frames (T, H, W)) of a batch as the loader delivers it."""
+    thw = (pipeline.T, pipeline.S, pipeline.S) if pipeline is not None else tuple(image.shape[2:])
+    spec_hw = (audio_pipeline.F, audio_pipeline.frames) if audio_pipeline is not None else tuple(spec.shape[1:])
+    return spec_hw, thw
+
+
+def _prefetch(step, batch, pipe, apipe):
+    """Start the copy of `batch` into the step's (DGLStep or EvalStep) other staging set.  With the device pipelines
+    batch[1] is the int32 [B, T, 6] table of host-drawn crop boxes, batch[0] {clip, start} with apipe."""
+    if pipe is None:
+        step.prefetch(*batch, audio_pipeline=apipe)
+    else:
+        step.prefetch(batch[0], batch[1].reshape(-1, 6), batch[2], pipeline=pipe, audio_pipeline=apipe)
+
+
+def _world():
+    return torch.distributed.get_world_size() if torch.distributed.is_available() and \
+        torch.distributed.is_initialized() else 1
+
+
 def _get_step(args, model, optimizer, spec, image, pipeline=None, audio_pipeline=None):
     inner = getattr(model, "module", model)
     B = spec.shape[0]
-    thw = (pipeline.T, pipeline.S, pipeline.S) if pipeline is not None else tuple(image.shape[2:])
-    spec_hw = (audio_pipeline.F, audio_pipeline.frames) if audio_pipeline is not None else tuple(spec.shape[1:])
-    world = torch.distributed.get_world_size() if torch.distributed.is_available() and \
-        torch.distributed.is_initialized() else 1
+    spec_hw, thw = _geometry(spec, image, pipeline, audio_pipeline)
+    world = _world()
     # args.dp_replicas (main_dgl.py --dp_replicas; 0 = one replica per process): R data-parallel replicas of
     # batch_size / R rows, R / world of them run one after another by each process (DGLStep replicas)
     replicas = getattr(args, 'dp_replicas', 0) or 0
@@ -146,18 +165,12 @@ def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, wr
 
     # one batch of look-ahead: the H2D copy of batch k+1 (copy stream) overlaps the kernels of step k
     pipe, apipe = _pipeline_of(dataloader), _audio_pipeline_of(dataloader)
-
-    def prefetch(step, batch):
-        if pipe is None:
-            step.prefetch(*batch)
-        else:  # batch[1] is the int32 [B, T, 6] table of host-drawn crop boxes, batch[0] {clip, start} with apipe
-            step.prefetch(batch[0], batch[1].reshape(-1, 6), batch[2], pipeline=pipe, audio_pipeline=apipe)
     it = iter(dataloader)
     nxt = next(it, None)
     st = None
     if nxt is not None:
         st = _get_step(args, model, optimizer, nxt[0], nxt[1], pipe, apipe)
-        prefetch(st, nxt)
+        _prefetch(st, nxt, pipe, apipe)
     step_i = -1
     while nxt is not None:
         step_i += 1
@@ -170,7 +183,7 @@ def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, wr
             st2 = _get_step(args, model, optimizer, nxt[0], nxt[1], pipe, apipe)
             if st2 is not st:  # geometry changed (last partial batch without drop_last): new engine
                 st = st2
-            prefetch(st, nxt)
+            _prefetch(st, nxt, pipe, apipe)
         hist[len(pending)].copy_(stats)
         pending.append(step_i)
         nsteps += 1
@@ -188,28 +201,52 @@ def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, wr
     return totals[0] / n, totals[1] / n, totals[2] / n, 0.0, 0.0, 0.0, 0.0
 
 
+def _sharded(dataloader):
+    """True for a data-parallel test loader: one rank's contiguous shards of the global batches."""
+    return _world() > 1 and isinstance(getattr(dataloader, "batch_sampler", None), ChunkShardBatchSampler)
+
+
 def valid(args, model, device, dataloader):
     """reference main_dgl.py:168-222: eval-mode forward (BN running statistics), softmax,
-    arg-max accuracy of the fused / audio / visual heads.  The per-sample host loop becomes
-    on-device counting with one D2H at the end; `drop_last` behaviour is the loader's."""
+    arg-max accuracy of the fused / audio / visual heads.  Runs on the cached EvalStep of the batch geometry (CUDA
+    graph, the next batch prefetched on the copy stream); the correct counts accumulate on the device and are read
+    once at the end.  `drop_last` behaviour is the loader's.
+    A data-parallel test loader (parallel.ChunkShardBatchSampler: each rank evaluates its shard of every global batch)
+    is evaluated like nn.DataParallel evaluates the reference's: every rank first takes rank 0's BatchNorm running
+    statistics, and the counts are summed over the ranks, so every rank returns the accuracy over all the samples."""
     inner = getattr(model, "module", model)
     inner.args.drop = 0
-    correct = torch.zeros(3, device=device, dtype=torch.float64)
-    total = 0
     with torch.no_grad():
         model.eval()
         print(inner.args.drop)
         pipe, apipe = _pipeline_of(dataloader), _audio_pipeline_of(dataloader)
-        for spec, image, label in dataloader:
-            spec, image, label = spec.to(device), image.to(device), label.to(device)
-            if pipe is not None:
-                image = pipe(image.reshape(-1, 6))
-            if apipe is not None:
-                spec = apipe(spec)
-            out, out_a, out_v = model(spec.unsqueeze(1).float(), image.float())
-            for i, o in enumerate((out, out_a, out_v)):  # softmax is monotone: arg-max of the logits
-                correct[i] += (o.argmax(1) == label).sum()
-            total += label.shape[0]
+        sharded = _sharded(dataloader)
+        if sharded:
+            broadcast_running_stats(inner)
+        counts = eval_counts(inner, next(inner.parameters()).device)
+        counts.zero_()
+        total = 0
+        it = iter(dataloader)
+        nxt = next(it, None)
+        ev = None
+
+        def get(batch):
+            spec_hw, thw = _geometry(batch[0], batch[1], pipe, apipe)
+            return get_eval_step(inner, batch[2].shape[0], spec_hw, thw)
+        if nxt is not None:
+            ev = get(nxt)
+            _prefetch(ev, nxt, pipe, apipe)
+        while nxt is not None:
+            ev.run()
+            total += ev.rows
+            nxt = next(it, None)
+            if nxt is not None:
+                ev = get(nxt)
+                _prefetch(ev, nxt, pipe, apipe)
+        res = torch.cat([counts, torch.tensor([total], device=counts.device, dtype=torch.int64)])
+        if sharded:
+            torch.distributed.all_reduce(res)
+        res = res.tolist()  # the one D2H of the evaluation
     inner.args.drop = 1
-    acc = (correct / max(total, 1)).tolist()
-    return acc[0], acc[1], acc[2]
+    n = max(res[3], 1)
+    return res[0] / n, res[1] / n, res[2] / n

@@ -254,6 +254,24 @@ int gdl_dgl_head_gated(const float* a, const float* v, const float* Wx, const fl
  * scratch f32 [B].  Used by the gated/film heads, whose layers run through gdl_linear_*. */
 int gdl_softmax_ce(const float* logits, const int64_t* labels, float loss_scale, float grad_scale,
                    float* loss_out, float* dlogits, float* scratch, int B, int n, gdl_stream_t s);
+/* Eval-mode head (reference valid(), main_dgl.py:168-222), one CTA per sample, from the bf16 NHWC layer-4 maps:
+ *   fa bf16 [B][Ga][512] (audio, Ga = h*w), fv bf16 [B][Gv][512] (visual, Gv = T*h*w), both 16-byte aligned;
+ *   global average pooling, then the three logit sets (out, out_a, out_v):
+ *     kind 0 = concat: Wx = fc_out.weight, Wy = Wx + 512, ldw = 1024, bias bx (by unused);
+ *     kind 1 = sum   : Wx = fc_x.weight, Wy = fc_y.weight, ldw = 512, biases bx, by;
+ *     kind 2 = gated : Wx/bx = fc_x, Wy/by = fc_y (512 x 512), Wo/bo = fc_out; out = fc_out(sig(hx) hy) with
+ *                      x_gate != 0, fc_out(sig(hy) hx) otherwise; out_a = fc_out(sig(hx) hx), out_v likewise;
+ *     kind 3 = pooling only (the FiLM head continues with its GEMMs and gdl_eval_count);
+ *   the arg-max of every row (lowest index on ties, NaN largest like torch.argmax) and, when labels != NULL,
+ *   counts[h] += number of rows whose arg-max equals the label (int64 [3], device; a label < 0 never counts).
+ *   a_out / v_out f32 [B][512] pooled features (may be NULL except for kind 3), logits f32 [3][B][n] (may be NULL);
+ *   n <= 512. */
+int gdl_eval_head(int kind, const void* fa, int Ga, const void* fv, int Gv, const float* Wx, const float* Wy,
+                  int ldw, const float* bx, const float* by, const float* Wo, const float* bo, int x_gate,
+                  const int64_t* labels, float* a_out, float* v_out, float* logits, int64_t* counts, int B, int n,
+                  gdl_stream_t s);
+/* counts[h] += #{b : argmax(logits[h][b][:]) == labels[b]} for h = 0, 1, 2; logits f32 [3][B][n]. */
+int gdl_eval_count(const float* logits, const int64_t* labels, int64_t* counts, int B, int n, gdl_stream_t s);
 /* Gated-head elementwise pieces (reference models/fusion_modules.py:230-250). */
 int gdl_gated_fwd(const float* hx, const float* hy, float* m_out, float* m_x, float* m_y,
                   int64_t numel, gdl_stream_t s);

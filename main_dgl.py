@@ -143,8 +143,16 @@ def main(argv=None):
     else:
         train_loader = DataLoader(train_dataset, batch_size=per_rank, shuffle=True, num_workers=8, pin_memory=True,
                                   drop_last=True)
-    test_loader = DataLoader(test_dataset, batch_size=per_rank, shuffle=False, num_workers=8, pin_memory=True,
-                             drop_last=True)  # the reference drops the test tail too (main_dgl.py:287-288)
+    if world > 1:
+        # the reference's test loader (batch_size = G, drop_last) whose batches DataParallel splits over the GPUs:
+        # rank r evaluates contiguous chunk r of every global batch and valid() sums the counts over the ranks
+        from gdl_b200.parallel import ChunkShardBatchSampler
+        test_loader = DataLoader(test_dataset, batch_sampler=ChunkShardBatchSampler(
+            torch.utils.data.SequentialSampler(test_dataset), args.batch_size, rank, world), num_workers=8,
+            pin_memory=True)
+    else:
+        test_loader = DataLoader(test_dataset, batch_size=per_rank, shuffle=False, num_workers=8, pin_memory=True,
+                                 drop_last=True)  # the reference drops the test tail too (main_dgl.py:287-288)
 
     start_epoch, best_acc = 0, 0.0
     if args.resume and args.train:
