@@ -207,6 +207,7 @@ class EncoderEngine:
         self.own_stats = True
         self._readers = {}
         self._eval_key_folded = None
+        self.x_in = None  # the staged bf16 stem input (stage_input), allocated on first use
         self._plan_backward()
         self.repack()
 
@@ -214,6 +215,23 @@ class EncoderEngine:
         u = _ConvBN(self, name, conv, bn, N, Hi, Wi, ci_store, relu)
         self.units.append(u)
         return u
+
+    # ------------------------------------------------------------------ input and pooling
+    def stage_input(self, src, B):
+        """fp32 batch of B rows ([B, F, Tt] spectrograms or [B, 3, T, H, W] frames) -> the engine's own bf16
+        space-to-depth stem input, which forward / backward read when they are given none (gdl_stem_layout: the
+        per-frame reshape of reference backbone.py:162-164 and main_dgl.py:100)."""
+        if self.x_in is None:
+            self.x_in = torch.empty(self.input_shape, device=self.device, dtype=torch.bfloat16)
+        ops.stem_layout(src, self.x_in, B, self.stem.ci_real, self.N // B, self.H, self.W)
+
+    def gap_fwd(self, feat, out, B):
+        """Global average pool of the layer4 map over (frames, h, w) (reference models/basic_model.py:73-82)."""
+        ops.gap_fwd(feat, out, B, self.N // B * self.Hf * self.Wf, 512)
+
+    def gap_bwd(self, dout, B):
+        """The pooling's backward: dout [B, 512] -> g_feat, the gradient the backward consumes."""
+        ops.gap_bwd(dout, self.g_feat, B, self.N // B * self.Hf * self.Wf, 512)
 
     # ------------------------------------------------------------------ weights
     def repack(self):
@@ -267,9 +285,10 @@ class EncoderEngine:
         ops.conv_pack_weights_multi(*self._pack_table_eval)
         self._eval_key_folded = key
 
-    def forward_eval(self, x16):
+    def forward_eval(self, x16=None):
         """Eval-mode forward with folded BatchNorm: stem conv -> (+shift, ReLU, max-pool) -> 8 blocks of three fused
-        conv kernels (reference backbone.py:52-68 with model.eval())."""
+        conv kernels (reference backbone.py:52-68 with model.eval()).  x16: default the staged input."""
+        x16 = self.x_in if x16 is None else x16
         self.fold_eval()
         s = self.stem
         ops.sweep(0)
@@ -292,13 +311,14 @@ class EncoderEngine:
         """The running-statistics pair a training-mode forward updates: the module's own, or the sink."""
         return (bn.running_mean, bn.running_var) if self.own_stats else self.stats_sink
 
-    def forward(self, x16, training=True, own_stats=True):
-        """x16: bf16 space-to-depth input [N,Hp,Wp,16] -> bf16 [N,Hf,Wf,512] (the layer4 map,
-        reference backbone.py:175-181).  training=False: eval mode, BatchNorm folded into the convolutions.
+    def forward(self, x16=None, training=True, own_stats=True):
+        """x16: bf16 space-to-depth input [N,Hp,Wp,16] (default: the staged input) -> bf16 [N,Hf,Wf,512] (the
+        layer4 map, reference backbone.py:175-181).  training=False: eval mode, BatchNorm folded into the convolutions.
         own_stats=False: batch statistics as usual, but the BatchNorm running buffers stay bit-identical (the
         choice is fixed into a CUDA graph that captures the call)."""
         if not training:
             return self.forward_eval(x16)
+        x16 = self.x_in if x16 is None else x16
         self.own_stats = own_stats
         s = self.stem
         u = s.forward(self, x16)  # stem conv + BN + ReLU + max-pool -> pool_y
@@ -397,11 +417,13 @@ class EncoderEngine:
                     out += [u.conv.weight, u.bn.weight, u.bn.bias]
         return out
 
-    def backward(self, x16, part=None):
+    def backward(self, x16=None, part=None):
         """Consumes self.g_feat (grad wrt the layer4 map, bf16) and writes every parameter
-        gradient of the encoder into p.grad (overwrite).  x16 is the stem input of the forward.
+        gradient of the encoder into p.grad (overwrite).  x16 is the stem input of the forward (default: the staged
+        input).
         part=None runs the whole backward; part=0 only layer4 + layer3 (after which the gradients of
         late_parameters() are final and their all-reduce can start), part=1 the rest (layer2, layer1, stem)."""
+        x16 = self.x_in if x16 is None else x16
         self._readers = {}
         chain = list(zip(reversed(self.blocks), self.bwd_plan, reversed(self._block_inputs())))
         if part == 0:

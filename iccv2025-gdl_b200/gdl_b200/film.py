@@ -85,33 +85,55 @@ class FilmChunkBuffers:
     def refresh(self, W1):
         ops.transpose_f32_to_bf16(W1, self.W1t, D, F2)
 
+    def forward(self, a, v, b1):
+        """H = sum over chunks of Zt_c^T * W1t_c + b1  (rows: [a(x)v | a(x)a | v(x)v])."""
+        B = self.B
+        for c in range(D // CHUNK_I):
+            ops.film_outer_chunk(a, v, self.Zt, B, D, self.ZB, 3, self.scratch, c * FC, FC)
+            if c == 0:
+                ops.gemm_tn_f32(self.Zt, self.W1t[:FC], b1, self.H, self.ZB, D, FC, self.ws)
+            else:
+                ops.gemm_tn_f32_acc(self.Zt, self.W1t[c * FC:(c + 1) * FC], self.H, self.ZB, D, FC, self.ws)
+
 
 class FilmHead:
-    def __init__(self, fm, B, n, dev):
+    """The FiLM head of heads.fusion_head: the fused training head, the eval head and the W1t shadow refresh."""
+
+    def __init__(self, fm, B=None, n=None, dev=None):
         self.fm, self.B, self.n = fm, B, n
+        if dev is None:
+            return
         self.buf = FilmChunkBuffers(B, dev)
         z = lambda *s: torch.empty(*s, device=dev)
         self.dl = z(3, B, n)
         self.dH = z(3, B, D)   # dH_f, dH_a, dH_v
         self.sc = z(B)
         self.ones = torch.ones(B, 1, device=dev)
-        self.buf.refresh(fm.fc.weight.data)
+        self.a_pool, self.v_pool = z(B, D), z(B, D)  # pooled features of the eval head
+        self.refresh_shadows()
 
-    def refresh(self):
+    def trainable(self):
+        fm = self.fm
+        return [fm.fc.weight, fm.fc.bias, fm.fc_out.weight, fm.fc_out.bias]
+
+    def refresh_shadows(self):
         self.buf.refresh(self.fm.fc.weight.data)
 
-    def run(self, st):
+    def eval(self, ev, fa, Ga, fv, Gv):
+        """Pooling (eval_head kind 3), the forward chunks, fc_out and the correct counts."""
+        fm, b, B, n = self.fm, self.buf, self.B, self.n
+        ops.eval_head(3, fa, Ga, fv, Gv, None, None, 0, None, None, None, None, 1, None, self.a_pool, self.v_pool,
+                      None, None, B, n)
+        b.forward(self.a_pool, self.v_pool, fm.fc.bias.data)
+        for i in range(3):
+            ops.linear_fwd(b.H[i * B:(i + 1) * B], fm.fc_out.weight.data, fm.fc_out.bias.data, ev.logits[i], B, D, n)
+        ops.eval_count(ev.logits, ev.label_in, ev.counts, B, n)
+
+    def train(self, st):
         """st: the DGLStep (features, labels, logits, losses, da/dv live there)."""
         fm, b, B, n = self.fm, self.buf, self.B, self.n
         W1, b1, W2, b2 = fm.fc.weight, fm.fc.bias, fm.fc_out.weight, fm.fc_out.bias
-        nch = D // CHUNK_I
-        # forward: H = sum over chunks of Zt_c^T * W1t_c  (rows: [z | a(x)a | v(x)v])
-        for c in range(nch):
-            ops.film_outer_chunk(st.a_feat, st.v_feat, b.Zt, B, D, b.ZB, 3, b.scratch, c * FC, FC)
-            if c == 0:
-                ops.gemm_tn_f32(b.Zt, b.W1t[:FC], b1.data, b.H, b.ZB, D, FC, b.ws)
-            else:
-                ops.gemm_tn_f32_acc(b.Zt, b.W1t[c * FC:(c + 1) * FC], b.H, b.ZB, D, FC, b.ws)
+        b.forward(st.a_feat, st.v_feat, b1.data)
         for i in range(3):                                                       # logits: out, out_a, out_v
             ops.linear_fwd(b.H[i * B:(i + 1) * B], W2.data, b2.data, st.logits[i], B, D, n)
             gs = st.inv_batch if i == 0 else st.alpha * st.inv_batch
@@ -126,7 +148,7 @@ class FilmHead:
         ops.cast_pad_bf16(self.dH[1], B, self.dH[2], B, D, D, False, b.dHs, b.NG, D)
         # backward, chunk by chunk: the outer products again (L2-resident), dW1 window (Lf only), G tile and its
         # contraction with a / v (unimodal only)
-        for c in range(nch):
+        for c in range(D // CHUNK_I):
             ops.film_outer_chunk(st.a_feat, st.v_feat, b.Zt, B, D, b.ZB, 3, b.scratch, c * FC, FC)
             ops.gemm_nt_bf16(b.Zt, b.ZB, b.dHfT, b.dW1t, FC, D, b.KB)
             ops.transpose_bf16_to_f32_window(b.dW1t, W1.grad, D, FC, F2, c * FC)

@@ -6,14 +6,14 @@ three cross-entropies, truncated gradients), both encoder backwards, [gradient a
 clip_grad_norm_(40), the audio/visual gradient diagnostics, the optimizer update (SGD-momentum, Adam or Adagrad:
 gdl_b200.optim.UpdateRule), and the refresh of
 the bf16 weight shadows — as a fixed sequence of libgdl_b200.so kernels on two CUDA streams
-(audio || visual), optionally captured into one CUDA graph.  The only device->host traffic is
-one 7-float read (3 losses + norm, clip coefficient, 2 diagnostics) when the caller asks.
+(audio || visual), schedule(), whose device segments are optionally replayed as CUDA graphs.  The only
+device->host traffic is one 7-float read (3 losses + norm, clip coefficient, 2 diagnostics) when the caller asks.
 
 Gradient routing (the point of DGL, reference main_dgl.py:108-122):
     encoders  <- alpha * d(La + Lv)        (the multimodal head saw detached features)
     head      <- d(Lf)                     (the unimodal gradient of the head is wiped)
-Parameters that never receive a gradient in the reference (ConcatFusion_DGL.fc_auxi,
-GatedFusion_DGL.fc_x / fc_y — SURVEY.md §8a quirks 1-2) are left untouched: no weight decay,
+Parameters that never receive a gradient in the reference (the concat head's fc_auxi,
+the gated head's fc_x / fc_y — SURVEY.md §8a quirks 1-2) are left untouched: no weight decay,
 no momentum, exactly like torch.optim.SGD skipping `grad is None`.
 """
 import os
@@ -21,10 +21,9 @@ import os
 import torch
 
 from . import ops, parallel
-from .engine import kernel_writes, note_writes
-from .autograd import to_nhwc8  # noqa: F401  (re-export for callers)
 from .basic_model import AVClassifier_DGL
-from .fusion_modules import ConcatFusion_DGL, FiLM_DGL, GatedFusion_DGL, SumFusion_DGL
+from .engine import kernel_writes, note_writes
+from .heads import fusion_head
 from .optim import UpdateRule
 
 _SEG_ALIGN = 64  # floats; keeps every tensor 256-byte aligned inside the arenas
@@ -44,17 +43,54 @@ def _pad(n):
     return (n + _SEG_ALIGN - 1) // _SEG_ALIGN * _SEG_ALIGN
 
 
-def head_trainable(fm):
-    """Head parameters that receive a gradient from Lf (everything else stays grad-less)."""
-    if isinstance(fm, ConcatFusion_DGL):
-        return [fm.fc_out.weight, fm.fc_out.bias]
-    if isinstance(fm, SumFusion_DGL):
-        return [fm.fc_x.weight, fm.fc_x.bias, fm.fc_y.weight, fm.fc_y.bias]
-    if isinstance(fm, GatedFusion_DGL):
-        return [fm.fc_out.weight, fm.fc_out.bias]
-    if isinstance(fm, FiLM_DGL):
-        return [fm.fc.weight, fm.fc.bias, fm.fc_out.weight, fm.fc_out.bias]
-    raise NotImplementedError('Incorrect fusion method: {}!'.format(type(fm).__name__))
+class GraphCache(dict):
+    """CUDA graphs by key."""
+
+    def capture(self, key, enqueue):
+        """The graph of `key`; under a new key, first capture what enqueue() launches (capture does not execute it)."""
+        if key not in self:
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, capture_error_mode=_CAPTURE_MODE):
+                enqueue()
+            self[key] = g
+        return self[key]
+
+
+# The segments of a global step: the DEVICE ones are capturable, the others (the stem layout of replica k's rows, the
+# NCCL calls) always run eagerly.
+DEVICE = ("replica0", "replica", "last", "update")
+
+
+def schedule(replicas, world_size, overlap):
+    """The global step (DESIGN.md §5) as an ordered list of (name, argument) segments:
+        ("inputs", k)           eager: the stem layout of replica k's rows (k = 0 first consumes a prefetched batch)
+        ("replica0", None)      replica 0's compute (it owns the BatchNorm running statistics), then acc <- grad
+        ("replica", None)       replica 1 .. R-2: compute, then acc += grad
+        ("last", part)          the last replica's compute, then grad += acc: whole (part None), or with the two
+                                all-reduce buckets of `overlap` forward + layer4/layer3 backward (0) and the rest (1)
+        ("allreduce", None), ("allreduce_late", None), ("allreduce_finish", None)     NCCL
+        ("update", None)        clip statistics, diagnostics, optimizer update, bf16 shadow refresh"""
+    seq = [("inputs", 0)]
+    for k in range(1, replicas):
+        seq += [("replica0" if k == 1 else "replica", None), ("inputs", k)]
+    if overlap and world_size > 1:
+        seq += [("last", 0), ("allreduce_late", None), ("last", 1), ("allreduce_finish", None)]
+    else:
+        seq += [("last", None)] + ([("allreduce", None)] if world_size > 1 else [])
+    return seq + [("update", None)]
+
+
+def graph_runs(seq):
+    """`seq` cut into runs: an eager segment alone, or a maximal run of consecutive device segments, which a graph
+    step replays as one CUDA graph cached under the run itself (so replicas 1 .. R-2 share one graph)."""
+    runs = []
+    for seg in seq:
+        if seg[0] in DEVICE and runs and runs[-1][-1][0] in DEVICE:
+            runs[-1] += (seg,)
+        else:
+            runs.append((seg,))
+    return runs
 
 
 class ParamArena:
@@ -65,7 +101,7 @@ class ParamArena:
     Adagrad `sum`.  `state_buffers` pairs each with its key in torch's `optimizer.state[p]`."""
 
     def __init__(self, model, device, rule=None):
-        groups = [(2, head_trainable(model.fusion_module)),
+        groups = [(2, fusion_head(model.fusion_module).trainable()),
                   (0, list(model.audio_net.parameters())),
                   (1, list(model.visual_net.parameters()))]
         self.params, seg_end, seg_group, seg_inv = [], [], [], []
@@ -120,7 +156,7 @@ class ParamArena:
     def owns(self, model, device):
         """True while every parameter of `model` still is the view into this arena that __init__ made (a
         `model.to(...)`, `load_state_dict(assign=True)` or a changed trainable set breaks that)."""
-        groups = head_trainable(model.fusion_module) + list(model.audio_net.parameters()) + \
+        groups = fusion_head(model.fusion_module).trainable() + list(model.audio_net.parameters()) + \
             list(model.visual_net.parameters())
         if self.param.device != device or len(groups) != len(self.params):
             return False
@@ -174,18 +210,20 @@ class InputStage:
         self.ready = [torch.cuda.Event() for _ in range(2)]
         self.free = [torch.cuda.Event() for _ in range(2)]
 
-    def current(self):
-        return self.sets[self.cur]
-
-    def acquire(self, stream):
-        """Make `stream` wait for a prefetched batch and make it the current set."""
-        if self.pending is not None:
-            stream.wait_event(self.ready[self.pending])
+    def stage_rows(self, k, parts, B, enc_a, enc_v, label_in):
+        """Eager, on the current stream: rows [k*B, (k+1)*B) of the current set -> both encoders' stem inputs
+        (stage_input) and `label_in`.  k = 0 first makes a prefetched batch the current set; after slice k = parts - 1
+        the set is free for the next prefetch."""
+        main = torch.cuda.current_stream()
+        if k == 0 and self.pending is not None:
+            main.wait_event(self.ready[self.pending])
             self.cur, self.pending = self.pending, None
-
-    def release(self, stream):
-        """The kernels enqueued on `stream` so far are the last readers of the current set."""
-        self.free[self.cur].record(stream)
+        spec, image, label = (t[k * B:(k + 1) * B] for t in self.sets[self.cur])
+        enc_a.stage_input(spec, B)
+        enc_v.stage_input(image, B)
+        label_in.copy_(label, non_blocking=True)
+        if k == parts - 1:
+            self.free[self.cur].record(main)
 
     def load(self, spec, image, label):
         """Copy a batch (host or device tensors) into the current set on the current stream."""
@@ -285,25 +323,19 @@ class DGLStep:
             self.enc_a = model.audio_net.engine(B, self.F_, self.Tt)
             self.enc_v = model.visual_net.engine(B * T, self.H, self.W)
         # Inputs: two staging sets (fp32 batch as the reference's DataLoader delivers it).  The layout kernels
-        # read the current set OUTSIDE the captured graph and write the fixed-address bf16 stem inputs a8/v8, so
+        # read the current set OUTSIDE the captured graphs and write the encoders' fixed-address bf16 stem inputs, so
         # the next batch can be copied H2D on a side stream into the other set while this step computes.
         self.stage = InputStage(dev, self.rows, spec_hw, image_thw)
-        self.copy_stream = self.stage.copy_stream
         self.label_in = torch.zeros(B, device=dev, dtype=torch.int64)  # fixed address: read inside the graph
-        self.a8 = self.v8 = None
-        if not self.check_fp32:
-            self.a8 = torch.empty(self.enc_a.input_shape, device=dev, dtype=torch.bfloat16)  # space-to-depth
-            self.v8 = torch.empty(self.enc_v.input_shape, device=dev, dtype=torch.bfloat16)
         D = 512
         self.a_feat, self.v_feat = torch.empty(B, D, device=dev), torch.empty(B, D, device=dev)
         self.da, self.dv = torch.empty(B, D, device=dev), torch.empty(B, D, device=dev)
         self.logits = torch.empty(3, B, self.n, device=dev)
-        self.head_scratch = torch.empty(ops.head_scratch_floats(B, self.n) + 64, device=dev)
         self.stats = torch.zeros(8, device=dev)  # [0:3] losses Lf,La,Lv  [4:8] norm, coef, audio, visual
         self.losses = self.arena.grad[self.arena.numel:self.arena.numel + 3]
         self._bn_counters = [m.num_batches_tracked for m in model.modules()
                              if isinstance(m, torch.nn.BatchNorm2d)]
-        self._init_head()
+        self.head = fusion_head(model.fusion_module, B, self.n, dev)
         # GDL_STREAM_PRIO: 0 = equal priorities, 1 = the visual encoder's stream (the long chain: 3x the audio work) is
         # high priority so its kernels' CTAs are placed first and the audio kernels fill the gaps, 2 = the reverse
         prio = int(os.environ.get("GDL_STREAM_PRIO", "1"))  # measured: 20.40 / 20.09 ms vs 20.48 / 20.40 ms per step, e2e +1.7 %
@@ -311,15 +343,12 @@ class DGLStep:
         self.stream_v = torch.cuda.Stream(dev, priority=-1 if prio == 1 else 0)
         self.steps_done = 0
         self.momentum_loaded = False  # set by train.adopt_momentum when a checkpoint's buffers were copied in
-        self._graph = None
-        self._graph_b = None
-        self._graph_update = None
-        self._graph_first = None  # replicas > 1: replica 0 (owns the running statistics), then acc <- grad
-        self._graph_mid = None    # replicas > 2: replicas 1 .. R-2, acc += grad
+        self.graphs = GraphCache()  # the device runs of the schedule, captured for self._graph_lr
         self._graph_lr = None
         self.launches_per_step = None
         # gradient buckets (views of the gradient arena; arena order: head | audio | visual)
         self.overlap = AR_OVERLAP and world_size > 1
+        self._runs = graph_runs(schedule(R, world_size, self.overlap))
         self._buckets = None
         if self.overlap:
             ar = self.arena
@@ -335,181 +364,81 @@ class DGLStep:
         else:
             self._acc_ranges = {"all": [(0, end)]}
 
-    # ------------------------------------------------------------------ heads
-    def _init_head(self):
-        fm, B, n, dev = self.model.fusion_module, self.B, self.n, self.device
-        self.film = None
-        if isinstance(fm, GatedFusion_DGL):
-            self.gated_scratch = torch.empty(ops.gated_head_scratch_floats(B, n) + 64, device=dev)
-        elif isinstance(fm, FiLM_DGL):
-            from .film import FilmHead
-            self.film = FilmHead(fm, B, n, dev)
-
-    def _head(self):
-        fm, B, n, D = self.model.fusion_module, self.B, self.n, 512
-        if isinstance(fm, ConcatFusion_DGL):
-            W, b = fm.fc_out.weight, fm.fc_out.bias
-            ops.dgl_head_linear(0, self.a_feat, self.v_feat, W.data_ptr(), W.data_ptr() + 4 * D, 2 * D,
-                                b.data, None, self.label_in, self.alpha, self.inv_batch, self.logits,
-                                self.losses, self.da, self.dv, W.grad.data_ptr(), W.grad.data_ptr() + 4 * D,
-                                2 * D, b.grad, None, self.head_scratch, B, D, n)
-        elif isinstance(fm, SumFusion_DGL):
-            ops.dgl_head_linear(1, self.a_feat, self.v_feat, fm.fc_x.weight.data_ptr(),
-                                fm.fc_y.weight.data_ptr(), D, fm.fc_x.bias.data, fm.fc_y.bias.data,
-                                self.label_in, self.alpha, self.inv_batch, self.logits, self.losses,
-                                self.da, self.dv, fm.fc_x.weight.grad.data_ptr(),
-                                fm.fc_y.weight.grad.data_ptr(), D, fm.fc_x.bias.grad, fm.fc_y.bias.grad,
-                                self.head_scratch, B, D, n)
-        elif isinstance(fm, GatedFusion_DGL):
-            self._head_gated(fm)
+    # ------------------------------------------------------------------ the segments of schedule()
+    def _enqueue(self, seg):
+        """Enqueue one segment on the current stream (+ the two encoder streams).  Every segment reads the streams,
+        lr and the rest of the step's state when it is enqueued."""
+        name, arg = seg
+        if name == "inputs":
+            self.stage.stage_rows(arg, self.replicas, self.B, self.enc_a, self.enc_v, self.label_in)
+        elif name in ("replica0", "replica"):
+            self._enqueue_compute(own_stats=name == "replica0")
+            ops.grad_accumulate(self.acc, self.arena.grad, self.arena.numel + 3, name == "replica")
+        elif name == "last":
+            self._enqueue_compute(arg, own_stats=self.replicas == 1)
+            if self.replicas > 1:  # part 0: the late bucket, so its all-reduce carries the sum over the replicas
+                for a, b in self._acc_ranges["all" if arg is None else ("late", "early")[arg]]:
+                    ops.grad_accumulate(self.arena.grad[a:b], self.acc[a:b], b - a, True)
+        elif name == "allreduce":
+            # each rank scaled its CE by 1/B_global, so a plain SUM reproduces the reference's
+            # full-batch mean (DataParallel gathers logits, main_dgl.py:102-104); BN stays per replica.
+            # The 3 losses ride in the tail of the gradient arena (one collective per step).
+            torch.distributed.all_reduce(self.arena.grad, group=self.pg)
+        elif name == "allreduce_late":
+            # bucket 1 (layer3 + layer4 of both encoders + the losses), asynchronously: NCCL's stream waits for what
+            # the current stream has enqueued so far and then runs beside the backward of layer2 / layer1 / stem
+            self._works = parallel.allreduce_async(self._buckets["late"], self.pg)
+        elif name == "allreduce_finish":
+            # join bucket 1, then bucket 2 (head + the early layers, 6 % of the bytes) on the critical path
+            parallel.allreduce_finish(self._works, self._buckets["early"], self.pg)
         else:
-            self.film.run(self)
-
-    def _head_gated(self, fm):
-        """reference fusion_modules.py:230-250 with the DGL routing, one fused pass (csrc/head.cu
-        dgl_gated_sample/param_kernel): fc_out <- Lf; a, v <- alpha*La/Lv through fc_out, the gates and fc_x / fc_y;
-        fc_x / fc_y themselves get no gradient."""
-        Wo, bo = fm.fc_out.weight, fm.fc_out.bias
-        ops.dgl_head_gated(self.a_feat, self.v_feat, fm.fc_x.weight.data, fm.fc_x.bias.data, fm.fc_y.weight.data,
-                           fm.fc_y.bias.data, Wo.data, bo.data, self.label_in, self.alpha, self.inv_batch, self.logits,
-                           self.losses, self.da, self.dv, Wo.grad, bo.grad, self.gated_scratch, self.B, 512, self.n)
-
-    # ------------------------------------------------------------------ the step
-    @property
-    def spec_in(self):
-        return self.stage.current()[0]
-
-    @property
-    def image_in(self):
-        return self.stage.current()[1]
-
-    def _enqueue_inputs(self, k=0):
-        """Eager, outside the graph: consume the prefetched batch if there is one (k = 0), then the per-frame
-        reshape + fp32->bf16 space-to-depth layout of both modalities (reference backbone.py:162-164,
-        main_dgl.py:100) of replica k's rows of the current staging set into the fixed-address stem inputs."""
-        B, T = self.B, self.T
-        main = torch.cuda.current_stream()
-        if k == 0:
-            self.stage.acquire(main)
-        spec, image, label = (t[k * B:(k + 1) * B] for t in self.stage.current())
-        if self.check_fp32:
-            self.enc_a.stage_input(spec, B)
-            self.enc_v.stage_input(image, B)
-        else:
-            ops.stem_layout(spec, self.a8, B, 1, 1, self.F_, self.Tt)
-            ops.stem_layout(image, self.v8, B, 3, T, self.H, self.W)
-        self.label_in.copy_(label, non_blocking=True)
-        if k == self.replicas - 1:
-            self.stage.release(main)
-
-    def _enqueue(self, lr, first):
-        """The last replica of the step (with replicas == 1 its only one), the all-reduce and the update."""
-        if self.overlap:
-            self._enqueue_last(part=0)
-            works = self._allreduce_late()
-            self._enqueue_last(part=1)
-            self._allreduce_finish(works)
-        else:
-            self._enqueue_last()
-            if self.world_size > 1:
-                self._allreduce()
-        self._enqueue_update(lr, first)
-
-    def _enqueue_last(self, part=None):
-        """Compute of the last replica; with replicas > 1 then grad += acc over the part's range (part 0: the late
-        bucket, so its all-reduce carries the sum over the replicas)."""
-        self._enqueue_compute(part, own_stats=self.replicas == 1)
-        if self.replicas > 1:
-            key = "all" if part is None else ("late", "early")[part]
-            for a, b in self._acc_ranges[key]:
-                ops.grad_accumulate(self.arena.grad[a:b], self.acc[a:b], b - a, True)
-
-    def _enqueue_replica(self, k):
-        """Replica k < replicas - 1: compute, then acc <- grad (k = 0) or acc += grad, over the arena + 3 losses.
-        Only replica 0 updates the BatchNorm running statistics."""
-        self._enqueue_compute(own_stats=k == 0)
-        n = self.arena.numel + 3
-        ops.grad_accumulate(self.acc, self.arena.grad, n, k > 0)
+            self._enqueue_update()
 
     def _enqueue_compute(self, part=None, own_stats=True):
         """Forward + head + backward on the current stream (+ the two encoder streams).
         part=0: forward, head and the backward of layer4 + layer3; part=1: the rest of the backward.
         own_stats=False: the forward leaves the BatchNorm running statistics untouched."""
-        B, T = self.B, self.T
+        B = self.B
         main = torch.cuda.current_stream()
         sa, sv = self.stream_a, self.stream_v
         if part != 1:
             sa.wait_stream(main)
             sv.wait_stream(main)
             with torch.cuda.stream(sa):
-                fa = self.enc_a.forward(self.a8, own_stats=own_stats)
-                self._gap_fwd(self.enc_a, fa, self.a_feat, 1)
+                self.enc_a.gap_fwd(self.enc_a.forward(own_stats=own_stats), self.a_feat, B)
             with torch.cuda.stream(sv):
-                fv = self.enc_v.forward(self.v8, own_stats=own_stats)
-                self._gap_fwd(self.enc_v, fv, self.v_feat, T)
+                self.enc_v.gap_fwd(self.enc_v.forward(own_stats=own_stats), self.v_feat, B)
             main.wait_stream(sa)
             main.wait_stream(sv)
-            self._head()
+            self.head.train(self)
         sa.wait_stream(main)
         sv.wait_stream(main)
         with torch.cuda.stream(sa):
             if part != 1:
-                self._gap_bwd(self.enc_a, self.da, 1)
-            self.enc_a.backward(self.a8, part)
+                self.enc_a.gap_bwd(self.da, B)
+            self.enc_a.backward(part=part)
         with torch.cuda.stream(sv):
             if part != 1:
-                self._gap_bwd(self.enc_v, self.dv, T)
-            self.enc_v.backward(self.v8, part)
+                self.enc_v.gap_bwd(self.dv, B)
+            self.enc_v.backward(part=part)
         main.wait_stream(sa)
         main.wait_stream(sv)
 
-    def _gap_fwd(self, enc, feat, out, frames):
-        """global average pool over (frames, h, w) (reference models/basic_model.py:73-82)."""
-        if self.check_fp32:
-            enc.gap_fwd(feat, out, self.B)
-        else:
-            ops.gap_fwd(feat, out, self.B, frames * enc.Hf * enc.Wf, 512)
-
-    def _gap_bwd(self, enc, dout, frames):
-        if self.check_fp32:
-            enc.gap_bwd(dout, self.B)
-        else:
-            ops.gap_bwd(dout, enc.g_feat, self.B, frames * enc.Hf * enc.Wf, 512)
-
-    def _allreduce(self):
-        # each rank scaled its CE by 1/B_global, so a plain SUM reproduces the reference's
-        # full-batch mean (DataParallel gathers logits, main_dgl.py:102-104); BN stays per replica.
-        # The 3 losses ride in the tail of the gradient arena (one collective per step).
-        torch.distributed.all_reduce(self.arena.grad, group=self.pg)
-
-    def _allreduce_late(self):
-        """Bucket 1 (layer3 + layer4 of both encoders + the losses): issued asynchronously — NCCL's stream waits
-        for what the current stream has enqueued so far (the backward of those layers) and then runs beside
-        the kernels enqueued next (the backward of layer2 / layer1 / stem)."""
-        return parallel.allreduce_async(self._buckets["late"], self.pg)
-
-    def _allreduce_finish(self, works):
-        """Join bucket 1, then bucket 2 (head + the early layers, 6 % of the bytes) on the critical path."""
-        parallel.allreduce_finish(works, self._buckets["early"], self.pg)
-
-    def _enqueue_update(self, lr, first):
+    def _enqueue_update(self):
         """Clip statistics + diagnostics + optimizer update + bf16 shadow refresh (after the all-reduce)."""
-        ar, r = self.arena, self.rule
+        ar, r, lr = self.arena, self.rule, self.lr
         ops.grad_stats(ar.grad, ar.numel, ar.seg_end, ar.seg_group, ar.seg_inv, ar.nseg, self.max_norm,
                        ar.scratch, self.stats[4:8])
         if r.kind == "sgd":
             ops.sgd_momentum(ar.param, ar.grad, ar.momentum, ar.numel, lr, self.mu, self.wd,
-                             first and not self.momentum_loaded, self.stats[4:8])
+                             self.steps_done == 0 and not self.momentum_loaded, self.stats[4:8])
         elif r.kind == "adam":
             ops.adam(ar.param, ar.grad, ar.exp_avg, ar.exp_avg_sq, ar.step_state, ar.numel, lr, r.betas[0], r.betas[1],
                      r.eps, self.wd, self.stats[4:8])
         else:
             ops.adagrad(ar.param, ar.grad, ar.sum, ar.step_state, ar.numel, lr, r.lr_decay, r.eps, self.wd,
                         self.stats[4:8])
-        self.enc_a.repack()
-        self.enc_v.repack()
-        if self.film is not None:
-            self.film.refresh()
+        self.refresh_shadows()
         self.stats[0:3].copy_(self.losses)
         torch._foreach_add_(self._bn_counters, 1)
 
@@ -518,8 +447,7 @@ class DGLStep:
         the same model — a different batch geometry — or a load_state_dict changed them)."""
         self.enc_a.repack()
         self.enc_v.repack()
-        if self.film is not None:
-            self.film.refresh()
+        self.head.refresh_shadows()
 
     def load_inputs(self, spec, image, label):
         """Copy a batch (host or device tensors of the reference contract) into the current staging set,
@@ -546,63 +474,24 @@ class DGLStep:
             self.lr = lr
         if spec is not None:
             self.load_inputs(spec, image, label)
-        first = self.steps_done == 0
-        n0 = ops.LAUNCHES
-        self._enqueue_inputs()
-        if first or not self.use_graph:
-            for k in range(1, self.replicas):
-                self._enqueue_replica(k - 1)
-                self._enqueue_inputs(k)
-            self._enqueue(self.lr, first)
-            self.launches_per_step = ops.LAUNCHES - n0  # kernels of libgdl_b200.so per (global) step
-        else:
-            if self._graph is None or self._graph_lr != self.lr:
-                torch.cuda.synchronize()
-                if self.world_size == 1:
-                    self._graph = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(self._graph, capture_error_mode=_CAPTURE_MODE):
-                        self._enqueue(self.lr, False)
-                    self._graph_update = None
-                else:
-                    # NCCL stays outside the captured regions: graph(compute) -> all-reduce -> graph(update), or with
-                    # the overlapped buckets graph(fwd + late bwd) -> [NCCL bucket 1 || graph(early bwd)] ->
-                    # NCCL bucket 2 -> graph(update)
-                    self._graph = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(self._graph, capture_error_mode=_CAPTURE_MODE):
-                        self._enqueue_last(part=0 if self.overlap else None)
-                    self._graph_b = None
-                    if self.overlap:
-                        self._graph_b = torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(self._graph_b, capture_error_mode=_CAPTURE_MODE):
-                            self._enqueue_last(part=1)
-                    self._graph_update = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(self._graph_update, capture_error_mode=_CAPTURE_MODE):
-                        self._enqueue_update(self.lr, False)
-                # replicas before the last: one graph for replica 0, one shared by replicas 1 .. R-2 (the eager
-                # input layout of the next replica runs between the replays)
-                self._graph_first = self._graph_mid = None
-                for k in range(min(self.replicas - 1, 2)):
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g, capture_error_mode=_CAPTURE_MODE):
-                        self._enqueue_replica(k)
-                    if k == 0:
-                        self._graph_first = g
-                    else:
-                        self._graph_mid = g
+        eager = self.steps_done == 0 or not self.use_graph
+        if not eager:
+            if self._graph_lr != self.lr:
+                self.graphs.clear()
                 self._graph_lr = self.lr
-                # capture does not execute: the replays below run this step
-            for k in range(1, self.replicas):
-                (self._graph_first if k == 1 else self._graph_mid).replay()
-                self._enqueue_inputs(k)
-            self._graph.replay()
-            if self._graph_b is not None:
-                works = self._allreduce_late()
-                self._graph_b.replay()
-                self._allreduce_finish(works)
-                self._graph_update.replay()
-            elif self._graph_update is not None:
-                self._allreduce()
-                self._graph_update.replay()
+            for run in self._runs:
+                if run[0][0] in DEVICE:
+                    self.graphs.capture(run, lambda run=run: [self._enqueue(seg) for seg in run])
+            # capture does not execute: the replays below run this step
+        n0 = ops.LAUNCHES
+        for run in self._runs:
+            if eager or run[0][0] not in DEVICE:
+                for seg in run:
+                    self._enqueue(seg)
+            else:
+                self.graphs[run].replay()
+        if eager:
+            self.launches_per_step = ops.LAUNCHES - n0  # kernels of libgdl_b200.so per (global) step
         self.steps_done += 1
         self.arena.steps += 1
         for m in (self.model.audio_net, self.model.visual_net, self.model.fusion_module):
@@ -617,10 +506,11 @@ class DGLStep:
 
 # ---------------------------------------------------------------------------------------------------- evaluation
 def _eval_resources(model, rows, spec_hw, image_thw):
-    """(b, audio engine, visual engine, training step or None) that an EvalStep of `rows` rows runs on.  When a
-    training step of this geometry has a per-replica batch b dividing `rows` (with --dp_replicas the step's rows are
-    R_local * b), evaluation runs in sub-batches of b on the training step's own engines, so nothing is evicted or
-    rebuilt and no second set of activation buffers is allocated.  Otherwise the modules' engine cache serves `rows`."""
+    """(b, audio engine, visual engine, head or None) that an EvalStep of `rows` rows runs on.  When a training step
+    of this geometry has a per-replica batch b dividing `rows` (with --dp_replicas the step's rows are R_local * b),
+    evaluation runs in sub-batches of b on the training step's own engines and head, so nothing is evicted or rebuilt
+    and no second set of activation buffers (or FiLM weight shadow) is allocated.  Otherwise the modules' engine cache
+    serves `rows`."""
     steps = list(getattr(model, "_gdl_steps", {}).values())
     cur = getattr(model, "_gdl_step", None)
     if cur is not None and cur not in steps:
@@ -628,7 +518,7 @@ def _eval_resources(model, rows, spec_hw, image_thw):
     for st in sorted(steps, key=lambda st: -st.B):
         if (not st.check_fp32 and (st.F_, st.Tt) == tuple(spec_hw) and (st.T, st.H, st.W) == tuple(image_thw)
                 and rows % st.B == 0):
-            return st.B, st.enc_a, st.enc_v, st
+            return st.B, st.enc_a, st.enc_v, st.head
     (F_, Tt), (T, H, W) = spec_hw, image_thw
     return rows, model.audio_net.engine(rows, F_, Tt), model.visual_net.engine(rows * T, H, W), None
 
@@ -647,8 +537,9 @@ class EvalStep:
     (EncoderEngine.forward_eval) on the audio and visual streams, then the eval head (gdl_eval_head: pooling, the
     three logit sets, arg-max and correct counts into `counts`; FiLM: pooling, the FiLM forward GEMMs, fc_out and
     gdl_eval_count).  Everything after the layout is one CUDA graph, captured on the second call and re-captured only
-    when a head parameter moves.  The BatchNorm fold and the FiLM weight shadow are refreshed outside the graph, and
-    only when a parameter or buffer changed.  The logits of the last sub-batch stay in `logits` [3, b, n]."""
+    when a head parameter moves or the gated head's x_gate flips.  The BatchNorm fold and the FiLM weight shadow are
+    refreshed outside the graph, and only when a parameter or buffer changed.  The logits of the last sub-batch stay
+    in `logits` [3, b, n]."""
 
     def __init__(self, model, rows, spec_hw, image_thw, use_graph=True):
         model = getattr(model, "module", model)
@@ -663,58 +554,30 @@ class EvalStep:
         self.T, self.H, self.W = image_thw
         self.n = model.n_classes
         self.use_graph = use_graph
-        self.B, self.enc_a, self.enc_v, train_step = _eval_resources(model, rows, spec_hw, image_thw)
+        self.B, self.enc_a, self.enc_v, head = _eval_resources(model, rows, spec_hw, image_thw)
         self.chunks = rows // self.B
-        B, dev_kw = self.B, dict(device=dev)
+        B = self.B
         self.stage = InputStage(dev, rows, spec_hw, image_thw)
-        if train_step is not None:  # the fixed-address stem inputs of the training step: rewritten before every use
-            self.a8, self.v8 = train_step.a8, train_step.v8
-        else:
-            self.a8 = torch.empty(self.enc_a.input_shape, dtype=torch.bfloat16, **dev_kw)
-            self.v8 = torch.empty(self.enc_v.input_shape, dtype=torch.bfloat16, **dev_kw)
-        self.label_in = torch.full((B,), -1, dtype=torch.int64, **dev_kw)
-        self.logits = torch.empty(3, B, self.n, **dev_kw)
+        self.label_in = torch.full((B,), -1, dtype=torch.int64, device=dev)
+        self.logits = torch.empty(3, B, self.n, device=dev)
         self.counts = eval_counts(model, dev)
-        fm = model.fusion_module
-        self.kind = "film" if isinstance(fm, FiLM_DGL) else "gated" if isinstance(fm, GatedFusion_DGL) else \
-            "sum" if isinstance(fm, SumFusion_DGL) else "concat" if isinstance(fm, ConcatFusion_DGL) else None
-        if self.kind is None:
-            raise NotImplementedError('Incorrect fusion method: {}!'.format(type(fm).__name__))
-        self.film, self._film_key = None, None
-        if self.kind == "film":
-            from .film import FilmChunkBuffers
-            self.a_feat, self.v_feat = torch.empty(B, 512, **dev_kw), torch.empty(B, 512, **dev_kw)
-            self.film = train_step.film.buf if train_step is not None and train_step.film is not None \
-                else FilmChunkBuffers(B, dev)
+        self.head = head if head is not None else fusion_head(model.fusion_module, B, self.n, dev)
+        self._head_key = None
         self.stream_a, self.stream_v = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
         self.calls = 0
-        self._graph, self._graph_key = None, None
+        self.graphs = GraphCache()
 
     # ------------------------------------------------------------------ outside the graph
     def refresh(self):
-        """Re-fold BatchNorm into the eval weight packs and re-derive the FiLM bf16 shadow, each only if its inputs
+        """Re-fold BatchNorm into the eval weight packs and re-derive the head's bf16 shadows, each only if its inputs
         changed since the last call (torch version counters + engine.note_writes counts)."""
         self.enc_a.fold_eval()
         self.enc_v.fold_eval()
-        if self.film is not None:
-            w = self.model.fusion_module.fc.weight
-            key = (w.data_ptr(), w._version, kernel_writes(self.model.fusion_module))
-            if key != self._film_key:
-                self.film.refresh(w.data)
-                self._film_key = key
-
-    def _enqueue_inputs(self, k):
-        """Sub-batch k of the current staging set -> the fixed-address stem inputs and labels."""
-        B, T = self.B, self.T
-        main = torch.cuda.current_stream()
-        if k == 0:
-            self.stage.acquire(main)
-        spec, image, label = (t[k * B:(k + 1) * B] for t in self.stage.current())
-        ops.stem_layout(spec, self.a8, B, 1, 1, self.F_, self.Tt)
-        ops.stem_layout(image, self.v8, B, 3, T, self.H, self.W)
-        self.label_in.copy_(label, non_blocking=True)
-        if k == self.chunks - 1:
-            self.stage.release(main)
+        fm = self.model.fusion_module
+        key = tuple((p.data_ptr(), p._version) for p in fm.parameters()) + (kernel_writes(fm),)
+        if key != self._head_key:
+            self.head.refresh_shadows()
+            self._head_key = key
 
     # ------------------------------------------------------------------ the captured part
     def _enqueue(self):
@@ -723,62 +586,31 @@ class EvalStep:
         sa.wait_stream(main)
         sv.wait_stream(main)
         with torch.cuda.stream(sa):
-            fa = self.enc_a.forward_eval(self.a8)
+            fa = self.enc_a.forward_eval()
         with torch.cuda.stream(sv):
-            fv = self.enc_v.forward_eval(self.v8)
+            fv = self.enc_v.forward_eval()
         main.wait_stream(sa)
         main.wait_stream(sv)
-        fm, B, n, D = self.model.fusion_module, self.B, self.n, 512
-        Ga, Gv = self.enc_a.Hf * self.enc_a.Wf, self.T * self.enc_v.Hf * self.enc_v.Wf
-        if self.kind == "concat":
-            W = fm.fc_out.weight
-            ops.eval_head(0, fa, Ga, fv, Gv, W.data_ptr(), W.data_ptr() + 4 * D, 2 * D, fm.fc_out.bias.data, None,
-                          None, None, 1, self.label_in, None, None, self.logits, self.counts, B, n)
-        elif self.kind == "sum":
-            ops.eval_head(1, fa, Ga, fv, Gv, fm.fc_x.weight.data_ptr(), fm.fc_y.weight.data_ptr(), D, fm.fc_x.bias.data,
-                          fm.fc_y.bias.data, None, None, 1, self.label_in, None, None, self.logits, self.counts, B, n)
-        elif self.kind == "gated":
-            ops.eval_head(2, fa, Ga, fv, Gv, fm.fc_x.weight.data_ptr(), fm.fc_y.weight.data_ptr(), D, fm.fc_x.bias.data,
-                          fm.fc_y.bias.data, fm.fc_out.weight.data, fm.fc_out.bias.data, fm.x_gate, self.label_in, None,
-                          None, self.logits, self.counts, B, n)
-        else:
-            from .film import CHUNK_I, FC
-            b = self.film
-            ops.eval_head(3, fa, Ga, fv, Gv, None, None, 0, None, None, None, None, 1, None, self.a_feat, self.v_feat,
-                          None, None, B, n)
-            # H = sum over chunks of Zt_c^T W1t_c + b1 (rows: [a (x) v | a (x) a | v (x) v]), as in FilmHead.run
-            for c in range(D // CHUNK_I):
-                ops.film_outer_chunk(self.a_feat, self.v_feat, b.Zt, B, D, b.ZB, 3, b.scratch, c * FC, FC)
-                if c == 0:
-                    ops.gemm_tn_f32(b.Zt, b.W1t[:FC], fm.fc.bias.data, b.H, b.ZB, D, FC, b.ws)
-                else:
-                    ops.gemm_tn_f32_acc(b.Zt, b.W1t[c * FC:(c + 1) * FC], b.H, b.ZB, D, FC, b.ws)
-            for i in range(3):
-                ops.linear_fwd(b.H[i * B:(i + 1) * B], fm.fc_out.weight.data, fm.fc_out.bias.data, self.logits[i],
-                               B, D, n)
-            ops.eval_count(self.logits, self.label_in, self.counts, B, n)
+        self.head.eval(self, fa, self.enc_a.Hf * self.enc_a.Wf, fv, self.T * self.enc_v.Hf * self.enc_v.Wf)
 
-    def _compute(self, k):
-        """Sub-batch k: eager the first time (and without graphs), a graph replay afterwards."""
+    def _compute(self):
+        """Eager the first time (and without graphs), a graph replay afterwards."""
         if not self.use_graph or self.calls == 0:
             self._enqueue()
             return
-        key = tuple(p.data_ptr() for p in self.model.fusion_module.parameters()) + (self.counts.data_ptr(),)
-        if self._graph is None or self._graph_key != key:
-            torch.cuda.synchronize()
-            self._graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self._graph, capture_error_mode=_CAPTURE_MODE):
-                self._enqueue()
-            self._graph_key = key
-        self._graph.replay()
+        fm = self.model.fusion_module
+        key = tuple(p.data_ptr() for p in fm.parameters()) + (self.counts.data_ptr(), getattr(fm, "x_gate", None))
+        if key not in self.graphs:
+            self.graphs.clear()  # a graph of moved parameters or another x_gate is never replayed again
+        self.graphs.capture(key, self._enqueue).replay()
 
     def run(self, out=None):
         """Evaluate the current (or just prefetched) batch: counts += correct arg-maxes of its rows.  out: optional
         f32 [3, rows, n] that receives the logits (out, out_a, out_v) of every row."""
         self.refresh()
         for k in range(self.chunks):
-            self._enqueue_inputs(k)
-            self._compute(k)
+            self.stage.stage_rows(k, self.chunks, self.B, self.enc_a, self.enc_v, self.label_in)
+            self._compute()
             if out is not None:
                 out[:, k * self.B:(k + 1) * self.B].copy_(self.logits)
         self.calls += 1

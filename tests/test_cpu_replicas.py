@@ -60,3 +60,31 @@ def test_train_rejects_a_batch_that_does_not_split_into_the_replicas():
     spec, image = torch.zeros(6, 4, 4), torch.zeros(6, 3, 1, 4, 4)
     with pytest.raises(ValueError, match="6 rows"):
         _get_step(_get_step_args(8, 4), torch.nn.Module(), None, spec, image)
+
+
+@pytest.mark.parametrize("R", [1, 2, 3])
+@pytest.mark.parametrize("W", [1, 2])
+@pytest.mark.parametrize("overlap", [True, False])
+def test_step_schedule_and_its_graphs(R, W, overlap):
+    """DESIGN.md §5: replica k < R-1 is [layout k] then graph(compute k + accumulate), replicas 1 .. R-2 sharing one
+    graph; then the last replica: W = 1 one graph with the update; W > 1 NCCL between graphs, with the two buckets
+    graph(forward + late backward) -> bucket 1 -> graph(early backward) -> bucket 2 -> graph(update), without them
+    graph(compute) -> all-reduce -> graph(update)."""
+    from gdl_b200.step import DEVICE, graph_runs, schedule
+    seq = schedule(R, W, overlap)
+    runs = graph_runs(seq)
+    assert [seg for run in runs for seg in run] == seq
+    replicas = [(("inputs", 0),)]
+    for k in range(1, R):
+        replicas += [(("replica0" if k == 1 else "replica", None),), (("inputs", k),)]
+    if W == 1:
+        last = [(("last", None), ("update", None))]
+    elif overlap:
+        last = [(("last", 0),), (("allreduce_late", None),), (("last", 1),), (("allreduce_finish", None),),
+                (("update", None),)]
+    else:
+        last = [(("last", None),), (("allreduce", None),), (("update", None),)]
+    assert runs == replicas + last
+    graphs = [run for run in runs if run[0][0] in DEVICE]
+    assert all(seg[0] in DEVICE for run in graphs for seg in run)
+    assert len(set(graphs)) == (R > 1) + (R > 2) + (1 if W == 1 else 3 if overlap else 2)

@@ -140,7 +140,7 @@ def test_train_epoch_dropin(tmp_path):
     assert "momentum_buffer" in opt.state[p] and float(opt.state[p]["momentum_buffer"].abs().sum()) > 0
 
 
-def test_train_epoch_over_a_pinning_dataloader_with_graph_capture(tmp_path):
+def test_train_epoch_over_a_pinning_dataloader_captures_graphs(tmp_path):
     """The step's CUDA graphs are captured lazily on the SECOND step — while a real DataLoader's pin-memory thread is
     calling cudaHostAlloc / cudaEventQuery (the combination main_dgl.py runs: pin_memory=True, num_workers > 0).
     capture_error_mode="thread_local" keeps those foreign-thread calls legal.  6 steps: eager, capture, 4 replays."""
@@ -170,7 +170,7 @@ def test_train_epoch_over_a_pinning_dataloader_with_graph_capture(tmp_path):
     torch.cuda.synchronize()
     assert len(rows) == 6 and all(float(r[0]) > 0 and float(r[1]) > 0 for r in rows)
     assert all(x == x and 0 < x < 50 for x in res[:3])  # finite epoch-mean losses
-    assert model._gdl_step._graph is not None           # the captured path really ran
+    assert model._gdl_step.graphs                       # the captured path really ran
 
 
 def test_train_epoch_with_a_short_tail_batch_shares_one_arena(tmp_path):

@@ -125,8 +125,7 @@ def test_valid_against_the_oracle_eval_forward(fusion, shape, B):
 
 
 def test_gated_x_gate_false_follows_the_module():
-    from gdl_b200.step import get_eval_step
-    from oracle.synth import SHAPES, make_batch
+    from oracle.synth import make_batch
     args, model = trained("gated", "tiny", 8, steps=1)
     model.eval()
     spec, image, _ = make_batch(8, 6, "tiny", seed=5)
@@ -134,7 +133,6 @@ def test_gated_x_gate_false_follows_the_module():
     with torch.no_grad():
         on = model(spec, image)[0].clone()
         model.fusion_module.x_gate = False
-        get_eval_step(model, 8, SHAPES["tiny"][:2], SHAPES["tiny"][2:])._graph = None  # x_gate is fixed per capture
         off = model(spec, image)
         fm = model.fusion_module
         a = F.adaptive_avg_pool2d(model.audio_net(spec), 1).flatten(1)
@@ -148,7 +146,7 @@ def test_gated_x_gate_false_follows_the_module():
 
 # ------------------------------------------------------------------------------------------------ graphs and caching
 @pytest.mark.parametrize("fusion", ["concat", "film"])
-def test_graph_replay_is_bit_identical_to_eager(fusion):
+def test_eval_graph_replay_is_bit_identical_to_eager(fusion):
     from gdl_b200.step import EvalStep, eval_counts
     from oracle.synth import SHAPES, make_batch
     args, model = trained(fusion, "tiny", 8, steps=1)
@@ -167,7 +165,7 @@ def test_graph_replay_is_bit_identical_to_eager(fusion):
             ev.run(out)
             outs.append(out)
         res[use_graph] = (torch.stack(outs), counts.clone())
-        assert (ev._graph is not None) == use_graph
+        assert bool(ev.graphs) == use_graph
     assert torch.equal(res[False][0], res[True][0]) and torch.equal(res[False][1], res[True][1])
 
 
@@ -222,7 +220,7 @@ def test_fold_is_cached_and_follows_training_and_load_state_dict():
 
 
 @pytest.mark.parametrize("dp_replicas", [0, 2])
-def test_second_epoch_captures_nothing_and_allocates_nothing(tmp_path, dp_replicas):
+def test_second_epoch_reuses_every_graph_and_allocates_nothing(tmp_path, dp_replicas):
     from gdl_b200.train import train_epoch, valid
     from oracle.synth import make_batch
     args, model = make_model("concat")
@@ -239,7 +237,7 @@ def test_second_epoch_captures_nothing_and_allocates_nothing(tmp_path, dp_replic
         torch.cuda.synchronize()
         st = model._gdl_step
         evs = dict(model._gdl_evals)
-        graphs = [st._graph] + [e._graph for e in evs.values()]
+        graphs = [dict(st.graphs)] + [dict(e.graphs) for e in evs.values()]
         mem = torch.cuda.memory_allocated()
         train_epoch(args, 1, model, dev, train, opt, None)
         acc = valid(args, model, dev, test)
@@ -247,7 +245,7 @@ def test_second_epoch_captures_nothing_and_allocates_nothing(tmp_path, dp_replic
     finally:
         os.chdir(cwd)
     assert model._gdl_step is st and dict(model._gdl_evals) == evs
-    assert [st._graph] + [e._graph for e in evs.values()] == graphs and all(g is not None for g in graphs)
+    assert [dict(st.graphs)] + [dict(e.graphs) for e in evs.values()] == graphs and all(graphs)
     assert torch.cuda.memory_allocated() == mem
     ev = next(iter(evs.values()))
     assert ev.enc_a is st.enc_a and ev.B == st.B == 8 // max(dp_replicas, 1)  # sub-batches of the training geometry

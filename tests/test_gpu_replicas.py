@@ -208,6 +208,25 @@ def test_bf16_step_matches_the_simulation_and_graph_replay_is_bit_identical():
     assert all(torch.equal(v, out[1][2][k]) for k, v in out[0][2].items())
 
 
+def test_graph_replay_with_a_shared_middle_replica_graph_is_bit_identical():
+    """R = 3: replicas 1 .. R-2 replay one graph.  3 steps through the graphs == 3 eager steps, bit for bit."""
+    from oracle.synth import make_batch
+    batches = [make_batch(12, 6, "tiny", seed=1 + s) for s in range(3)]
+    out = []
+    for use_graph in (False, True):
+        model, step = _product(3, 4, use_graph, shape="tiny")
+        for batch in batches:
+            step.step(*[t.cuda() for t in batch])
+        torch.cuda.synchronize()
+        assert bool(step.graphs) == use_graph
+        out.append((step.stats.clone(), step.arena.param.clone(), step.arena.momentum.clone(),
+                    {k: v.clone() for k, v in model.named_buffers()}))
+        del model, step
+    for a, b in zip(out[0][:3], out[1][:3]):
+        assert torch.equal(a, b), "CUDA-graph replay differs from eager execution"
+    assert all(torch.equal(v, out[1][3][k]) for k, v in out[0][3].items())
+
+
 def test_later_replicas_leave_the_running_statistics_bit_identical():
     """After one R = 2 step the running statistics are bit-identical to those of a one-replica step on replica 0's
     rows alone (same weights, same kernels): replica 1 did not touch them.  num_batches_tracked advanced once."""

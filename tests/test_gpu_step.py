@@ -165,11 +165,11 @@ def test_backward_parity_with_forced_forward(fusion):
         assert 0.99 < ratio < 1.01, (k, ratio)
 
 
-def test_step_is_deterministic_and_graph_equals_eager():
+def _deterministic_and_graph_equals_eager(fusion):
     from oracle.synth import make_batch
     outs = []
     for use_graph in (False, False, True):
-        model, step = build("concat", "CREMAD", 4, "tiny", use_graph=use_graph)
+        model, step = build(fusion, "CREMAD", 4, "tiny", use_graph=use_graph)
         for s in range(3):
             batch = make_batch(4, 6, "tiny", seed=1 + s)
             step.step(*[t.cuda() for t in batch])
@@ -179,6 +179,15 @@ def test_step_is_deterministic_and_graph_equals_eager():
         assert torch.equal(a, b), "two eager runs differ: the step is not deterministic"
     for a, b in zip(outs[0], outs[2]):
         assert torch.equal(a, b), "CUDA-graph replay differs from eager execution"
+
+
+def test_step_is_deterministic_and_graph_equals_eager():
+    _deterministic_and_graph_equals_eager("concat")
+
+
+@pytest.mark.parametrize("fusion", ["sum", "gated", "film"])
+def test_step_of_every_head_is_deterministic_and_graph_equals_eager(fusion):
+    _deterministic_and_graph_equals_eager(fusion)
 
 
 def test_alpha_linearity_at_bench_size():
