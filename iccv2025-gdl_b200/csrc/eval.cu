@@ -6,6 +6,8 @@
 //    sets of the concat / sum / gated head (gated honours x_gate), the arg-max of each row and the per-head correct
 //    counts, added into an int64 device counter.  kind 3 only pools (the FiLM head runs its GEMMs next).
 //  * gdl_eval_count : arg-max + counts over given logits [3,B,n] (the FiLM head's count step).
+//  * gdl_eval_confusion : arg-max over given logits [3,B,n] + per-head confusion matrices conf[h][label][pred]
+//    (the per-class report of valid_report(); a separate launch, paid only when a report is asked for).
 // Every reduction runs in a fixed order and the counts are integers, so the results are deterministic.
 #include "common.cuh"
 
@@ -184,6 +186,25 @@ __global__ void eval_count_kernel(const float* __restrict__ logits, const int64_
   if ((threadIdx.x & 31) == 0 && (int64_t)pred == labels[b]) atomicAdd(counts + h, 1ull);
 }
 
+// one warp per (head, row) of logits [3][B][n]: conf[h][label][pred] += 1; a label < 0 is skipped, a label >= n is
+// counted once per row (head 0) in *out_of_range and never indexes conf
+__global__ void eval_confusion_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels,
+                                      unsigned long long* __restrict__ conf,
+                                      unsigned long long* __restrict__ out_of_range, int B, int n) {
+  pdl_enter();
+  const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= 3 * (int64_t)B) return;
+  const int h = int(w / B), b = int(w - (int64_t)h * B);
+  const int64_t label = labels[b];
+  if (label < 0) return;
+  if (label >= n) {
+    if (h == 0 && (threadIdx.x & 31) == 0) atomicAdd(out_of_range, 1ull);
+    return;
+  }
+  const int pred = warp_argmax(logits + ((int64_t)h * B + b) * n, n);
+  if ((threadIdx.x & 31) == 0) atomicAdd(conf + ((int64_t)h * n + label) * n + pred, 1ull);
+}
+
 }  // namespace gdl
 
 using namespace gdl;
@@ -219,5 +240,17 @@ extern "C" int gdl_eval_count(const float* logits, const int64_t* labels, int64_
   launch_pdl(eval_count_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s, logits, labels,
              (unsigned long long*)counts, B, n);
   GDL_CHECK_LAUNCH("eval_count_kernel");
+  return GDL_OK;
+}
+
+extern "C" int gdl_eval_confusion(const float* logits, const int64_t* labels, int64_t* conf, int64_t* out_of_range,
+                                  int B, int n, gdl_stream_t s) {
+  GDL_REQUIRE(logits && labels && conf && out_of_range, "gdl_eval_confusion: null pointer");
+  GDL_REQUIRE(B > 0, "gdl_eval_confusion: B must be positive");
+  GDL_REQUIRE(n > 0 && n <= kEvalMaxN, "gdl_eval_confusion: n must be in 1..512");
+  const int64_t threads = 3 * (int64_t)B * 32;
+  launch_pdl(eval_confusion_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s, logits, labels,
+             (unsigned long long*)conf, (unsigned long long*)out_of_range, B, n);
+  GDL_CHECK_LAUNCH("eval_confusion_kernel");
   return GDL_OK;
 }

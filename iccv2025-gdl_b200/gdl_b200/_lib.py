@@ -97,6 +97,7 @@ SIGNATURES = {
     "gdl_softmax_ce": (_i, [_p, _p, _f, _f, _p, _p, _p, _i, _i, _p]),
     "gdl_eval_head": (_i, [_i, _p, _i, _p, _i, _p, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p]),
     "gdl_eval_count": (_i, [_p, _p, _p, _i, _i, _p]),
+    "gdl_eval_confusion": (_i, [_p, _p, _p, _p, _i, _i, _p]),
     "gdl_gated_fwd": (_i, [_p, _p, _p, _p, _p, _l, _p]),
     "gdl_gated_bwd": (_i, [_p, _p, _p, _p, _p, _p, _l, _p]),
     "gdl_optim_scratch_floats": (_l, [_l, _i]),

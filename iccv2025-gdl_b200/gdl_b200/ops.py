@@ -408,6 +408,14 @@ def eval_count(logits, labels, counts, B, n):
     check(_lib.load().gdl_eval_count(_ptr(logits), _ptr(labels), _ptr(counts), B, n, _stream()), "gdl_eval_count")
 
 
+@_op("eval_confusion", 1, lambda logits, labels, conf, out_of_range, B, n: ("bytes", 12.0 * B * n + 8.0 * B))
+def eval_confusion(logits, labels, conf, out_of_range, B, n):
+    """conf[h][label][pred] += 1 for the arg-max pred of every row of logits[h] ([3, B, n]) and its label (conf int64
+    [3, n, n]); labels < 0 are skipped, labels >= n only add to out_of_range (int64 [1])."""
+    check(_lib.load().gdl_eval_confusion(_ptr(logits), _ptr(labels), _ptr(conf), _ptr(out_of_range), B, n, _stream()),
+          "gdl_eval_confusion")
+
+
 @_op("softmax_ce", 2)
 def softmax_ce(logits, labels, loss_scale, grad_scale, loss_out, dlogits, scratch, B, n):
     check(_lib.load().gdl_softmax_ce(_ptr(logits), _ptr(labels), loss_scale, grad_scale, _ptr(loss_out),

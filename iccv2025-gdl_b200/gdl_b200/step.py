@@ -531,6 +531,17 @@ def eval_counts(model, device):
     return c
 
 
+def eval_confusion(model, device):
+    """The model's int64 [1 + 3 n n] device buffer of the per-class report (valid_report), allocated on first use:
+    element 0 counts the rows whose label is >= n, the rest is the confusion matrices [3, n, n] (out, out_a, out_v;
+    rows = true class, columns = arg-max) that an EvalStep adds to when run(report=True)."""
+    c = getattr(model, "_gdl_eval_confusion", None)
+    if c is None or c.device != device:
+        n = model.n_classes
+        c = model._gdl_eval_confusion = torch.zeros(1 + 3 * n * n, device=device, dtype=torch.int64)
+    return c
+
+
 class EvalStep:
     """Eval-mode forward of AVClassifier_DGL for batches of `rows` rows (reference valid(), main_dgl.py:168-222, and
     `model(...)` in eval mode): stem layout of each sub-batch of b rows, both encoders with BatchNorm folded
@@ -539,7 +550,9 @@ class EvalStep:
     gdl_eval_count).  Everything after the layout is one CUDA graph, captured on the second call and re-captured only
     when a head parameter moves or the gated head's x_gate flips.  The BatchNorm fold and the FiLM weight shadow are
     refreshed outside the graph, and only when a parameter or buffer changed.  The logits of the last sub-batch stay
-    in `logits` [3, b, n]."""
+    in `logits` [3, b, n].  run(report=True) appends gdl_eval_confusion (the per-class confusion matrices of
+    eval_confusion) to the head; that variant is captured as a graph of its own, so the two alternate without
+    re-capture and run(report=False) launches exactly what it would without the report."""
 
     def __init__(self, model, rows, spec_hw, image_thw, use_graph=True):
         model = getattr(model, "module", model)
@@ -561,6 +574,7 @@ class EvalStep:
         self.label_in = torch.full((B,), -1, dtype=torch.int64, device=dev)
         self.logits = torch.empty(3, B, self.n, device=dev)
         self.counts = eval_counts(model, dev)
+        self.report, self.confusion = False, None
         self.head = head if head is not None else fusion_head(model.fusion_module, B, self.n, dev)
         self._head_key = None
         self.stream_a, self.stream_v = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
@@ -592,6 +606,9 @@ class EvalStep:
         main.wait_stream(sa)
         main.wait_stream(sv)
         self.head.eval(self, fa, self.enc_a.Hf * self.enc_a.Wf, fv, self.T * self.enc_v.Hf * self.enc_v.Wf)
+        if self.report:
+            c = self.confusion
+            ops.eval_confusion(self.logits, self.label_in, c[1:], c[:1], self.B, self.n)
 
     def _compute(self):
         """Eager the first time (and without graphs), a graph replay afterwards."""
@@ -599,14 +616,20 @@ class EvalStep:
             self._enqueue()
             return
         fm = self.model.fusion_module
-        key = tuple(p.data_ptr() for p in fm.parameters()) + (self.counts.data_ptr(), getattr(fm, "x_gate", None))
+        base = tuple(p.data_ptr() for p in fm.parameters()) + (self.counts.data_ptr(), getattr(fm, "x_gate", None))
+        key = (base, self.confusion.data_ptr() if self.report else None)
         if key not in self.graphs:
-            self.graphs.clear()  # a graph of moved parameters or another x_gate is never replayed again
+            for k in [k for k in self.graphs if k[0] != base]:
+                del self.graphs[k]  # a graph of moved parameters or another x_gate is never replayed again
         self.graphs.capture(key, self._enqueue).replay()
 
-    def run(self, out=None):
+    def run(self, out=None, report=False):
         """Evaluate the current (or just prefetched) batch: counts += correct arg-maxes of its rows.  out: optional
-        f32 [3, rows, n] that receives the logits (out, out_a, out_v) of every row."""
+        f32 [3, rows, n] that receives the logits (out, out_a, out_v) of every row.  report: also add the rows to the
+        model's confusion matrices (eval_confusion)."""
+        self.report = report
+        if report:
+            self.confusion = eval_confusion(self.model, self.device)
         self.refresh()
         for k in range(self.chunks):
             self.stage.stage_rows(k, self.chunks, self.B, self.enc_a, self.enc_v, self.label_in)

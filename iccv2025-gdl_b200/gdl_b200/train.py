@@ -8,6 +8,7 @@ in is only read for its update rule, hyper-parameters and lr schedule (gdl_b200.
 Adam or Adagrad; anything else raises) — the update itself is a fused kernel over the parameter arena (its state is
 exposed through `optimizer.state[p]` — `momentum_buffer`, `exp_avg` / `exp_avg_sq` / `step`, `sum` / `step` — so
 reference-format checkpoints still carry it).
+`valid_report` is an addition: `valid` plus the per-class confusion matrices of the three heads (EvalReport).
 """
 import csv
 
@@ -15,7 +16,7 @@ import torch
 
 from .optim import update_rule
 from .parallel import ChunkShardBatchSampler, broadcast_running_stats, replicas_per_rank
-from .step import DGLStep, eval_counts, get_eval_step
+from .step import DGLStep, eval_confusion, eval_counts, get_eval_step
 
 LOG_EVERY = 100  # the reference prints every 100 steps (main_dgl.py:125,144)
 GRAD_CSV = 'audio_visual_grad_vanilla.csv'  # main_dgl.py:148
@@ -206,14 +207,11 @@ def _sharded(dataloader):
     return _world() > 1 and isinstance(getattr(dataloader, "batch_sampler", None), ChunkShardBatchSampler)
 
 
-def valid(args, model, device, dataloader):
-    """reference main_dgl.py:168-222: eval-mode forward (BN running statistics), softmax,
-    arg-max accuracy of the fused / audio / visual heads.  Runs on the cached EvalStep of the batch geometry (CUDA
-    graph, the next batch prefetched on the copy stream); the correct counts accumulate on the device and are read
-    once at the end.  `drop_last` behaviour is the loader's.
-    A data-parallel test loader (parallel.ChunkShardBatchSampler: each rank evaluates its shard of every global batch)
-    is evaluated like nn.DataParallel evaluates the reference's: every rank first takes rank 0's BatchNorm running
-    statistics, and the counts are summed over the ranks, so every rank returns the accuracy over all the samples."""
+def _evaluate(model, dataloader, report):
+    """The evaluation pass of valid() and valid_report() on the model's cached EvalSteps, with the reference's
+    args.drop flips, print, eval() and no_grad.  Returns the CPU int64 tensor [counts (3), total] and, with `report`,
+    then the out-of-range row count and the confusion matrices [3 n n] (step.eval_confusion), summed over the ranks of
+    a sharded loader by one all-reduce after rank 0's BatchNorm statistics were broadcast."""
     inner = getattr(model, "module", model)
     inner.args.drop = 0
     with torch.no_grad():
@@ -223,8 +221,10 @@ def valid(args, model, device, dataloader):
         sharded = _sharded(dataloader)
         if sharded:
             broadcast_running_stats(inner)
-        counts = eval_counts(inner, next(inner.parameters()).device)
+        dev = next(inner.parameters()).device
+        counts = eval_counts(inner, dev)
         counts.zero_()
+        conf = eval_confusion(inner, dev).zero_() if report else None
         total = 0
         it = iter(dataloader)
         nxt = next(it, None)
@@ -237,16 +237,80 @@ def valid(args, model, device, dataloader):
             ev = get(nxt)
             _prefetch(ev, nxt, pipe, apipe)
         while nxt is not None:
-            ev.run()
+            ev.run(report=report)
             total += ev.rows
             nxt = next(it, None)
             if nxt is not None:
                 ev = get(nxt)
                 _prefetch(ev, nxt, pipe, apipe)
-        res = torch.cat([counts, torch.tensor([total], device=counts.device, dtype=torch.int64)])
+        res = torch.cat([counts, torch.tensor([total], device=dev, dtype=torch.int64)] + ([conf] if report else []))
         if sharded:
             torch.distributed.all_reduce(res)
-        res = res.tolist()  # the one D2H of the evaluation
+        res = res.cpu()  # the one D2H of the evaluation
     inner.args.drop = 1
+    return res
+
+
+def valid(args, model, device, dataloader):
+    """reference main_dgl.py:168-222: eval-mode forward (BN running statistics), softmax,
+    arg-max accuracy of the fused / audio / visual heads.  Runs on the cached EvalStep of the batch geometry (CUDA
+    graph, the next batch prefetched on the copy stream); the correct counts accumulate on the device and are read
+    once at the end.  `drop_last` behaviour is the loader's.
+    A data-parallel test loader (parallel.ChunkShardBatchSampler: each rank evaluates its shard of every global batch)
+    is evaluated like nn.DataParallel evaluates the reference's: every rank first takes rank 0's BatchNorm running
+    statistics, and the counts are summed over the ranks, so every rank returns the accuracy over all the samples."""
+    res = _evaluate(model, dataloader, False).tolist()
     n = max(res[3], 1)
     return res[0] / n, res[1] / n, res[2] / n
+
+
+HEADS = ("out", "out_a", "out_v")
+
+
+class EvalReport:
+    """Per-class result of valid_report().
+    confusion  CPU int64 [3, n, n]: heads (out, out_a, out_v), rows = true class, columns = arg-max
+    total      evaluated rows (as valid() counts them)
+    support    int64 [n]: rows per true class (the row sums, the same for every head)
+    correct    int64 [3, n]: the diagonals
+    acc, acc_a, acc_v   the traces over max(total, 1): what valid() returns for the same loader
+    per_class  float64 [3, n]: correct / support, NaN for a class without samples"""
+
+    def __init__(self, confusion, total):
+        self.confusion = confusion
+        self.total = int(total)
+        self.n = confusion.shape[-1]
+        self.support = confusion[0].sum(1)
+        self.correct = confusion.diagonal(dim1=1, dim2=2).clone()
+        hits = self.correct.sum(1).tolist()
+        den = max(self.total, 1)
+        self.acc, self.acc_a, self.acc_v = hits[0] / den, hits[1] / den, hits[2] / den
+        self.per_class = torch.where(self.support > 0, self.correct.double() / self.support.clamp(min=1).double(),
+                                     torch.tensor(float("nan"), dtype=torch.float64))
+
+    def rows(self, epoch):
+        """[epoch, head, class, support, correct, accuracy] for every head and class (accuracy 'nan' for an empty
+        class): the rows of main_dgl.py --per_class's per-class CSV."""
+        sup, cor, acc = self.support.tolist(), self.correct.tolist(), self.per_class.tolist()
+        return [[epoch, HEADS[h], c, sup[c], cor[h][c], acc[h][c]] for h in range(3) for c in range(self.n)]
+
+    def table(self):
+        """The per-class accuracies as text: one line per class, one column per head."""
+        acc = self.per_class.tolist()
+        lines = ["{:>5} {:>7} {:>8} {:>8} {:>8}".format("class", "support", *HEADS)]
+        for c, sup in enumerate(self.support.tolist()):
+            lines.append("{:>5} {:>7} {:>8.4f} {:>8.4f} {:>8.4f}".format(c, sup, acc[0][c], acc[1][c], acc[2][c]))
+        return "\n".join(lines)
+
+
+def valid_report(args, model, device, dataloader):
+    """valid() with the per-class confusion matrices of the three heads (EvalReport), counted on the device by
+    gdl_eval_confusion in the same graph-captured pass and read with the counts in its one D2H (one all-reduce for a
+    sharded loader).  Same args.drop flips, print and accuracies as valid().  Raises ValueError when a label is >= the
+    head width (the reference fails with an IndexError on `num[label]`)."""
+    res = _evaluate(model, dataloader, True)
+    n = getattr(model, "module", model).n_classes
+    if int(res[4]):
+        raise ValueError("{} evaluated rows have a label outside the {} classes of the heads (0..{})"
+                         .format(int(res[4]), n, n - 1))
+    return EvalReport(res[5:].view(3, n, n), int(res[3]))

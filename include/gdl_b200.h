@@ -272,6 +272,13 @@ int gdl_eval_head(int kind, const void* fa, int Ga, const void* fv, int Gv, cons
                   gdl_stream_t s);
 /* counts[h] += #{b : argmax(logits[h][b][:]) == labels[b]} for h = 0, 1, 2; logits f32 [3][B][n]. */
 int gdl_eval_count(const float* logits, const int64_t* labels, int64_t* counts, int B, int n, gdl_stream_t s);
+/* Per-class report (opt-in beside gdl_eval_head / gdl_eval_count): for h = 0, 1, 2 and every row b of logits
+ * f32 [3][B][n], pred = arg-max of the row (the same order as gdl_eval_head: NaN largest, ties to the lowest index)
+ * and conf[h][labels[b]][pred] += 1 (int64 [3][n][n], device; rows = true class, columns = prediction).  A label < 0
+ * is skipped; a label >= n adds 1 (once per row) to *out_of_range (int64, device) and writes nothing else.
+ * 1 <= n <= 512, B > 0. */
+int gdl_eval_confusion(const float* logits, const int64_t* labels, int64_t* conf, int64_t* out_of_range, int B, int n,
+                       gdl_stream_t s);
 /* Gated-head elementwise pieces (reference models/fusion_modules.py:230-250). */
 int gdl_gated_fwd(const float* hx, const float* hy, float* m_out, float* m_x, float* m_y,
                   int64_t numel, gdl_stream_t s);

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """CLI-compatible entry point for the reference's main_dgl.py (same flags, same defaults,
 same prints / csv / checkpoint file names, same evaluation-mode checkpoint loading), running the B200-native DGL step.
-Deviations: no TensorBoard branch; `--resume`, `--synthetic_len` and `--dp_replicas` are additions.
+Deviations: no TensorBoard branch; `--resume`, `--synthetic_len`, `--dp_replicas` and `--per_class` are additions.
 
     python main_dgl.py --train --ckpt_path ckpt --dataset CREMAD --fusion_method concat \
         --fps 3 --alpha 4 --batch_size 64 --audio_path synthetic
@@ -27,7 +27,7 @@ from torch.utils.data import DataLoader  # noqa: E402
 from gdl_b200 import AVClassifier_DGL, setup_seed, weight_init  # noqa: E402
 from gdl_b200.parallel import replicas_per_rank  # noqa: E402
 from gdl_b200.synthetic import SyntheticAV  # noqa: E402
-from gdl_b200.train import train_epoch, valid  # noqa: E402
+from gdl_b200.train import train_epoch, valid, valid_report  # noqa: E402
 
 
 def get_arguments(argv=None):
@@ -67,7 +67,31 @@ def get_arguments(argv=None):
     parser.add_argument('--dp_replicas', default=0, type=int,
                         help='data-parallel replicas R (0 = one per process): batch_size / R rows per BatchNorm batch, '
                              'R / processes of them run one after another on each GPU, like nn.DataParallel over R GPUs')
+    parser.add_argument('--per_class', action='store_true',
+                        help='evaluate with per-class accuracies of the fused, audio and visual heads: appended to '
+                             '<ckpt_path>/<dataset>_<modality>_per_class.csv when training, printed in evaluation mode')
     return parser.parse_args(argv)
+
+
+PER_CLASS_HEADER = ['epoch', 'head', 'class', 'support', 'correct', 'accuracy']
+
+
+def evaluate_epoch(args, model, device, loader, epoch, rank=0):
+    """The evaluation pass of a training epoch: valid() (acc, acc_a, acc_v), or with --per_class valid_report(),
+    whose accuracies are the same; rank 0 then appends the epoch's per-class rows to
+    <ckpt_path>/<dataset>_<modality>_per_class.csv (a header first when the file is new)."""
+    if not args.per_class:
+        return valid(args, model, device, loader)
+    report = valid_report(args, model, device, loader)
+    if rank == 0:
+        path = os.path.join(args.ckpt_path, args.dataset + '_' + args.modality + '_per_class.csv')
+        new = not os.path.exists(path)
+        with open(path, 'a+', newline='') as f:
+            w = csv.writer(f)
+            if new:
+                w.writerow(PER_CLASS_HEADER)
+            w.writerows(report.rows(epoch))
+    return report.acc, report.acc_a, report.acc_v
 
 
 def main(argv=None):
@@ -181,7 +205,7 @@ def main(argv=None):
             if shard_sampler is not None:
                 from gdl_b200.parallel import assert_same_order
                 assert_same_order(shard_sampler.order_digest)
-            acc, acc_a, acc_v = valid(args, model, device, test_loader)
+            acc, acc_a, acc_v = evaluate_epoch(args, model, device, test_loader, epoch, rank)
             if rank == 0:
                 with open(log, 'a+', newline='') as f:
                     csv.writer(f).writerow([acc, acc_a, acc_v])
@@ -217,8 +241,15 @@ def main(argv=None):
             'inconsistency between fusion method of loaded model and args !'
         model.load_state_dict(loaded_dict['model'])
         print('Trained model loaded!')
-        acc, acc_a, acc_v = valid(args, model, device, test_loader)
+        if args.per_class:
+            report = valid_report(args, model, device, test_loader)
+            acc, acc_a, acc_v = report.acc, report.acc_a, report.acc_v
+        else:
+            acc, acc_a, acc_v = valid(args, model, device, test_loader)
         print('Accuracy: {}, accuracy_a: {}, accuracy_v: {}'.format(acc, acc_a, acc_v))
+        if args.per_class:
+            print('Per-class accuracy ({} samples):'.format(report.total))
+            print(report.table())
 
 
 if __name__ == "__main__":
