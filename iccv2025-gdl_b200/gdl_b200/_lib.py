@@ -98,6 +98,9 @@ SIGNATURES = {
     "gdl_eval_head": (_i, [_i, _p, _i, _p, _i, _p, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p]),
     "gdl_eval_count": (_i, [_p, _p, _p, _i, _i, _p]),
     "gdl_eval_confusion": (_i, [_p, _p, _p, _p, _i, _i, _p]),
+    "gdl_eval_scores": (_i, [_p, _p, _i, _i, _i, _p, _p, _l, _p, _p, _p, _p]),
+    "gdl_eval_ap_workspace_bytes": (_l, [_l, _i]),
+    "gdl_eval_ap": (_i, [_p, _p, _p, _l, _i, _p, _p, _p, _p, _l, _p]),
     "gdl_gated_fwd": (_i, [_p, _p, _p, _p, _p, _l, _p]),
     "gdl_gated_bwd": (_i, [_p, _p, _p, _p, _p, _p, _l, _p]),
     "gdl_optim_scratch_floats": (_l, [_l, _i]),

@@ -416,6 +416,36 @@ def eval_confusion(logits, labels, conf, out_of_range, B, n):
           "gdl_eval_confusion")
 
 
+@_op("eval_scores", 2, lambda logits, labels, store, store_labels, cursor, hits, overflow, B, n, k:
+     ("bytes", 24.0 * B * n + 12.0 * B))
+def eval_scores(logits, labels, store, store_labels, cursor, hits, overflow, B, n, k):
+    """Append softmax(logits[h]) of the B rows of logits [3, B, n] class-major to store f32 [3, n, cap] at row
+    cursor (int64 [1], advanced by B) and their labels to store_labels int32 [cap] (-1 outside 0..n-1); hits int64 [3]
+    += the rows whose label ranks < k (NaN largest, ties to the lower index); labelled rows beyond cap only add to
+    overflow (int64 [1])."""
+    check(_lib.load().gdl_eval_scores(_ptr(logits), _ptr(labels), B, n, k, _ptr(store), _ptr(store_labels),
+                                      store.shape[-1], _ptr(cursor), _ptr(hits), _ptr(overflow), _stream()),
+          "gdl_eval_scores")
+
+
+def eval_ap_workspace_bytes(cap, n):
+    """Device workspace gdl_eval_ap needs for a store of cap rows (0 when a column sorts in shared memory)."""
+    return int(_lib.load().gdl_eval_ap_workspace_bytes(cap, n))
+
+
+@_op("eval_ap", 2, lambda store, store_labels, cursor, ap, support, nonfinite, workspace=None:
+     ("bytes", 4.0 * store.numel() + 4.0 * store_labels.numel() * (store.shape[0] * store.shape[1] + 1)))
+def eval_ap(store, store_labels, cursor, ap, support, nonfinite, workspace=None):
+    """ap f64 [3, n] = the average precision of every (head, class) column of store f32 [3, n, cap] over its first
+    min(cursor, cap) rows whose store_labels (int32 [cap]) are in 0..n-1 (NaN for a class without rows); support
+    int64 [n] = rows per class; nonfinite int64 [1] = rows with a non-finite score.  workspace: uint8 of at least
+    eval_ap_workspace_bytes(cap, n) bytes when that is not 0."""
+    cap, n = store.shape[-1], store.shape[1]
+    check(_lib.load().gdl_eval_ap(_ptr(store), _ptr(store_labels), _ptr(cursor), cap, n, _ptr(ap), _ptr(support),
+                                  _ptr(nonfinite), _ptr(workspace), 0 if workspace is None else workspace.numel(),
+                                  _stream()), "gdl_eval_ap")
+
+
 @_op("softmax_ce", 2)
 def softmax_ce(logits, labels, loss_scale, grad_scale, loss_out, dlogits, scratch, B, n):
     check(_lib.load().gdl_softmax_ce(_ptr(logits), _ptr(labels), loss_scale, grad_scale, _ptr(loss_out),

@@ -542,6 +542,53 @@ def eval_confusion(model, device):
     return c
 
 
+class EvalScores:
+    """The device buffers of valid_report(ap=True) for a model with n classes and room for `capacity` rows:
+    store      f32 [3, n, capacity]: softmax scores, class-major (heads out, out_a, out_v), written by gdl_eval_scores
+    labels     int32 [capacity]: the rows' labels (-1 outside 0..n-1)
+    state      int64 [5]: cursor (rows appended so far), overflow (labelled rows that did not fit), hits [3] (top-k)
+    ap, support, nonfinite   what gdl_eval_ap writes: f64 [3, n], int64 [n], int64 [1]
+    workspace  gdl_eval_ap's sort workspace (None when a column sorts in shared memory)
+    k          the top-k of the hits (set before a pass)"""
+
+    def __init__(self, n, capacity, device):
+        self.n, self.capacity = n, capacity
+        self.store = torch.empty(3, n, capacity, device=device)
+        self.labels = torch.full((capacity,), -1, dtype=torch.int32, device=device)
+        self.state = torch.zeros(5, dtype=torch.int64, device=device)
+        self.cursor, self.overflow, self.hits = self.state[0:1], self.state[1:2], self.state[2:5]
+        self.ap = torch.empty(3, n, dtype=torch.float64, device=device)
+        self.support = torch.empty(n, dtype=torch.int64, device=device)
+        self.nonfinite = torch.empty(1, dtype=torch.int64, device=device)
+        ws = ops.eval_ap_workspace_bytes(capacity, n)
+        self.workspace = torch.empty(ws, dtype=torch.uint8, device=device) if ws else None
+        self.k = min(5, n)
+        self.gathered = None  # the store of every rank's rows (train.valid_report on a sharded loader)
+
+    def graph_key(self):
+        """What a captured gdl_eval_scores launch depends on."""
+        return (self.store.data_ptr(), self.labels.data_ptr(), self.state.data_ptr(), self.capacity, self.k)
+
+    def append(self, logits, labels, B):
+        """gdl_eval_scores of logits [3, B, n] and labels [B]: append at the cursor, add the top-k hits."""
+        ops.eval_scores(logits, labels, self.store, self.labels, self.cursor, self.hits, self.overflow, B, self.n,
+                        self.k)
+
+    def average_precision(self):
+        """gdl_eval_ap over the appended rows into ap, support and nonfinite."""
+        ops.eval_ap(self.store, self.labels, self.cursor, self.ap, self.support, self.nonfinite, self.workspace)
+
+
+def eval_scores(model, device, capacity):
+    """The model's EvalScores (the score store of valid_report(ap=True)), allocated on first use and re-allocated only
+    when `capacity` rows do not fit in it."""
+    sc = getattr(model, "_gdl_eval_scores", None)
+    if sc is None or sc.store.device != device or sc.capacity < capacity:
+        sc = model._gdl_eval_scores = None  # free the smaller store first
+        sc = model._gdl_eval_scores = EvalScores(model.n_classes, max(int(capacity), 1), device)
+    return sc
+
+
 class EvalStep:
     """Eval-mode forward of AVClassifier_DGL for batches of `rows` rows (reference valid(), main_dgl.py:168-222, and
     `model(...)` in eval mode): stem layout of each sub-batch of b rows, both encoders with BatchNorm folded
@@ -552,7 +599,9 @@ class EvalStep:
     refreshed outside the graph, and only when a parameter or buffer changed.  The logits of the last sub-batch stay
     in `logits` [3, b, n].  run(report=True) appends gdl_eval_confusion (the per-class confusion matrices of
     eval_confusion) to the head; that variant is captured as a graph of its own, so the two alternate without
-    re-capture and run(report=False) launches exactly what it would without the report."""
+    re-capture and run(report=False) launches exactly what it would without the report.  run(scores=True) appends
+    gdl_eval_scores (the softmax scores and top-k hits of the model's EvalScores, after the confusion matrices when
+    both are asked for): one more graph variant, keyed by the store it writes."""
 
     def __init__(self, model, rows, spec_hw, image_thw, use_graph=True):
         model = getattr(model, "module", model)
@@ -574,7 +623,7 @@ class EvalStep:
         self.label_in = torch.full((B,), -1, dtype=torch.int64, device=dev)
         self.logits = torch.empty(3, B, self.n, device=dev)
         self.counts = eval_counts(model, dev)
-        self.report, self.confusion = False, None
+        self.report, self.confusion, self.scores = False, None, None
         self.head = head if head is not None else fusion_head(model.fusion_module, B, self.n, dev)
         self._head_key = None
         self.stream_a, self.stream_v = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
@@ -609,6 +658,8 @@ class EvalStep:
         if self.report:
             c = self.confusion
             ops.eval_confusion(self.logits, self.label_in, c[1:], c[:1], self.B, self.n)
+        if self.scores is not None:
+            self.scores.append(self.logits, self.label_in, self.B)
 
     def _compute(self):
         """Eager the first time (and without graphs), a graph replay afterwards."""
@@ -617,19 +668,27 @@ class EvalStep:
             return
         fm = self.model.fusion_module
         base = tuple(p.data_ptr() for p in fm.parameters()) + (self.counts.data_ptr(), getattr(fm, "x_gate", None))
-        key = (base, self.confusion.data_ptr() if self.report else None)
+        key = (base, self.confusion.data_ptr() if self.report else None,
+               self.scores.graph_key() if self.scores is not None else None)
         if key not in self.graphs:
             for k in [k for k in self.graphs if k[0] != base]:
                 del self.graphs[k]  # a graph of moved parameters or another x_gate is never replayed again
         self.graphs.capture(key, self._enqueue).replay()
 
-    def run(self, out=None, report=False):
+    def run(self, out=None, report=False, scores=False):
         """Evaluate the current (or just prefetched) batch: counts += correct arg-maxes of its rows.  out: optional
         f32 [3, rows, n] that receives the logits (out, out_a, out_v) of every row.  report: also add the rows to the
-        model's confusion matrices (eval_confusion)."""
+        model's confusion matrices (eval_confusion).  scores: also append the rows' softmax scores to the model's
+        EvalScores (allocated beforehand by eval_scores) and add their top-k hits."""
         self.report = report
         if report:
             self.confusion = eval_confusion(self.model, self.device)
+        self.scores = None
+        if scores:
+            self.scores = getattr(self.model, "_gdl_eval_scores", None)
+            if self.scores is None or self.scores.store.device != self.device:
+                raise RuntimeError("run(scores=True) appends to the store of step.eval_scores(model, device, "
+                                   "capacity): allocate it first")
         self.refresh()
         for k in range(self.chunks):
             self.stage.stage_rows(k, self.chunks, self.B, self.enc_a, self.enc_v, self.label_in)

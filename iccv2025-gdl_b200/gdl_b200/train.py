@@ -8,7 +8,8 @@ in is only read for its update rule, hyper-parameters and lr schedule (gdl_b200.
 Adam or Adagrad; anything else raises) — the update itself is a fused kernel over the parameter arena (its state is
 exposed through `optimizer.state[p]` — `momentum_buffer`, `exp_avg` / `exp_avg_sq` / `step`, `sum` / `step` — so
 reference-format checkpoints still carry it).
-`valid_report` is an addition: `valid` plus the per-class confusion matrices of the three heads (EvalReport).
+`valid_report` is an addition: `valid` plus the per-class confusion matrices of the three heads (EvalReport), and
+with ap=True the per-class average precision, mAP and top-k accuracy of the three heads.
 """
 import csv
 
@@ -16,7 +17,7 @@ import torch
 
 from .optim import update_rule
 from .parallel import ChunkShardBatchSampler, broadcast_running_stats, replicas_per_rank
-from .step import DGLStep, eval_confusion, eval_counts, get_eval_step
+from .step import DGLStep, EvalScores, eval_confusion, eval_counts, eval_scores, get_eval_step
 
 LOG_EVERY = 100  # the reference prints every 100 steps (main_dgl.py:125,144)
 GRAD_CSV = 'audio_visual_grad_vanilla.csv'  # main_dgl.py:148
@@ -207,11 +208,15 @@ def _sharded(dataloader):
     return _world() > 1 and isinstance(getattr(dataloader, "batch_sampler", None), ChunkShardBatchSampler)
 
 
-def _evaluate(model, dataloader, report):
+def _evaluate(model, dataloader, report, topk=None):
     """The evaluation pass of valid() and valid_report() on the model's cached EvalSteps, with the reference's
     args.drop flips, print, eval() and no_grad.  Returns the CPU int64 tensor [counts (3), total] and, with `report`,
     then the out-of-range row count and the confusion matrices [3 n n] (step.eval_confusion), summed over the ranks of
-    a sharded loader by one all-reduce after rank 0's BatchNorm statistics were broadcast."""
+    a sharded loader by one all-reduce after rank 0's BatchNorm statistics were broadcast.  With `topk` (an int) the
+    pass also appends every row's softmax scores to the model's EvalScores, sized len(loader) x the first batch's rows,
+    and the tensor goes on with [overflow, top-k hits (3), capacity, rows beyond it, total^2, capacity^2] (summed
+    with the rest) and gdl_eval_ap's results: ap [3 n] (f64 bits), support [n], nonfinite.  A sharded loader's stores
+    are gathered after the all-reduce and every rank computes the AP of all the rows."""
     inner = getattr(model, "module", model)
     inner.args.drop = 0
     with torch.no_grad():
@@ -229,6 +234,12 @@ def _evaluate(model, dataloader, report):
         it = iter(dataloader)
         nxt = next(it, None)
         ev = None
+        sc, capacity = None, 0
+        if topk is not None:
+            capacity = len(dataloader) * (nxt[2].shape[0] if nxt is not None else 0)
+            sc = eval_scores(inner, dev, capacity)
+            sc.state.zero_()
+            sc.k = max(1, min(int(topk), inner.n_classes))
 
         def get(batch):
             spec_hw, thw = _geometry(batch[0], batch[1], pipe, apipe)
@@ -237,18 +248,54 @@ def _evaluate(model, dataloader, report):
             ev = get(nxt)
             _prefetch(ev, nxt, pipe, apipe)
         while nxt is not None:
-            ev.run(report=report)
+            ev.run(report=report, scores=sc is not None)
             total += ev.rows
             nxt = next(it, None)
             if nxt is not None:
                 ev = get(nxt)
                 _prefetch(ev, nxt, pipe, apipe)
-        res = torch.cat([counts, torch.tensor([total], device=dev, dtype=torch.int64)] + ([conf] if report else []))
+        parts = [counts, torch.tensor([total], device=dev, dtype=torch.int64)] + ([conf] if report else [])
+        if sc is not None:
+            parts += [sc.state[1:], torch.tensor([capacity, max(total - capacity, 0), total * total, sc.capacity,
+                                                  sc.capacity * sc.capacity], device=dev, dtype=torch.int64)]
+        res = torch.cat(parts)
         if sharded:
             torch.distributed.all_reduce(res)
+        if sc is not None:
+            g = _gather_scores(sc, res, total) if sharded else sc
+            if g is not None:
+                g.average_precision()
+                res = torch.cat([res, g.ap.view(-1).view(torch.int64), g.support, g.nonfinite])
         res = res.cpu()  # the one D2H of the evaluation
     inner.args.drop = 1
     return res
+
+
+def _gather_scores(sc, res, rows):
+    """Every rank's stored rows (all_gather_into_tensor of the score and label stores) in one EvalScores of W x rows
+    rows, or None when the all-reduced tail of `res` shows that the ranks cannot be gathered: a rank ran out of store
+    rows, or the ranks evaluated different numbers of rows or hold stores of different sizes (checked as
+    sum^2 == W x sum of squares, so every rank takes the same decision).  ChunkShardBatchSampler with drop_last gives
+    every rank the same rows."""
+    W = torch.distributed.get_world_size()
+    overflow = int(res[-9])
+    _, beyond, rows_sq, caps, caps_sq = res[-5:].tolist()  # the only read before the gather
+    total = int(res[3])
+    if overflow or beyond or total * total != W * rows_sq or caps * caps != W * caps_sq:
+        return None
+    g = sc.gathered
+    if g is None or g.capacity != max(W * rows, 1) or g.flat.numel() != W * sc.store.numel():
+        g = sc.gathered = EvalScores(sc.n, max(W * rows, 1), sc.store.device)
+        g.flat = torch.empty(W * sc.store.numel(), device=sc.store.device)
+        g.flat_labels = torch.empty(W * sc.capacity, dtype=torch.int32, device=sc.store.device)
+    torch.distributed.all_gather_into_tensor(g.flat, sc.store.view(-1))
+    torch.distributed.all_gather_into_tensor(g.flat_labels, sc.labels)
+    n, cap = sc.n, sc.capacity
+    if rows:
+        g.store.view(3, n, W, rows).copy_(g.flat.view(W, 3, n, cap)[..., :rows].permute(1, 2, 0, 3))
+        g.labels.view(W, rows).copy_(g.flat_labels.view(W, cap)[:, :rows])
+    g.cursor.fill_(W * rows)
+    return g
 
 
 def valid(args, model, device, dataloader):
@@ -274,25 +321,58 @@ class EvalReport:
     support    int64 [n]: rows per true class (the row sums, the same for every head)
     correct    int64 [3, n]: the diagonals
     acc, acc_a, acc_v   the traces over max(total, 1): what valid() returns for the same loader
-    per_class  float64 [3, n]: correct / support, NaN for a class without samples"""
+    per_class  float64 [3, n]: correct / support, NaN for a class without samples
+    With valid_report(ap=True) (None otherwise):
+    ap         float64 [3, n]: average precision of every head and class on the softmax scores (sklearn's
+               average_precision_score, ties included), NaN for a class without samples (sklearn gives 0.0 there)
+    map, map_a, map_v   the mean AP over the classes with samples (NaN when there is none)
+    k          the k of the top-k accuracy (5, or n when there are fewer classes)
+    hits       int64 [3]: rows whose label ranks < k in each head's logits (the arg-max order)
+    top5, top5_a, top5_v   hits / max(total, 1)
+    nonfinite  rows with a non-finite score in some head (counted, not raised)"""
 
-    def __init__(self, confusion, total):
+    def __init__(self, confusion, total, ap=None, hits=None, k=None, nonfinite=None):
         self.confusion = confusion
         self.total = int(total)
         self.n = confusion.shape[-1]
         self.support = confusion[0].sum(1)
         self.correct = confusion.diagonal(dim1=1, dim2=2).clone()
-        hits = self.correct.sum(1).tolist()
+        hits_1 = self.correct.sum(1).tolist()
         den = max(self.total, 1)
-        self.acc, self.acc_a, self.acc_v = hits[0] / den, hits[1] / den, hits[2] / den
+        self.acc, self.acc_a, self.acc_v = hits_1[0] / den, hits_1[1] / den, hits_1[2] / den
         self.per_class = torch.where(self.support > 0, self.correct.double() / self.support.clamp(min=1).double(),
                                      torch.tensor(float("nan"), dtype=torch.float64))
+        self.ap, self.hits, self.k = ap, hits, k
+        self.nonfinite = None if nonfinite is None else int(nonfinite)
+        self.map = self.map_a = self.map_v = self.top5 = self.top5_a = self.top5_v = None
+        if ap is not None:
+            present = self.support > 0
+            m = [ap[h][present].mean().item() if bool(present.any()) else float("nan") for h in range(3)]
+            self.map, self.map_a, self.map_v = m
+            t = [int(x) / den for x in hits]
+            self.top5, self.top5_a, self.top5_v = t
 
     def rows(self, epoch):
         """[epoch, head, class, support, correct, accuracy] for every head and class (accuracy 'nan' for an empty
         class): the rows of main_dgl.py --per_class's per-class CSV."""
         sup, cor, acc = self.support.tolist(), self.correct.tolist(), self.per_class.tolist()
         return [[epoch, HEADS[h], c, sup[c], cor[h][c], acc[h][c]] for h in range(3) for c in range(self.n)]
+
+    def ap_rows(self, epoch):
+        """Per head: [epoch, head, class, support, ap] for every class (ap nan for an empty class), then
+        [epoch, head, 'mAP', classes with samples, map] and [epoch, head, 'top5', total, top-5 accuracy] (the label
+        is 'top<k>'): the rows of main_dgl.py --ap's CSV."""
+        if self.ap is None:
+            raise ValueError("ap_rows() needs a report of valid_report(ap=True)")
+        sup, ap = self.support.tolist(), self.ap.tolist()
+        present = int((self.support > 0).sum())
+        maps, tops = (self.map, self.map_a, self.map_v), (self.top5, self.top5_a, self.top5_v)
+        out = []
+        for h in range(3):
+            out += [[epoch, HEADS[h], c, sup[c], ap[h][c]] for c in range(self.n)]
+            out.append([epoch, HEADS[h], "mAP", present, maps[h]])
+            out.append([epoch, HEADS[h], "top%d" % self.k, self.total, tops[h]])
+        return out
 
     def table(self):
         """The per-class accuracies as text: one line per class, one column per head."""
@@ -302,15 +382,51 @@ class EvalReport:
             lines.append("{:>5} {:>7} {:>8.4f} {:>8.4f} {:>8.4f}".format(c, sup, acc[0][c], acc[1][c], acc[2][c]))
         return "\n".join(lines)
 
+    def ap_table(self):
+        """The per-class average precisions as text: one line per class, one column per head, then the mAP line."""
+        ap = self.ap.tolist()
+        lines = ["{:>5} {:>7} {:>8} {:>8} {:>8}".format("class", "support", *HEADS)]
+        for c, sup in enumerate(self.support.tolist()):
+            lines.append("{:>5} {:>7} {:>8.4f} {:>8.4f} {:>8.4f}".format(c, sup, ap[0][c], ap[1][c], ap[2][c]))
+        lines.append("{:>5} {:>7} {:>8.4f} {:>8.4f} {:>8.4f}".format("mAP", int((self.support > 0).sum()), self.map,
+                                                                     self.map_a, self.map_v))
+        return "\n".join(lines)
 
-def valid_report(args, model, device, dataloader):
+
+def valid_report(args, model, device, dataloader, ap=False, topk=5):
     """valid() with the per-class confusion matrices of the three heads (EvalReport), counted on the device by
     gdl_eval_confusion in the same graph-captured pass and read with the counts in its one D2H (one all-reduce for a
     sharded loader).  Same args.drop flips, print and accuracies as valid().  Raises ValueError when a label is >= the
-    head width (the reference fails with an IndexError on `num[label]`)."""
-    res = _evaluate(model, dataloader, True)
+    head width (the reference fails with an IndexError on `num[label]`).
+    ap=True: the same pass also appends every row's softmax scores to a device store (gdl_eval_scores, room for
+    len(dataloader) x the first batch's rows) and counts the top-`topk` hits; gdl_eval_ap then computes the per-class
+    average precision, read in the same D2H.  A sharded loader's stores are gathered so that every rank computes the
+    AP of all the rows, bit for bit the same.  Raises ValueError for a loader without len(), for more rows than the
+    store holds, and for a sharded loader whose ranks evaluated different numbers of rows."""
+    if ap:
+        try:
+            len(dataloader)
+        except TypeError:
+            raise ValueError("valid_report(ap=True) sizes its score store as len(loader) x the first batch's rows; "
+                             "{} has no len()".format(type(dataloader).__name__)) from None
+    res = _evaluate(model, dataloader, True, topk if ap else None)
     n = getattr(model, "module", model).n_classes
     if int(res[4]):
         raise ValueError("{} evaluated rows have a label outside the {} classes of the heads (0..{})"
                          .format(int(res[4]), n, n - 1))
-    return EvalReport(res[5:].view(3, n, n), int(res[3]))
+    base = 5 + 3 * n * n
+    conf, total = res[5:base].view(3, n, n), int(res[3])
+    if not ap:
+        return EvalReport(conf, total)
+    overflow, capacity, beyond = int(res[base]), int(res[base + 4]), int(res[base + 5])
+    if overflow or beyond:
+        raise ValueError("{} evaluated rows do not fit in the {} rows of the score store (len(loader) x the first "
+                         "batch's rows{})".format(total, capacity, ", over all ranks" if _sharded(dataloader) else ""))
+    if res.numel() == base + 9:
+        raise ValueError("average precision over a sharded test loader needs the same number of rows on every rank "
+                         "(ChunkShardBatchSampler with drop_last): {} rows over {} ranks"
+                         .format(total, _world()))
+    tail = res[base + 9:]
+    k = max(1, min(int(topk), n))
+    return EvalReport(conf, total, ap=tail[:3 * n].view(torch.float64).view(3, n).clone(),
+                      hits=res[base + 1:base + 4].clone(), k=k, nonfinite=int(tail[-1]))

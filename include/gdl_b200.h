@@ -279,6 +279,27 @@ int gdl_eval_count(const float* logits, const int64_t* labels, int64_t* counts, 
  * 1 <= n <= 512, B > 0. */
 int gdl_eval_confusion(const float* logits, const int64_t* labels, int64_t* conf, int64_t* out_of_range, int B, int n,
                        gdl_stream_t s);
+/* Scores for average precision and top-k accuracy (opt-in, valid_report(ap=True)).  For h = 0, 1, 2 and every row b
+ * of logits f32 [3][B][n]: p = softmax(logits[h][b]) in fp32 (row maximum subtracted first; fixed summation order) is
+ * written class-major to store f32 [3][n][cap] at row *cursor + b, i.e. store[(h n + c) cap + *cursor + b], and the
+ * label to store_labels int32 [cap] (-1 for a label outside 0..n-1).  hits[h] (int64 [3]) += the rows with a label in
+ * 0..n-1 whose rank #{j : z_j > z_y} + #{j < y : z_j == z_y} (NaN largest, the arg-max order) is < k.  A row whose
+ * store index is >= cap is not written; if its label is >= 0 it adds 1 to *overflow.  Then *cursor += B (a second,
+ * one-thread launch), so a captured graph appends batch after batch.  1 <= n <= 512, 1 <= k <= n, B > 0,
+ * 1 <= cap <= 2^28; all pointers are device pointers. */
+int gdl_eval_scores(const float* logits, const int64_t* labels, int B, int n, int k, float* store,
+                    int32_t* store_labels, int64_t cap, int64_t* cursor, int64_t* hits, int64_t* overflow,
+                    gdl_stream_t s);
+/* Per-class average precision over the N = min(*cursor, cap) rows of a gdl_eval_scores store whose label is in
+ * 0..n-1: for column (h, c), AP = (1 / P_c) sum over the P_c rows i with label c of TP(>= s_i) / N(>= s_i), s_i the
+ * row's score, N(>= t) the rows scoring >= t and TP(>= t) the positives among them (sklearn's
+ * average_precision_score, ties included; a NaN score is the largest and ties with NaN).  Writes ap f64 [3][n] (NaN
+ * for a class without rows), support int64 [n] (P_c) and *nonfinite (int64: the rows with a non-finite score in some
+ * column).  Deterministic and bit-identical for any order of the rows.  Stores of more than 16384 rows sort in a
+ * device workspace of gdl_eval_ap_workspace_bytes(cap, n) bytes (0 otherwise; 8-byte aligned). */
+int64_t gdl_eval_ap_workspace_bytes(int64_t cap, int n);
+int gdl_eval_ap(const float* store, const int32_t* store_labels, const int64_t* cursor, int64_t cap, int n, double* ap,
+                int64_t* support, int64_t* nonfinite, void* workspace, int64_t workspace_bytes, gdl_stream_t s);
 /* Gated-head elementwise pieces (reference models/fusion_modules.py:230-250). */
 int gdl_gated_fwd(const float* hx, const float* hy, float* m_out, float* m_x, float* m_y,
                   int64_t numel, gdl_stream_t s);

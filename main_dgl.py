@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """CLI-compatible entry point for the reference's main_dgl.py (same flags, same defaults,
 same prints / csv / checkpoint file names, same evaluation-mode checkpoint loading), running the B200-native DGL step.
-Deviations: no TensorBoard branch; `--resume`, `--synthetic_len`, `--dp_replicas` and `--per_class` are additions.
+Deviations: no TensorBoard branch; `--resume`, `--synthetic_len`, `--dp_replicas`, `--per_class` and `--ap` are
+additions.
 
     python main_dgl.py --train --ckpt_path ckpt --dataset CREMAD --fusion_method concat \
         --fps 3 --alpha 4 --batch_size 64 --audio_path synthetic
@@ -70,27 +71,50 @@ def get_arguments(argv=None):
     parser.add_argument('--per_class', action='store_true',
                         help='evaluate with per-class accuracies of the fused, audio and visual heads: appended to '
                              '<ckpt_path>/<dataset>_<modality>_per_class.csv when training, printed in evaluation mode')
+    parser.add_argument('--ap', action='store_true',
+                        help='evaluate with per-class average precision, mAP and top-5 accuracy of the fused, audio and '
+                             'visual heads: appended to <ckpt_path>/<dataset>_<modality>_ap.csv and printed as an mAP '
+                             'line when training, printed with the per-class table in evaluation mode')
     return parser.parse_args(argv)
 
 
 PER_CLASS_HEADER = ['epoch', 'head', 'class', 'support', 'correct', 'accuracy']
+AP_HEADER = ['epoch', 'head', 'class', 'support', 'ap']
 
 
-def evaluate_epoch(args, model, device, loader, epoch, rank=0):
-    """The evaluation pass of a training epoch: valid() (acc, acc_a, acc_v), or with --per_class valid_report(),
-    whose accuracies are the same; rank 0 then appends the epoch's per-class rows to
-    <ckpt_path>/<dataset>_<modality>_per_class.csv (a header first when the file is new)."""
-    if not args.per_class:
+def _append_csv(path, header, rows):
+    new = not os.path.exists(path)
+    with open(path, 'a+', newline='') as f:
+        w = csv.writer(f)
+        if new:
+            w.writerow(header)
+        w.writerows(rows)
+
+
+def ap_line(report):
+    """The --ap summary line of an EvalReport of valid_report(ap=True)."""
+    return 'mAP: {:.4f}, Audio mAP: {:.4f}, Visual mAP: {:.4f}, Top-{} Acc: {:.4f}'.format(
+        report.map, report.map_a, report.map_v, report.k, report.top5)
+
+
+def evaluate_epoch(args, model, device, loader, epoch, rank=0, reports=None):
+    """The evaluation pass of a training epoch: valid() (acc, acc_a, acc_v), or with --per_class / --ap
+    valid_report(), whose accuracies are the same; rank 0 then appends the epoch's per-class rows to
+    <ckpt_path>/<dataset>_<modality>_per_class.csv (--per_class) and its AP rows to
+    <ckpt_path>/<dataset>_<modality>_ap.csv (--ap), a header first when a file is new.  The report is appended to
+    `reports` when given."""
+    use_ap = getattr(args, 'ap', False)
+    if not args.per_class and not use_ap:
         return valid(args, model, device, loader)
-    report = valid_report(args, model, device, loader)
+    report = valid_report(args, model, device, loader, ap=True) if use_ap else valid_report(args, model, device, loader)
     if rank == 0:
-        path = os.path.join(args.ckpt_path, args.dataset + '_' + args.modality + '_per_class.csv')
-        new = not os.path.exists(path)
-        with open(path, 'a+', newline='') as f:
-            w = csv.writer(f)
-            if new:
-                w.writerow(PER_CLASS_HEADER)
-            w.writerows(report.rows(epoch))
+        stem = os.path.join(args.ckpt_path, args.dataset + '_' + args.modality)
+        if args.per_class:
+            _append_csv(stem + '_per_class.csv', PER_CLASS_HEADER, report.rows(epoch))
+        if use_ap:
+            _append_csv(stem + '_ap.csv', AP_HEADER, report.ap_rows(epoch))
+    if reports is not None:
+        reports.append(report)
     return report.acc, report.acc_a, report.acc_v
 
 
@@ -205,7 +229,8 @@ def main(argv=None):
             if shard_sampler is not None:
                 from gdl_b200.parallel import assert_same_order
                 assert_same_order(shard_sampler.order_digest)
-            acc, acc_a, acc_v = evaluate_epoch(args, model, device, test_loader, epoch, rank)
+            reports = []
+            acc, acc_a, acc_v = evaluate_epoch(args, model, device, test_loader, epoch, rank, reports)
             if rank == 0:
                 with open(log, 'a+', newline='') as f:
                     csv.writer(f).writerow([acc, acc_a, acc_v])
@@ -226,6 +251,8 @@ def main(argv=None):
             else:
                 print("Loss: {:.3f}, Acc: {:.3f}, Best Acc: {:.3f}".format(batch_loss, acc, best_acc))
             print("Audio Acc: {:.3f}， Visual Acc: {:.3f} ".format(acc_a, acc_v))
+            if args.ap:
+                print(ap_line(reports[0]))
             print("Audio similar: {:.3f}， Visual similar: {:.3f} ".format(a_div, v_div))
             print("Audio regurize: {:.3f}， Visual regurize: {:.3f} ".format(a_re, v_re))
     else:
@@ -241,15 +268,23 @@ def main(argv=None):
             'inconsistency between fusion method of loaded model and args !'
         model.load_state_dict(loaded_dict['model'])
         print('Trained model loaded!')
-        if args.per_class:
+        if args.ap:
+            report = valid_report(args, model, device, test_loader, ap=True)
+            acc, acc_a, acc_v = report.acc, report.acc_a, report.acc_v
+        elif args.per_class:
             report = valid_report(args, model, device, test_loader)
             acc, acc_a, acc_v = report.acc, report.acc_a, report.acc_v
         else:
             acc, acc_a, acc_v = valid(args, model, device, test_loader)
         print('Accuracy: {}, accuracy_a: {}, accuracy_v: {}'.format(acc, acc_a, acc_v))
+        if args.ap:
+            print(ap_line(report))
         if args.per_class:
             print('Per-class accuracy ({} samples):'.format(report.total))
             print(report.table())
+        if args.ap:
+            print('Per-class average precision ({} samples):'.format(report.total))
+            print(report.ap_table())
 
 
 if __name__ == "__main__":
