@@ -104,14 +104,18 @@ __global__ void grad_stats_finalize_kernel(const float* __restrict__ partial, in
   }
 }
 
+// lr_dev (may be NULL => lr): the learning rate as one float64 in device memory, cast to float here as ctypes casts
+// a Python float passed as lr, so a captured update follows a per-iteration lr schedule without re-capture.
 __global__ void __launch_bounds__(256) sgd_momentum_kernel(float* __restrict__ param,
                                                            float* __restrict__ grad,
                                                            float* __restrict__ buf, int64_t n4,
-                                                           int64_t numel, float lr, float mu,
+                                                           int64_t numel, float lr_host,
+                                                           const double* __restrict__ lr_dev, float mu,
                                                            float wd, int first,
                                                            const float* __restrict__ stats) {
   pdl_enter();
   const float coef = stats ? stats[1] : 1.f;
+  const float lr = lr_dev ? (float)*lr_dev : lr_host;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
        i += (int64_t)gridDim.x * blockDim.x) {
     float4 p = reinterpret_cast<float4*>(param)[i];
@@ -143,14 +147,16 @@ __global__ void __launch_bounds__(256) sgd_momentum_kernel(float* __restrict__ p
 }
 
 // ---- Adam / Adagrad (torch.optim.Adam / Adagrad, non-capturable single-tensor and foreach formulas) ----
-// The update runs inside a CUDA graph captured once per lr, so the step count cannot be a kernel argument: it lives
-// in step_state[0] on the device.  One thread advances it and writes the step's scalars into step_state[1..2]
-// before the element kernel reads them (stream order), so every block of the element kernel sees the same step.
+// The update runs inside a CUDA graph captured once, so the step count cannot be a kernel argument: it lives in
+// step_state[0] on the device, and so may the lr (lr_dev, one float64; NULL => lr_host).  One thread advances the
+// count and writes the step's scalars into step_state[1..2] before the element kernel reads them (stream order), so
+// every block of the element kernel sees the same step.
 enum { kRuleAdam = 0, kRuleAdagrad = 1 };
 
-__global__ void optim_step_prologue_kernel(int32_t* __restrict__ step_state, int rule, double lr, double a,
-                                           double b) {
+__global__ void optim_step_prologue_kernel(int32_t* __restrict__ step_state, int rule, double lr_host,
+                                           const double* __restrict__ lr_dev, double a, double b) {
   pdl_enter();
+  const double lr = lr_dev ? *lr_dev : lr_host;
   const int32_t step = step_state[0] + 1;
   step_state[0] = step;
   float* f = reinterpret_cast<float*>(step_state + 1);
@@ -314,26 +320,28 @@ extern "C" int gdl_grad_stats(const float* grad, int64_t numel, const int64_t* s
   return GDL_OK;
 }
 
-extern "C" int gdl_sgd_momentum(float* param, float* grad, float* momentum_buf, int64_t numel,
-                                float lr, float mu, float wd, int first_step, const float* stats,
-                                gdl_stream_t s) {
+// The host-lr entries and the device-lr entries (*_lr_dev) launch the same kernels: lr_dev NULL selects lr_host.
+static int sgd_momentum_launch(float* param, float* grad, float* momentum_buf, int64_t numel, float lr,
+                               const double* lr_dev, float mu, float wd, int first_step, const float* stats,
+                               gdl_stream_t s) {
   GDL_REQUIRE(param && grad && momentum_buf && numel > 0, "gdl_sgd_momentum: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)momentum_buf) & 15) == 0,
               "gdl_sgd_momentum: arenas must be 16-byte aligned");
   launch_pdl(sgd_momentum_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, momentum_buf,
-             numel / 4, numel, lr, mu, wd, first_step, stats);
+             numel / 4, numel, lr, lr_dev, mu, wd, first_step, stats);
   GDL_CHECK_LAUNCH("sgd_momentum_kernel");
   return GDL_OK;
 }
 
-extern "C" int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
-                        int64_t numel, double lr, double beta1, double beta2, double eps, double wd,
-                        const float* stats, gdl_stream_t s) {
+static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
+                       int64_t numel, double lr, const double* lr_dev, double beta1, double beta2, double eps,
+                       double wd, const float* stats, gdl_stream_t s) {
   GDL_REQUIRE(param && grad && exp_avg && exp_avg_sq && step_state && numel > 0, "gdl_adam: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
               "gdl_adam: arenas must be 16-byte aligned");
   GDL_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0, "gdl_adam: betas must lie in [0, 1)");
-  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdam, lr, beta1, beta2);
+  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdam, lr, lr_dev, beta1,
+             beta2);
   GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
   launch_pdl(adam_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, exp_avg, exp_avg_sq,
              numel / 4, numel, (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)eps, (float)wd,
@@ -342,17 +350,58 @@ extern "C" int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_av
   return GDL_OK;
 }
 
-extern "C" int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
-                           double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s) {
+static int adagrad_launch(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
+                          const double* lr_dev, double lr_decay, double eps, double wd, const float* stats,
+                          gdl_stream_t s) {
   GDL_REQUIRE(param && grad && sum && step_state && numel > 0, "gdl_adagrad: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)sum) & 15) == 0,
               "gdl_adagrad: arenas must be 16-byte aligned");
-  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdagrad, lr, lr_decay, 0.0);
+  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdagrad, lr, lr_dev,
+             lr_decay, 0.0);
   GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
   launch_pdl(adagrad_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, sum, numel / 4, numel,
              (float)eps, (float)wd, stats, (const int32_t*)step_state);
   GDL_CHECK_LAUNCH("adagrad_kernel");
   return GDL_OK;
+}
+
+extern "C" int gdl_sgd_momentum(float* param, float* grad, float* momentum_buf, int64_t numel,
+                                float lr, float mu, float wd, int first_step, const float* stats,
+                                gdl_stream_t s) {
+  return sgd_momentum_launch(param, grad, momentum_buf, numel, lr, nullptr, mu, wd, first_step, stats, s);
+}
+
+extern "C" int gdl_sgd_momentum_lr_dev(float* param, float* grad, float* momentum_buf, int64_t numel,
+                                       const double* lr, float mu, float wd, int first_step, const float* stats,
+                                       gdl_stream_t s) {
+  GDL_REQUIRE(lr, "gdl_sgd_momentum_lr_dev: null lr");
+  return sgd_momentum_launch(param, grad, momentum_buf, numel, 0.f, lr, mu, wd, first_step, stats, s);
+}
+
+extern "C" int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
+                        int64_t numel, double lr, double beta1, double beta2, double eps, double wd,
+                        const float* stats, gdl_stream_t s) {
+  return adam_launch(param, grad, exp_avg, exp_avg_sq, step_state, numel, lr, nullptr, beta1, beta2, eps, wd, stats,
+                     s);
+}
+
+extern "C" int gdl_adam_lr_dev(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
+                               int64_t numel, const double* lr, double beta1, double beta2, double eps, double wd,
+                               const float* stats, gdl_stream_t s) {
+  GDL_REQUIRE(lr, "gdl_adam_lr_dev: null lr");
+  return adam_launch(param, grad, exp_avg, exp_avg_sq, step_state, numel, 0.0, lr, beta1, beta2, eps, wd, stats, s);
+}
+
+extern "C" int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
+                           double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s) {
+  return adagrad_launch(param, grad, sum, step_state, numel, lr, nullptr, lr_decay, eps, wd, stats, s);
+}
+
+extern "C" int gdl_adagrad_lr_dev(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel,
+                                  const double* lr, double lr_decay, double eps, double wd, const float* stats,
+                                  gdl_stream_t s) {
+  GDL_REQUIRE(lr, "gdl_adagrad_lr_dev: null lr");
+  return adagrad_launch(param, grad, sum, step_state, numel, 0.0, lr, lr_decay, eps, wd, stats, s);
 }
 
 extern "C" int gdl_grad_accumulate(float* dst, const float* src, int64_t numel, int accumulate, gdl_stream_t s) {

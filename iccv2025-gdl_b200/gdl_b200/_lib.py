@@ -108,6 +108,9 @@ SIGNATURES = {
     "gdl_sgd_momentum": (_i, [_p, _p, _p, _l, _f, _f, _f, _i, _p, _p]),
     "gdl_adam": (_i, [_p, _p, _p, _p, _p, _l, _d, _d, _d, _d, _d, _p, _p]),
     "gdl_adagrad": (_i, [_p, _p, _p, _p, _l, _d, _d, _d, _d, _p, _p]),
+    "gdl_sgd_momentum_lr_dev": (_i, [_p, _p, _p, _l, _p, _f, _f, _i, _p, _p]),
+    "gdl_adam_lr_dev": (_i, [_p, _p, _p, _p, _p, _l, _p, _d, _d, _d, _d, _p, _p]),
+    "gdl_adagrad_lr_dev": (_i, [_p, _p, _p, _p, _l, _p, _d, _d, _d, _p, _p]),
     "gdl_grad_accumulate": (_i, [_p, _p, _l, _i, _p]),
     "gdl_check_conv_fwd": (_i, [_dp, _i, _p, _p, _p, _p]),
     "gdl_check_conv_dgrad": (_i, [_dp, _i, _p, _p, _p, _p, _p]),

@@ -556,23 +556,49 @@ def grad_stats(grad, numel, seg_end, seg_group, seg_inv_numel, nseg, max_norm, s
                                      _stream()), "gdl_grad_stats")
 
 
+def _lr_dev(lr):
+    """The device pointer of an lr held in device memory (a float64 CUDA tensor of one element), or None for a Python
+    number (the host-lr entries)."""
+    if not isinstance(lr, torch.Tensor):
+        return None
+    assert lr.is_cuda and lr.dtype == torch.float64 and lr.numel() == 1, "a device lr is one float64 on the GPU"
+    return _ptr(lr)
+
+
+# lr: a Python number, or a float64 CUDA tensor of one element that the update reads on the device (the *_lr_dev
+# entries: a captured update then follows whatever the tensor holds when it is replayed)
 @_op("sgd_momentum", 1, lambda param, grad, buf, numel, *a: ("bytes", 24.0 * numel))
 def sgd_momentum(param, grad, buf, numel, lr, mu, wd, first_step, stats):
-    check(_lib.load().gdl_sgd_momentum(_ptr(param), _ptr(grad), _ptr(buf), numel, lr, mu, wd,
-                                       int(first_step), _ptr(stats), _stream()), "gdl_sgd_momentum")
+    lib, dev = _lib.load(), _lr_dev(lr)
+    if dev is None:
+        check(lib.gdl_sgd_momentum(_ptr(param), _ptr(grad), _ptr(buf), numel, lr, mu, wd, int(first_step),
+                                   _ptr(stats), _stream()), "gdl_sgd_momentum")
+    else:
+        check(lib.gdl_sgd_momentum_lr_dev(_ptr(param), _ptr(grad), _ptr(buf), numel, dev, mu, wd, int(first_step),
+                                          _ptr(stats), _stream()), "gdl_sgd_momentum_lr_dev")
 
 
 # Adam / Adagrad: step_state is the int32 [3] device counter of include/gdl_b200.h (one launch advances it, one updates)
 @_op("adam", 2, lambda param, grad, m, v, step_state, numel, *a: ("bytes", 32.0 * numel))
 def adam(param, grad, exp_avg, exp_avg_sq, step_state, numel, lr, beta1, beta2, eps, wd, stats):
-    check(_lib.load().gdl_adam(_ptr(param), _ptr(grad), _ptr(exp_avg), _ptr(exp_avg_sq), _ptr(step_state), numel,
-                               lr, beta1, beta2, eps, wd, _ptr(stats), _stream()), "gdl_adam")
+    lib, dev = _lib.load(), _lr_dev(lr)
+    if dev is None:
+        check(lib.gdl_adam(_ptr(param), _ptr(grad), _ptr(exp_avg), _ptr(exp_avg_sq), _ptr(step_state), numel, lr,
+                           beta1, beta2, eps, wd, _ptr(stats), _stream()), "gdl_adam")
+    else:
+        check(lib.gdl_adam_lr_dev(_ptr(param), _ptr(grad), _ptr(exp_avg), _ptr(exp_avg_sq), _ptr(step_state), numel,
+                                  dev, beta1, beta2, eps, wd, _ptr(stats), _stream()), "gdl_adam_lr_dev")
 
 
 @_op("adagrad", 2, lambda param, grad, s, step_state, numel, *a: ("bytes", 24.0 * numel))
 def adagrad(param, grad, state_sum, step_state, numel, lr, lr_decay, eps, wd, stats):
-    check(_lib.load().gdl_adagrad(_ptr(param), _ptr(grad), _ptr(state_sum), _ptr(step_state), numel, lr, lr_decay,
-                                  eps, wd, _ptr(stats), _stream()), "gdl_adagrad")
+    lib, dev = _lib.load(), _lr_dev(lr)
+    if dev is None:
+        check(lib.gdl_adagrad(_ptr(param), _ptr(grad), _ptr(state_sum), _ptr(step_state), numel, lr, lr_decay, eps,
+                              wd, _ptr(stats), _stream()), "gdl_adagrad")
+    else:
+        check(lib.gdl_adagrad_lr_dev(_ptr(param), _ptr(grad), _ptr(state_sum), _ptr(step_state), numel, dev,
+                                     lr_decay, eps, wd, _ptr(stats), _stream()), "gdl_adagrad_lr_dev")
 
 
 @_op("grad_accumulate", 1, lambda dst, src, numel, accumulate: ("bytes", (12.0 if accumulate else 8.0) * numel))

@@ -33,7 +33,7 @@ _SEG_ALIGN = 64  # floats; keeps every tensor 256-byte aligned inside the arenas
 # reference main_dgl.py:244 nn.DataParallel's reduce-add).  0 = one all-reduce after the whole backward.
 AR_OVERLAP = os.environ.get("GDL_AR_OVERLAP", "1") != "0"
 
-# The step is captured lazily (second step, and again when MultiStepLR changes lr) while a DataLoader's pin-memory
+# The step is captured lazily (on its second step, once for its lifetime) while a DataLoader's pin-memory
 # thread may be calling cudaHostAlloc / cudaEventQuery: in the default "global" capture mode those calls from OTHER
 # threads are illegal and can invalidate the capture; "thread_local" restricts the check to the capturing thread.
 _CAPTURE_MODE = "thread_local"
@@ -138,6 +138,9 @@ class ParamArena:
         # on the device (also under CUDA-graph replay), `steps` the host's, advanced by DGLStep.step; `step_tensors`
         # are the CPU tensors train.adopt_momentum put into optimizer.state[p]['step'], refreshed by sync_step_tensors.
         self.step_state = torch.zeros(3, device=device, dtype=torch.int32)
+        # the lr the update reads on the device (one float64): DGLStep.step writes it before every step, so a captured
+        # update follows any lr schedule without re-capture
+        self.lr = torch.zeros(1, device=device, dtype=torch.float64)
         self.steps = 0
         self.step_tensors = {}
         for p, o in zip(self.params, self.offsets):
@@ -343,8 +346,7 @@ class DGLStep:
         self.stream_v = torch.cuda.Stream(dev, priority=-1 if prio == 1 else 0)
         self.steps_done = 0
         self.momentum_loaded = False  # set by train.adopt_momentum when a checkpoint's buffers were copied in
-        self.graphs = GraphCache()  # the device runs of the schedule, captured for self._graph_lr
-        self._graph_lr = None
+        self.graphs = GraphCache()  # the device runs of the schedule, captured once
         self.launches_per_step = None
         # gradient buckets (views of the gradient arena; arena order: head | audio | visual)
         self.overlap = AR_OVERLAP and world_size > 1
@@ -366,8 +368,8 @@ class DGLStep:
 
     # ------------------------------------------------------------------ the segments of schedule()
     def _enqueue(self, seg):
-        """Enqueue one segment on the current stream (+ the two encoder streams).  Every segment reads the streams,
-        lr and the rest of the step's state when it is enqueued."""
+        """Enqueue one segment on the current stream (+ the two encoder streams).  Every segment reads the streams
+        and the rest of the step's state when it is enqueued; the update reads the lr from the arena on the device."""
         name, arg = seg
         if name == "inputs":
             self.stage.stage_rows(arg, self.replicas, self.B, self.enc_a, self.enc_v, self.label_in)
@@ -426,7 +428,7 @@ class DGLStep:
 
     def _enqueue_update(self):
         """Clip statistics + diagnostics + optimizer update + bf16 shadow refresh (after the all-reduce)."""
-        ar, r, lr = self.arena, self.rule, self.lr
+        ar, r, lr = self.arena, self.rule, self.arena.lr
         ops.grad_stats(ar.grad, ar.numel, ar.seg_end, ar.seg_group, ar.seg_inv, ar.nseg, self.max_norm,
                        ar.scratch, self.stats[4:8])
         if r.kind == "sgd":
@@ -469,16 +471,16 @@ class DGLStep:
         self.stage.prefetch(spec, image, label, pipeline, audio_pipeline)
 
     def step(self, spec=None, image=None, label=None, lr=None):
-        """Run one training step; returns the device tensor `stats` (8 floats, see __init__)."""
+        """Run one training step at learning rate `lr` (default: the last one given, initially the rule's); returns
+        the device tensor `stats` (8 floats, see __init__)."""
         if lr is not None:
             self.lr = lr
+        # stream-ordered behind the previous step's update, which read the arena's lr
+        self.arena.lr.fill_(self.lr)
         if spec is not None:
             self.load_inputs(spec, image, label)
         eager = self.steps_done == 0 or not self.use_graph
         if not eager:
-            if self._graph_lr != self.lr:
-                self.graphs.clear()
-                self._graph_lr = self.lr
             for run in self._runs:
                 if run[0][0] in DEVICE:
                     self.graphs.capture(run, lambda run=run: [self._enqueue(seg) for seg in run])

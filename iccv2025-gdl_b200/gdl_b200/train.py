@@ -8,6 +8,9 @@ in is only read for its update rule, hyper-parameters and lr schedule (gdl_b200.
 Adam or Adagrad; anything else raises) — the update itself is a fused kernel over the parameter arena (its state is
 exposed through `optimizer.state[p]` — `momentum_buffer`, `exp_avg` / `exp_avg_sq` / `step`, `sum` / `step` — so
 reference-format checkpoints still carry it).
+`train_epoch(..., step_scheduler=)` is an addition: an lr scheduler stepped once per optimizer step (warm-up, cosine
+decay, OneCycleLR), which the captured step follows without re-capture; a scheduler that changes another setting of
+the optimizer (momentum, betas, weight decay, ...) is refused (gdl_b200.optim.follow_rule).
 `valid_report` is an addition: `valid` plus the per-class confusion matrices of the three heads (EvalReport), and
 with ap=True the per-class average precision, mAP and top-k accuracy of the three heads.
 """
@@ -15,7 +18,7 @@ import csv
 
 import torch
 
-from .optim import update_rule
+from .optim import follow_rule, update_rule
 from .parallel import ChunkShardBatchSampler, broadcast_running_stats, replicas_per_rank
 from .step import DGLStep, EvalScores, eval_confusion, eval_counts, eval_scores, get_eval_step
 
@@ -139,7 +142,10 @@ def adopt_momentum(arena, optimizer, step=None):
     return loaded
 
 
-def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, writer=None):
+def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, writer=None, step_scheduler=None):
+    """scheduler: stepped at the start of the epoch, like the reference's MultiStepLR.  step_scheduler (a
+    torch.optim.lr_scheduler.LRScheduler) is stepped right after every optimizer step, torch's per-iteration
+    convention: step k of a run trains with the lr the schedule gives after k of its steps.  Either may be None."""
     if scheduler is not None:
         scheduler.step()  # stepped at epoch START like the reference (main_dgl.py:73-74)
     if epoch < 20:
@@ -179,7 +185,10 @@ def train_epoch(args, epoch, model, device, dataloader, optimizer, scheduler, wr
         spec, image, label = nxt
         if hist is None:
             hist = torch.zeros(LOG_EVERY, 8, device=st.device)
+        follow_rule(optimizer, st.rule)
         stats = st.step(lr=optimizer.param_groups[0]['lr'])
+        if step_scheduler is not None:
+            step_scheduler.step()
         nxt = next(it, None)
         if nxt is not None:
             st2 = _get_step(args, model, optimizer, nxt[0], nxt[1], pipe, apipe)

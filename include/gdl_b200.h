@@ -404,7 +404,7 @@ int gdl_sgd_momentum(float* param, float* grad, float* momentum_buf, int64_t num
  * weight decay).  step_state int32 [3], device memory owned by the caller: [0] is the step count t (0 before the
  * first update, torch's state['step']), [1..2] scratch.  Each call launches a one-thread kernel that advances
  * t by one and derives the step's scalars from it in double precision, then the element kernel, so the count
- * advances on every replay of a captured graph and lr is the only host-side argument that changes the result.
+ * advances on every replay of a captured graph (the *_lr_dev entries below read the lr on the device too).
  * Adam (32 bytes per element):
  *   g = grad*coef (written back); g += wd*p; m = lerp(m, g, 1-beta1); v = beta2*v + (1-beta2)*g*g;
  *   p -= (lr/(1-beta1^t)) * m / (sqrt(v)/sqrt(1-beta2^t) + eps).
@@ -415,6 +415,18 @@ int gdl_adam(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32
              double lr, double beta1, double beta2, double eps, double wd, const float* stats, gdl_stream_t s);
 int gdl_adagrad(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, double lr,
                 double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s);
+/* The same three updates with the learning rate read from device memory (reference main_dgl.py:154
+ * `optimizer.step()` under an lr scheduler): lr points to ONE float64 that the caller writes, stream-ordered, before
+ * each update, so a graph captured once follows any lr schedule.  Same kernels, launches and results as the host-lr
+ * entries above at the same lr: SGD casts *lr to float (as a float lr argument is rounded), Adam / Adagrad read it
+ * in double in the one-thread kernel. */
+int gdl_sgd_momentum_lr_dev(float* param, float* grad, float* momentum_buf, int64_t numel, const double* lr,
+                            float mu, float wd, int first_step, const float* stats, gdl_stream_t s);
+int gdl_adam_lr_dev(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_state,
+                    int64_t numel, const double* lr, double beta1, double beta2, double eps, double wd,
+                    const float* stats, gdl_stream_t s);
+int gdl_adagrad_lr_dev(float* param, float* grad, float* sum, int32_t* step_state, int64_t numel, const double* lr,
+                       double lr_decay, double eps, double wd, const float* stats, gdl_stream_t s);
 /* Gradient accumulation over several replicas run one after another on one GPU (DGLStep replicas > 1):
  * dst = src (accumulate == 0, 8 bytes per element) or dst = dst + src (accumulate != 0, 12 bytes per element),
  * fp32, element-wise.  dst and src 16-byte aligned, numel > 0 (any value: a scalar tail covers numel % 4). */

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """CLI-compatible entry point for the reference's main_dgl.py (same flags, same defaults,
 same prints / csv / checkpoint file names, same evaluation-mode checkpoint loading), running the B200-native DGL step.
-Deviations: no TensorBoard branch; `--resume`, `--synthetic_len`, `--dp_replicas`, `--per_class` and `--ap` are
-additions.
+Deviations: no TensorBoard branch; `--resume`, `--synthetic_len`, `--dp_replicas`, `--per_class`, `--ap`,
+`--lr_schedule` and `--warmup_steps` are additions.
 
     python main_dgl.py --train --ckpt_path ckpt --dataset CREMAD --fusion_method concat \
         --fps 3 --alpha 4 --batch_size 64 --audio_path synthetic
@@ -26,6 +26,7 @@ import torch.optim as optim  # noqa: E402
 from torch.utils.data import DataLoader  # noqa: E402
 
 from gdl_b200 import AVClassifier_DGL, setup_seed, weight_init  # noqa: E402
+from gdl_b200.optim import warmup_cosine  # noqa: E402
 from gdl_b200.parallel import replicas_per_rank  # noqa: E402
 from gdl_b200.synthetic import SyntheticAV  # noqa: E402
 from gdl_b200.train import train_epoch, valid, valid_report  # noqa: E402
@@ -75,7 +76,30 @@ def get_arguments(argv=None):
                         help='evaluate with per-class average precision, mAP and top-5 accuracy of the fused, audio and '
                              'visual heads: appended to <ckpt_path>/<dataset>_<modality>_ap.csv and printed as an mAP '
                              'line when training, printed with the per-class table in evaluation mode')
+    parser.add_argument('--lr_schedule', default='multistep', type=str, choices=['multistep', 'cosine'],
+                        help="multistep: the reference's MultiStepLR(lr_decay_step, lr_decay_ratio) stepped at every "
+                             "epoch start; cosine: per-iteration linear warm-up over --warmup_steps steps, then cosine "
+                             "decay to 0 at the end of the last epoch")
+    parser.add_argument('--warmup_steps', default=0, type=int, help='warm-up steps of --lr_schedule cosine')
     return parser.parse_args(argv)
+
+
+def check_lr_schedule(args):
+    """ValueError for a --lr_schedule / --warmup_steps combination main() cannot run (before any device work)."""
+    if args.warmup_steps < 0:
+        raise ValueError('--warmup_steps must be >= 0, got {}'.format(args.warmup_steps))
+    if args.warmup_steps and args.lr_schedule != 'cosine':
+        # a per-iteration warm-up beside the per-epoch MultiStepLR would need a second scheduler state in checkpoints
+        raise ValueError('--warmup_steps applies to --lr_schedule cosine only, not {}'.format(args.lr_schedule))
+
+
+def make_schedulers(args, optimizer, steps_per_epoch):
+    """(scheduler, step_scheduler) for train_epoch: the reference's MultiStepLR stepped at epoch start, or with
+    --lr_schedule cosine one LambdaLR stepped per iteration over epochs x steps_per_epoch steps."""
+    if args.lr_schedule == 'multistep':
+        return optim.lr_scheduler.MultiStepLR(optimizer, eval(args.lr_decay_step), args.lr_decay_ratio), None
+    factor = warmup_cosine(args.epochs * steps_per_epoch, args.warmup_steps)
+    return None, optim.lr_scheduler.LambdaLR(optimizer, factor)
 
 
 PER_CLASS_HEADER = ['epoch', 'head', 'class', 'support', 'correct', 'accuracy']
@@ -125,6 +149,7 @@ def main(argv=None):
     setup_seed(args.random_seed)
     if args.backbone != 'resnet':
         raise EOFError  # reference main_dgl.py:236-240
+    check_lr_schedule(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.dp_replicas and args.train:
         replicas_per_rank(args.batch_size, args.dp_replicas, world)  # ValueError before any device or data work
@@ -155,7 +180,6 @@ def main(argv=None):
         optimizer = optim.Adam(model.parameters(), lr=args.learning_rate, betas=(0.9, 0.999), eps=1e-08)
     else:
         raise ValueError('Incorrect optimizer: {}'.format(args.optimizer))  # reference main_dgl.py:259
-    scheduler = optim.lr_scheduler.MultiStepLR(optimizer, eval(args.lr_decay_step), args.lr_decay_ratio)
 
     if args.audio_path not in ('synthetic', 'synthetic_exact', 'synthetic_device'):
         raise NotImplementedError("this environment ships no datasets: pass --audio_path synthetic (random tensors) "
@@ -201,6 +225,8 @@ def main(argv=None):
     else:
         test_loader = DataLoader(test_dataset, batch_size=per_rank, shuffle=False, num_workers=8, pin_memory=True,
                                  drop_last=True)  # the reference drops the test tail too (main_dgl.py:287-288)
+    scheduler, step_scheduler = make_schedulers(args, optimizer, len(train_loader))
+    saved_scheduler = step_scheduler or scheduler  # checkpoints keep it under the reference's 'scheduler' key
 
     start_epoch, best_acc = 0, 0.0
     if args.resume and args.train:
@@ -208,9 +234,13 @@ def main(argv=None):
         # no way to load it back; the optimizer state (momentum, Adam moments, Adagrad sums, step count) is adopted by
         # the fused update on the first batch
         ckpt = torch.load(args.resume, map_location=device)
+        saved = ckpt.get('lr_schedule', 'multistep')  # the reference's checkpoints: MultiStepLR
+        if saved != args.lr_schedule:
+            raise ValueError('{} was trained with --lr_schedule {}; it cannot be resumed with --lr_schedule {}'
+                             .format(args.resume, saved, args.lr_schedule))
         model.load_state_dict(ckpt['model'])
         optimizer.load_state_dict(ckpt['optimizer'])
-        scheduler.load_state_dict(ckpt['scheduler'])
+        saved_scheduler.load_state_dict(ckpt['scheduler'])
         start_epoch = int(ckpt['saved_epoch']) + 1
         best_acc = float(ckpt.get('acc', 0.0))  # a resumed run only overwrites "best" with something better
         print('Resumed from {} (epoch {}, acc {})'.format(args.resume, ckpt['saved_epoch'], ckpt.get('acc')))
@@ -225,7 +255,7 @@ def main(argv=None):
             print('Epoch: {}: '.format(epoch))
             args.epoch_now = epoch
             batch_loss, batch_loss_a, batch_loss_v, a_div, v_div, a_re, v_re = train_epoch(
-                args, epoch, model, device, train_loader, optimizer, scheduler)
+                args, epoch, model, device, train_loader, optimizer, scheduler, step_scheduler=step_scheduler)
             if shard_sampler is not None:
                 from gdl_b200.parallel import assert_same_order
                 assert_same_order(shard_sampler.order_digest)
@@ -244,7 +274,8 @@ def main(argv=None):
                 if rank == 0:
                     torch.save({'saved_epoch': epoch, 'modulation': args.modulation, 'alpha': args.alpha,
                                 'fusion': args.fusion_method, 'acc': acc, 'model': model.state_dict(),
-                                'optimizer': optimizer.state_dict(), 'scheduler': scheduler.state_dict()},
+                                'optimizer': optimizer.state_dict(), 'scheduler': saved_scheduler.state_dict(),
+                                'lr_schedule': args.lr_schedule},
                                os.path.join(args.ckpt_path, name))
                 print('The best model has been saved at {}.'.format(os.path.join(args.ckpt_path, name)))
                 print("Loss: {:.3f}, Acc: {:.3f}".format(batch_loss, acc))
