@@ -103,43 +103,6 @@ __device__ __forceinline__ void st_global32(void* p, const uint4& lo, const uint
 
 static const int kNumSMs = 148;
 
-// ---- programmatic dependent launch (PDL), opt-in: GDL_PDL=1 ----
-// Measured (B200, CUDA-graph-captured step, A/B inside one gpurun call): 20.36 / 20.59 ms per step with PDL against
-// 20.54 / 20.39 ms without at B = 256, and 7.42 against 7.18 ms at 64 samples per GPU (KineticSound shape) — inside a
-// captured graph the kernel-to-kernel gap is already too small for the early launch to pay, and pre-launched CTAs
-// compete with the tail of the running kernel.  Kept behind the switch, off by default.
-// With GDL_PDL=1 every kernel of the training step is launched with cudaLaunchAttributeProgrammaticStreamSerialization: kernel k+1 may be
-// scheduled while kernel k is still running (its CTAs take whatever SM resources are free), runs its prologue
-// (barrier / TMEM set-up, descriptor prefetch, index arithmetic) and blocks in griddepcontrol.wait until kernel k has
-// completed and flushed its memory — so the launch latency and the prologue of k+1 hide under the tail of k instead of
-// sitting between the two (373 launches per step).  Inside CUDA-graph capture these become programmatic dependency edges.
-// Rule: a kernel launched through launch_pdl must execute pdl_wait() (every thread) before its first access to global
-// memory that an earlier kernel may have written, or that an earlier kernel may still be reading when this one writes it.
-// Without the switch everything is launched in plain stream order (the waits are then no-ops).
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_enter() {
-  pdl_launch_dependents();
-  pdl_wait();
-}
-bool pdl_enabled();  // tma.cu: GDL_PDL (default off)
-
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                                     Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 // gdl_set_sweep() hint (elementwise.cu): non-zero = walk pixel ranges in descending order
 extern thread_local int g_sweep_rev;
 

@@ -446,7 +446,6 @@ __global__ void pack_weights_kernel(const float* __restrict__ w, bf16* __restric
 // Multi-tensor variant: one launch refreshes the bf16 shadows of a whole encoder (reference
 // main_dgl.py:154 optimizer.step() is followed by nothing — the shadows are this library's own state).
 __global__ void pack_weights_multi_kernel(const gdl_pack_entry* __restrict__ tab, int n, int64_t total) {
-  pdl_enter();
   for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (int64_t)gridDim.x * blockDim.x) {
     int lo = 0, hi = n - 1;  // last entry with start <= idx
@@ -478,7 +477,6 @@ __global__ void pack_weights_multi_kernel(const gdl_pack_entry* __restrict__ tab
 // coalesced fp32 reads (64*R*S contiguous floats per co), 128-byte runs into wp[co][tap][ci], 64-byte runs into
 // wT[ci][tap][co].  blockIdx.y = table entry, blockIdx.x = tile (CTAs beyond the entry's tile count exit).
 __global__ void __launch_bounds__(256) pack_weights_tiled_kernel(const gdl_pack_entry* __restrict__ tab) {
-  pdl_enter();
   extern __shared__ bf16 s_tile[];  // [32 co][RS][64 ci + 2 pad] (row stride 33 words: the transposed read is conflict-free)
   constexpr int LD = 66;
   const gdl_pack_entry e = tab[blockIdx.y];
@@ -533,7 +531,6 @@ struct TapSplits {
 template <int G>
 __global__ void __launch_bounds__(256) wgrad_reduce_t_kernel(const float* __restrict__ partial, float* __restrict__ dw,
                                                              const TapSplits ts, int Kp, int Co, int Ci, int taps) {
-  pdl_enter();
   constexpr int OB = 256 / G;  // outputs per block
   __shared__ float red[G > 1 ? 256 : 1];
   const int o = threadIdx.x % OB, g = threadIdx.x / OB;
@@ -574,11 +571,11 @@ static int launch_wgrad_reduce_t(const float* partial, float* dw, int splits, co
   // 2-5 % slower per weight gradient than the per-element kernel below: the partials are L2-resident and the
   // 36-byte-stride stores of 2.4 M elements do not bound it.)
   if (total < 400000 && splits >= 16) {
-    launch_pdl(wgrad_reduce_t_kernel<8>, (unsigned)ceil_div64(total, 32), 256, 0, s, partial, dw, ts, Kp, Co, Ci, taps);
+    wgrad_reduce_t_kernel<8><<<(unsigned)ceil_div64(total, 32), 256, 0, s>>>(partial, dw, ts, Kp, Co, Ci, taps);
   } else if (total < 800000 && splits >= 8) {
-    launch_pdl(wgrad_reduce_t_kernel<4>, (unsigned)ceil_div64(total, 64), 256, 0, s, partial, dw, ts, Kp, Co, Ci, taps);
+    wgrad_reduce_t_kernel<4><<<(unsigned)ceil_div64(total, 64), 256, 0, s>>>(partial, dw, ts, Kp, Co, Ci, taps);
   } else {
-    launch_pdl(wgrad_reduce_t_kernel<1>, (unsigned)ceil_div64(total, 256), 256, 0, s, partial, dw, ts, Kp, Co, Ci, taps);
+    wgrad_reduce_t_kernel<1><<<(unsigned)ceil_div64(total, 256), 256, 0, s>>>(partial, dw, ts, Kp, Co, Ci, taps);
   }
   GDL_CHECK_LAUNCH("wgrad_reduce_t_kernel");
   return GDL_OK;
@@ -685,14 +682,7 @@ static int flat_policy() {
 }
 // 1x1 convolutions up to this many input channels take the flat kernel (round 1 stopped at 128: the 256 -> 512
 // downsample of layer4 ran on the legacy gather kernel at 8 % tensor-pipe activity)
-static int flat_1x1_max_ci() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GDL_FLAT_1X1_MAX_CI");
-    v = e ? atoi(e) : 512;
-  }
-  return v;
-}
+constexpr int kFlat1x1MaxCi = 512;
 static bool prefer_flat_s1(int, int) { return flat_policy() != 0; }
 
 // conv_wgrad_flat.cu
@@ -776,7 +766,7 @@ static int conv_fwd_impl(const gdl_conv_desc* d, const void* x, const void* w_pa
                            d->Co, res, amode, (cudaStream_t)s, stats, stats_rows, bias, relu);
     if (rc != 0) return rc < 0 ? rc : GDL_OK;
   }
-  if (d->R == 1 && d->S == 1 && d->pad == 0 && d->Ci % 64 == 0 && d->Ci <= flat_1x1_max_ci() && flat_policy() != 0) {
+  if (d->R == 1 && d->S == 1 && d->pad == 0 && d->Ci % 64 == 0 && d->Ci <= kFlat1x1MaxCi && flat_policy() != 0) {
     // 1x1 (stride 1 or 2): a single tap over the strided view x[:, ::stride, ::stride, :]
     int rc = try_conv_flat(3, d->N, d->Ho, d->Wo, d->Ci, (int64_t)d->stride * d->Ci,
                            (int64_t)d->stride * d->Wi * d->Ci, (int64_t)d->Hi * d->Wi * d->Ci, x, w_packed, d->Co,
@@ -810,7 +800,7 @@ extern "C" int gdl_conv_pack_weights_tiled(const gdl_pack_entry* table_dev, int 
                                            gdl_stream_t s) {
   GDL_REQUIRE(table_dev && n > 0 && max_tiles > 0 && max_rs > 0 && max_rs <= 9, "gdl_conv_pack_weights_tiled: bad arguments");
   const size_t smem = (size_t)32 * max_rs * 66 * sizeof(bf16);
-  launch_pdl(pack_weights_tiled_kernel, dim3(max_tiles, n), 256, smem, (cudaStream_t)s, table_dev);
+  pack_weights_tiled_kernel<<<dim3(max_tiles, n), 256, smem, (cudaStream_t)s>>>(table_dev);
   GDL_CHECK_LAUNCH("pack_weights_tiled_kernel");
   return GDL_OK;
 }
@@ -819,7 +809,7 @@ extern "C" int gdl_conv_pack_weights_multi(const gdl_pack_entry* table_dev, int 
   GDL_REQUIRE(table_dev && n > 0 && total > 0, "gdl_conv_pack_weights_multi: bad arguments");
   int64_t blocks = ceil_div64(total, 256);
   if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-  launch_pdl(pack_weights_multi_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)s, table_dev, n, total);
+  pack_weights_multi_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)s>>>(table_dev, n, total);
   GDL_CHECK_LAUNCH("pack_weights_multi_kernel");
   return GDL_OK;
 }
@@ -896,26 +886,15 @@ extern "C" int gdl_conv_wgrad(const gdl_conv_desc* d, int ci_real, const void* x
   GDL_REQUIRE(x && dy && dw_oihw && workspace, "gdl_conv_wgrad: null pointer");
   GDL_REQUIRE(ci_real > 0 && ci_real <= d->Ci, "gdl_conv_wgrad: ci_real out of range");
   if (ci_real == d->Ci && prefer_wflat(d)) {
-    // GDL_WGRAD_T (default 1): co-major partials (coalesced epilogue stores) + the group-parallel reduction
-    static const int tr = []() {
-      const char* e = getenv("GDL_WGRAD_T");
-      return e ? atoi(e) : 1;
-    }();
+    // co-major partials (coalesced epilogue stores) + the group-parallel reduction
     TapSplits ts;
     for (int i = 0; i < 9; ++i) ts.n[i] = 0;
     int ns = try_wgrad_flat(d->N, d->Hi, d->Wi, d->Ho, d->Wo, d->Ci, d->Co, d->R, d->stride, x, dy, (float*)workspace,
-                            workspace_bytes, (cudaStream_t)s, tr, tr ? ts.n : nullptr);
+                            workspace_bytes, (cudaStream_t)s, 1, ts.n);
     if (ns < 0) return ns;
-    if (ns > 0) {
-      int Kp = d->R * d->S * d->Ci;
-      if (tr) return launch_wgrad_reduce_t((const float*)workspace, dw_oihw, ns, ts, Kp, d->Co, d->Ci, d->R * d->S,
-                                           (cudaStream_t)s);
-      int64_t total = (int64_t)Kp * d->Co;
-      wgrad_reduce_kernel<<<(unsigned)ceil_div64(total, 256), 256, 0, (cudaStream_t)s>>>(
-          (const float*)workspace, dw_oihw, ns, Kp, d->Co, d->Ci, ci_real, d->R, d->S);
-      GDL_CHECK_LAUNCH("wgrad_reduce_kernel");
-      return GDL_OK;
-    }
+    if (ns > 0)
+      return launch_wgrad_reduce_t((const float*)workspace, dw_oihw, ns, ts, d->R * d->S * d->Ci, d->Co, d->Ci,
+                                   d->R * d->S, (cudaStream_t)s);
   }
   WgradPlan w = plan_wgrad(d);
   int64_t need = (int64_t)w.splits * w.Kp * d->Co * (int64_t)sizeof(float);

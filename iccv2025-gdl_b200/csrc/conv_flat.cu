@@ -277,7 +277,6 @@ __device__ __forceinline__ void flat_load_rows(const FlatParams& p, int plane, u
 // receives and reads the whole tile — and was removed; the CTA-pair kernel below splits the tile instead.)
 template <int BN, int MT, int WST, bool STATS, bool RES = false>
 __global__ void __launch_bounds__(kFlatThreads, 1) conv_flat_kernel(const __grid_constant__ FlatParams p) {
-  pdl_launch_dependents();  // the next kernel may start its prologue now (common.cuh: PDL)
   constexpr int W_BYTES = BN * 128;
   constexpr int TM = MT * 128;
   constexpr int kMaxWin = 4;
@@ -327,7 +326,6 @@ __global__ void __launch_bounds__(kFlatThreads, 1) conv_flat_kernel(const __grid
     tma_prefetch_desc(&p.tm_x[0]);
     tma_prefetch_desc(&p.tm_w);
   }
-  pdl_wait();  // everything above touched only shared memory / TMEM / kernel parameters
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -496,7 +494,6 @@ __global__ void __launch_bounds__(kFlatThreads, 1) conv_flat_kernel(const __grid
 //   for their shared-memory-bandwidth bound: no weight ring traffic and 5 KB instead of 6 KB of operands per MMA.
 template <int BN, int MT, int WST, bool STATS, bool RES = false>
 __global__ void __launch_bounds__(kFlatThreads, 1) conv_flat2_kernel(const __grid_constant__ FlatParams p) {
-  pdl_launch_dependents();  // the next kernel may start its prologue now (common.cuh: PDL)
   constexpr int HB = BN / 2;
   constexpr int W_BYTES = HB * 128;
   constexpr int TM = MT * 128;
@@ -547,7 +544,6 @@ __global__ void __launch_bounds__(kFlatThreads, 1) conv_flat2_kernel(const __gri
     tma_prefetch_desc(&p.tm_x[0]);
     tma_prefetch_desc(&p.tm_w_half);
   }
-  pdl_wait();  // everything above touched only shared memory / TMEM / kernel parameters
   tc_fence_before();
   __syncthreads();
   cluster_sync_all();  // both CTAs' barriers exist before any remote arrive / multicast commit / remote complete_tx
@@ -738,9 +734,9 @@ static int launch_flat(FlatParams& p, int64_t Q, cudaStream_t s) {
   int grid = p.items_total < kNumSMs ? p.items_total : kNumSMs;
   g_flat_last_grid = grid;
   if (st)
-    launch_pdl(conv_flat_kernel<BN, MT, WST, true, RES>, grid, kFlatThreads, total, s, p);
+    conv_flat_kernel<BN, MT, WST, true, RES><<<grid, kFlatThreads, total, s>>>(p);
   else
-    launch_pdl(conv_flat_kernel<BN, MT, WST, false, RES>, grid, kFlatThreads, total, s, p);
+    conv_flat_kernel<BN, MT, WST, false, RES><<<grid, kFlatThreads, total, s>>>(p);
   GDL_CHECK_LAUNCH("conv_flat_kernel");
   return 1;
 }
@@ -785,15 +781,13 @@ static int launch_flat2(FlatParams& p, int64_t Q, cudaStream_t s) {
   cfg.blockDim = dim3(kFlatThreads);
   cfg.dynamicSmemBytes = total;
   cfg.stream = s;
-  cudaLaunchAttribute at[2];
+  cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = 2;
   at[0].val.clusterDim.y = 1;
   at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
   cfg.attrs = at;
-  cfg.numAttrs = 2;
+  cfg.numAttrs = 1;
   g_flat_last_grid = grid2;
   cudaError_t e = st ? cudaLaunchKernelEx(&cfg, conv_flat2_kernel<BN, MT, WST, true, RES>, p)
                      : cudaLaunchKernelEx(&cfg, conv_flat2_kernel<BN, MT, WST, false, RES>, p);
@@ -801,12 +795,7 @@ static int launch_flat2(FlatParams& p, int64_t Q, cudaStream_t s) {
   return 1;
 }
 
-thread_local int g_fused_stats_min_k = -1;  // per calling thread, like gdl_set_sweep; -1: GDL_FUSED_STATS_MIN_K or the default
-
-static int env_int3(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
+thread_local int g_fused_stats_min_k = -1;  // per calling thread, like gdl_set_sweep; -1: the default (0)
 
 // kind: 0 forward 3x3/s1, 1 dgrad 3x3/s1, 2 dgrad 3x3/s2 (parity classes), 3 single tap (1x1),
 // 4 forward 3x3/s2: (Hs,Ws) is the OUTPUT grid, src is the whole input [N,Hi,Wi,Cs] (sH = Wi*Cs, sN = Hi*Wi*Cs)
@@ -817,7 +806,6 @@ int try_conv_flat(int kind, int N, int Hs, int Ws, int Cs, int64_t sW, int64_t s
                   const void* wt, int64_t wt_rows, int64_t wt_k, void* dst, int Hd, int Wd, int Cd,
                   const void* add_src, int add_mode, cudaStream_t s, float* stats, int* stats_rows, const float* bias,
                   int relu) {
-  static const int mt_force = env_int3("GDL_FLAT_MT", 0);
   if (Cs % 64 != 0 || Cd % 64 != 0) return 0;
   const int P = Ws + 1;
   if (P > 256) return 0;
@@ -833,10 +821,8 @@ int try_conv_flat(int kind, int N, int Hs, int Ws, int Cs, int64_t sW, int64_t s
   p.relu = relu;
   p.rev = g_sweep_rev;
   // BatchNorm statistics in the epilogue (stat_chunk above) for convolutions with K >= the threshold: default every
-  // convolution this kernel runs (GDL_FUSED_STATS_MIN_K / gdl_set_fused_stats_min_k(K) raise it; tests/ cover both paths).
-  static const int stats_min_k_env = env_int3("GDL_FUSED_STATS_MIN_K", 0);
-  const int stats_min_k = g_fused_stats_min_k >= 0 ? g_fused_stats_min_k : stats_min_k_env;
-  if (stats != nullptr && wt_k < stats_min_k) stats = nullptr;
+  // convolution this kernel runs (gdl_set_fused_stats_min_k(K) raises it; tests/ cover both paths).
+  if (stats != nullptr && wt_k < g_fused_stats_min_k) stats = nullptr;
   p.stats = stats;
   p.N = N; p.Hs = Hs; p.Ws = Ws; p.Cs = Cs;
   p.Hd = Hd; p.Wd = Wd; p.Cd = Cd;
@@ -910,11 +896,10 @@ int try_conv_flat(int kind, int N, int Hs, int Ws, int Cs, int64_t sW, int64_t s
       if (p.taps[c][t].shift > p.smax) p.smax = p.taps[c][t].shift;
     }
   const int BN = (Cd % 128 == 0) ? 128 : 64;
-  // GDL_FLAT_ROWBOX (default 3): bit 0 = four-row boxes, bit 1 = whole-image boxes for maps of at most 32 KB per slab
-  static const int rowbox = env_int3("GDL_FLAT_ROWBOX", 3);
+  // four-row boxes, and whole-image boxes for maps of at most 32 KB per slab (flat_load_rows)
   const int rows_img = Hs + 1;
-  p.use_r4 = (rowbox & 1) && rows_img >= 4;
-  p.use_img = (rowbox & 2) && rows_img <= 256 && (int64_t)rows_img * P * 128 <= 32 * 1024;
+  p.use_r4 = rows_img >= 4;
+  p.use_img = rows_img <= 256 && (int64_t)rows_img * P * 128 <= 32 * 1024;
   auto views = [&](const void* base, int w, int h, int64_t vW, int64_t vH, int idx) -> bool {
     const CUtensorMap* t = tmap_view4(base, Cs, w, h, N, vW, vH, sN, P);
     if (!t) return false;
@@ -954,44 +939,25 @@ int try_conv_flat(int kind, int N, int Hs, int Ws, int Cs, int64_t sW, int64_t s
   const double cost_mt2 = 2.0 * double((items2 + kNumSMs - 1) / kNumSMs);
   const double cost_mt1 = 1.15 * double((items1 + kNumSMs - 1) / kNumSMs);
   const double cost_pair = 1.7 * double((pairs2 + kNumSMs / 2 - 1) / (kNumSMs / 2));
-  int mt = cost_mt2 <= cost_mt1 ? 2 : 1;
+  const int mt = cost_mt2 <= cost_mt1 ? 2 : 1;
   const bool pair_wins = cost_pair <= (mt == 2 ? cost_mt2 : cost_mt1);
-  if (mt_force) mt = mt_force;
   int rc = 0;
-  // GDL_FLAT_PAIR (default 1): CTA-pair kernel (cta_group::2) where the wave-count model above prefers it
-  static const int pair = env_int3("GDL_FLAT_PAIR", 1);
+  if (pair_wins) {  // CTA-pair kernel (cta_group::2) where the wave-count model above prefers it
+    const CUtensorMap* th = tmap_rows(wt, wt_rows, wt_k, BN / 2);
+    if (!th) return GDL_ECUDA;
+    p.tm_w_half = *th;
+  }
   if (BN == 128) {
-    if (pair && pair_wins && !mt_force) {
-      const CUtensorMap* th = tmap_rows(wt, wt_rows, wt_k, BN / 2);
-      if (!th) return GDL_ECUDA;
-      p.tm_w_half = *th;
-      rc = launch_flat2<128, 2, 6>(p, Q, s);
-    }
+    if (pair_wins) rc = launch_flat2<128, 2, 6>(p, Q, s);
     if (rc == 0 && mt == 2) rc = launch_flat<128, 2, 4>(p, Q, s);
     if (rc == 0) rc = launch_flat<128, 1, 4>(p, Q, s);
   } else {
-    // GDL_FLAT_RESIDENT (default 1): 64 -> 64 channel 3x3 layers keep their 72 KB of weights in shared memory
-    // (measured: 56x56 forward / dgrad 700-730 -> 800+ TF, step 23.11 -> 22.82 ms; step parity tests green)
-    static const int resident = env_int3("GDL_FLAT_RESIDENT", 1);
-    // GDL_FLAT_PAIR64: CTA-pair kernel for 64-channel tiles (N = 64 MMAs read 6 KB of operands per 32 clocks on one
-    // SM, 5 KB as a pair).  1 = wherever eligible (instead of the resident-weights kernel too), 2 = only where the
-    // resident-weights kernel does not apply (e.g. the 128 -> 64 channel stride-2 data gradients), 0 = off.
-    static const int pair64 = env_int3("GDL_FLAT_PAIR64", 2);
-    const bool res_ok = resident && mt == 2 && Cs == 64 && Cd == 64 && (kind == 0 || kind == 1);
-    // GDL_FLAT_PAIR64RES (default 1): CTA pair AND resident weights for the 64 -> 64 channel 3x3 layers
-    static const int pair64res = env_int3("GDL_FLAT_PAIR64RES", 1);
-    if (pair && pair64res && pair_wins && !mt_force && res_ok) {
-      const CUtensorMap* th = tmap_rows(wt, wt_rows, wt_k, BN / 2);
-      if (!th) return GDL_ECUDA;
-      p.tm_w_half = *th;
-      rc = launch_flat2<64, 2, 8, true>(p, Q, s);
-    }
-    if (rc == 0 && pair && pair64 && pair_wins && !mt_force && !(pair64 == 2 && res_ok)) {
-      const CUtensorMap* th = tmap_rows(wt, wt_rows, wt_k, BN / 2);
-      if (!th) return GDL_ECUDA;
-      p.tm_w_half = *th;
-      rc = launch_flat2<64, 2, 8>(p, Q, s);
-    }
+    // 64 -> 64 channel 3x3 layers keep their 72 KB of weights in shared memory (resident; measured: 56x56 forward /
+    // dgrad 700-730 -> 800+ TF, step 23.11 -> 22.82 ms), as a CTA pair where the model prefers one.  The CTA pair
+    // also serves the other 64-channel tiles (e.g. the 128 -> 64 channel stride-2 data gradients): N = 64 MMAs read
+    // 6 KB of operands per 32 clocks on one SM, 5 KB as a pair.
+    const bool res_ok = mt == 2 && Cs == 64 && Cd == 64 && (kind == 0 || kind == 1);
+    if (pair_wins) rc = res_ok ? launch_flat2<64, 2, 8, true>(p, Q, s) : launch_flat2<64, 2, 8>(p, Q, s);
     if (rc == 0 && res_ok) rc = launch_flat<64, 2, 6, true>(p, Q, s);
     if (rc == 0 && mt == 2) rc = launch_flat<64, 2, 6>(p, Q, s);
     if (rc == 0) rc = launch_flat<64, 1, 6>(p, Q, s);

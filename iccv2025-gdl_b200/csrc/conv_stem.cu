@@ -39,7 +39,6 @@ constexpr int kSThreads = 192;
 template <int C>
 __global__ void __launch_bounds__(128) stem_layout_kernel(const float* __restrict__ src, bf16* __restrict__ dst,
                                                           int T, int H, int W, int Hp, int Wp) {
-  pdl_enter();
   const int row = blockIdx.x;
   const int bt = row / Hp, pp = row - bt * Hp;
   const int b = bt / T, t = bt - b * T;
@@ -76,7 +75,6 @@ __global__ void __launch_bounds__(128) stem_layout_kernel(const float* __restric
 
 // fp32 OIHW [64][C][7][7] -> bf16 [64][256]  (k = (a*4+b)*16 + (dy*2+dx)*C + c)
 __global__ void stem_pack_kernel(const float* __restrict__ w, const float* __restrict__ scale, bf16* __restrict__ wp, int C) {
-  pdl_enter();
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= 64 * 256) return;
   int co = idx >> 8, k = idx & 255;
@@ -113,9 +111,7 @@ struct StemFwdSmem {
   static constexpr int TOTAL = STAT_OFF + 2048 + 1024;
 };
 
-template <int ROLES>  // bit 0: elect.sync for the MMA issuer, bit 1: for the TMA producer (else lane 0 by thread id)
 __global__ void __launch_bounds__(kSThreads, 1) stem_fwd_kernel(const __grid_constant__ StemParams p) {
-  pdl_launch_dependents();  // the next kernel may start its prologue now (common.cuh: PDL)
   using L = StemFwdSmem;
   constexpr int HST = kSFwdHaloStages;
   extern __shared__ uint8_t smem_raw[];
@@ -150,14 +146,13 @@ __global__ void __launch_bounds__(kSThreads, 1) stem_fwd_kernel(const __grid_con
     tma_prefetch_desc(&p.tm_w);
     tma_prefetch_desc(&p.tm_out);
   }
-  pdl_wait();  // everything above touched only shared memory / TMEM / kernel parameters
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t smem_base = smem_u32(smem);
 
-  if ((ROLES & 2) ? (warp == 5 && elect_one()) : (tid == 5 * 32)) {
+  if (warp == 5 && elect_one()) {
     // ---------------- TMA producer: weights once, then one halo per tile ----------------
     mbar_arrive_expect_tx(w_full, kSWBytes);
     for (int tap = 0; tap < 16; ++tap)
@@ -173,7 +168,7 @@ __global__ void __launch_bounds__(kSThreads, 1) stem_fwd_kernel(const __grid_con
       tma_load_4d(smem_base + L::HALO_OFF + hs * kSHaloBytes, &p.tm_x, &halo_full[hs], 0, tw * kSTileW,
                   th * kSTileH, n);
     }
-  } else if ((ROLES & 1) ? (warp == 4 && elect_one()) : (tid == 4 * 32)) {
+  } else if (warp == 4 && elect_one()) {
     // ---------------- MMA issuer: 16 taps = 16 shifted views, one K=16 MMA each ----------------
     constexpr uint32_t idesc = make_idesc_bf16(128, 64, 0, 0);
     const uint32_t a_hi = desc_hi_sw32(kSHaloW * 32), b_hi = desc_hi_sw32(256);
@@ -311,7 +306,6 @@ struct StemWgSmem {
 // missing for a-1: tiles of the first tile row run one more K step over "rows -2, -1", where block 0 reads the 2 KB of
 // zeros kept in front of the tile and block 1 reads (zeros, row 0).
 __global__ void __launch_bounds__(kSThreads, 1) stem_wgrad_kernel(const __grid_constant__ StemWgradParams p) {
-  pdl_launch_dependents();  // the next kernel may start its prologue now (common.cuh: PDL)
   using L = StemWgSmem;
   constexpr int ST = kSWgStages;
   extern __shared__ uint8_t smem_raw[];
@@ -347,7 +341,6 @@ __global__ void __launch_bounds__(kSThreads, 1) stem_wgrad_kernel(const __grid_c
     tma_prefetch_desc(&p.tm_dy);
   }
   fence_proxy_async();
-  pdl_wait();  // everything above touched only shared memory / TMEM / kernel parameters
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -423,7 +416,6 @@ __global__ void __launch_bounds__(kSThreads, 1) stem_wgrad_kernel(const __grid_c
 // partial [splits][a][co][b*16+ch] -> dw OIHW [64][C][7][7]
 __global__ void stem_wgrad_reduce_kernel(const float* __restrict__ partial, float* __restrict__ dw, int splits,
                                          int C) {
-  pdl_enter();
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= 64 * C * 49) return;
   int s = idx % 7;
@@ -464,10 +456,10 @@ extern "C" int gdl_stem_layout(const float* src, void* dst, int B, int C, int T,
   GDL_REQUIRE(rows < ((int64_t)1 << 31), "gdl_stem_layout: too many rows");
   const cudaStream_t st = (cudaStream_t)s;
   switch (C) {
-    case 1: launch_pdl(stem_layout_kernel<1>, (unsigned)rows, 128, 0, st, src, (bf16*)dst, T, H, W, Hp, Wp); break;
-    case 2: launch_pdl(stem_layout_kernel<2>, (unsigned)rows, 128, 0, st, src, (bf16*)dst, T, H, W, Hp, Wp); break;
-    case 3: launch_pdl(stem_layout_kernel<3>, (unsigned)rows, 128, 0, st, src, (bf16*)dst, T, H, W, Hp, Wp); break;
-    default: launch_pdl(stem_layout_kernel<4>, (unsigned)rows, 128, 0, st, src, (bf16*)dst, T, H, W, Hp, Wp); break;
+    case 1: stem_layout_kernel<1><<<(unsigned)rows, 128, 0, st>>>(src, (bf16*)dst, T, H, W, Hp, Wp); break;
+    case 2: stem_layout_kernel<2><<<(unsigned)rows, 128, 0, st>>>(src, (bf16*)dst, T, H, W, Hp, Wp); break;
+    case 3: stem_layout_kernel<3><<<(unsigned)rows, 128, 0, st>>>(src, (bf16*)dst, T, H, W, Hp, Wp); break;
+    default: stem_layout_kernel<4><<<(unsigned)rows, 128, 0, st>>>(src, (bf16*)dst, T, H, W, Hp, Wp); break;
   }
   GDL_CHECK_LAUNCH("stem_layout_kernel");
   return GDL_OK;
@@ -475,7 +467,7 @@ extern "C" int gdl_stem_layout(const float* src, void* dst, int B, int C, int T,
 
 extern "C" int gdl_stem_pack_weights(const float* w_oihw, void* w_packed, int C, gdl_stream_t s) {
   GDL_REQUIRE(w_oihw && w_packed && C > 0 && C <= 4, "gdl_stem_pack_weights: bad arguments");
-  launch_pdl(stem_pack_kernel, 64, 256, 0, (cudaStream_t)s, w_oihw, nullptr, (bf16*)w_packed, C);
+  stem_pack_kernel<<<64, 256, 0, (cudaStream_t)s>>>(w_oihw, nullptr, (bf16*)w_packed, C);
   GDL_CHECK_LAUNCH("stem_pack_kernel");
   return GDL_OK;
 }
@@ -483,7 +475,7 @@ extern "C" int gdl_stem_pack_weights(const float* w_oihw, void* w_packed, int C,
 extern "C" int gdl_stem_pack_weights_scaled(const float* w_oihw, const float* scale64, void* w_packed, int C,
                                             gdl_stream_t s) {
   GDL_REQUIRE(w_oihw && scale64 && w_packed && C >= 1 && C <= 4, "gdl_stem_pack_weights_scaled: bad arguments");
-  launch_pdl(stem_pack_kernel, 64, 256, 0, (cudaStream_t)s, w_oihw, scale64, (bf16*)w_packed, C);
+  stem_pack_kernel<<<64, 256, 0, (cudaStream_t)s>>>(w_oihw, scale64, (bf16*)w_packed, C);
   GDL_CHECK_LAUNCH("stem_pack_kernel(scaled)");
   return GDL_OK;
 }
@@ -504,27 +496,16 @@ static int stem_fwd_impl(const void* x16, const void* w_packed, void* y, int N, 
   p.tiles_h = (Ho + kSTileH - 1) / kSTileH;
   p.tiles_w = (Wo + kSTileW - 1) / kSTileW;
   p.tiles_total = N * p.tiles_h * p.tiles_w;
-  static int roles = -1;
-  if (roles < 0) {
-    const char* e = getenv("GDL_STEM_ROLES");
-    roles = e ? atoi(e) & 3 : 3;
-    cudaError_t err = cudaSuccess;
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(stem_fwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, StemFwdSmem::TOTAL);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(stem_fwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, StemFwdSmem::TOTAL);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(stem_fwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, StemFwdSmem::TOTAL);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(stem_fwd_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, StemFwdSmem::TOTAL);
+  static bool attr_set = false;
+  if (!attr_set) {
+    cudaError_t err = cudaFuncSetAttribute(stem_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, StemFwdSmem::TOTAL);
     if (err != cudaSuccess) return cuda_fail(err, "cudaFuncSetAttribute(stem_fwd)");
+    attr_set = true;
   }
   // two CTAs per SM (80 KB of shared memory, 128 TMEM columns each): the kernel is bound by its output writes,
   // and a second resident CTA hides their latency (measured 0.42 -> 0.32 ms on the visual stem)
-  int grid = p.tiles_total < 2 * kNumSMs ? p.tiles_total : 2 * kNumSMs;
-  if (const char* g = getenv("GDL_STEM_GRID")) grid = atoi(g) < p.tiles_total ? atoi(g) : p.tiles_total;
-  switch (roles) {
-    case 0: launch_pdl(stem_fwd_kernel<0>, grid, kSThreads, StemFwdSmem::TOTAL, (cudaStream_t)s, p); break;
-    case 1: launch_pdl(stem_fwd_kernel<1>, grid, kSThreads, StemFwdSmem::TOTAL, (cudaStream_t)s, p); break;
-    case 2: launch_pdl(stem_fwd_kernel<2>, grid, kSThreads, StemFwdSmem::TOTAL, (cudaStream_t)s, p); break;
-    default: launch_pdl(stem_fwd_kernel<3>, grid, kSThreads, StemFwdSmem::TOTAL, (cudaStream_t)s, p); break;
-  }
+  const int grid = p.tiles_total < 2 * kNumSMs ? p.tiles_total : 2 * kNumSMs;
+  stem_fwd_kernel<<<grid, kSThreads, StemFwdSmem::TOTAL, (cudaStream_t)s>>>(p);
   GDL_CHECK_LAUNCH("stem_fwd_kernel");
   if (stats_rows) *stats_rows = grid;
   return GDL_OK;
@@ -576,9 +557,9 @@ extern "C" int gdl_stem_wgrad(const void* x16, const void* dy, float* dw_oihw, i
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(stem_wgrad)");
     attr_set = true;
   }
-  launch_pdl(stem_wgrad_kernel, splits, kSThreads, StemWgSmem::TOTAL, (cudaStream_t)s, p);
+  stem_wgrad_kernel<<<splits, kSThreads, StemWgSmem::TOTAL, (cudaStream_t)s>>>(p);
   GDL_CHECK_LAUNCH("stem_wgrad_kernel");
-  launch_pdl(stem_wgrad_reduce_kernel, (64 * C * 49 + 255) / 256, 256, 0, (cudaStream_t)s, (const float*)workspace, dw_oihw, splits, C);
+  stem_wgrad_reduce_kernel<<<(64 * C * 49 + 255) / 256, 256, 0, (cudaStream_t)s>>>((const float*)workspace, dw_oihw, splits, C);
   GDL_CHECK_LAUNCH("stem_wgrad_reduce_kernel");
   return GDL_OK;
 }

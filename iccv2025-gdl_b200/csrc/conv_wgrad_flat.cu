@@ -76,7 +76,6 @@ __global__ void __launch_bounds__(kWfThreads, 1) conv_wgrad_flat_kernel(const __
   const int type = y % p.ntypes;
   const int t0 = min(blockIdx.x * p.tps[type], p.tiles_total);
   const int t1 = min(t0 + p.tps[type], p.tiles_total);
-  pdl_launch_dependents();  // the next kernel may start its prologue now (common.cuh: PDL)
   if (t0 >= t1) return;  // this type has fewer splits than the grid is wide (whole CTA, before any setup)
   y /= p.ntypes;
   const int co0 = (y % p.co_tiles) * BN;
@@ -106,7 +105,6 @@ __global__ void __launch_bounds__(kWfThreads, 1) conv_wgrad_flat_kernel(const __
     tma_prefetch_desc(&p.tm_dy);
   }
   fence_proxy_async();
-  pdl_wait();  // everything above touched only shared memory / TMEM / kernel parameters
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -377,33 +375,24 @@ static bool plan_wgrad_flat(int N, int Ho, int Wo, int Ci, int Co, int R, int st
   if (w.xwin_bytes >= (1 << 18) || w.dywin_bytes >= (1 << 18)) return false;  // LBO field
   w.gy = w.ci_tiles * w.co_tiles * w.ntypes;
   // One CTA per SM (the stage ring takes ~200 KB) and all 512 TMEM columns: CTAs of a second wave cannot
-  // overlap the first wave's epilogue, they only add a prologue, an epilogue and a set of partials each.
-  // GDL_WGRAD_WAVES (default 1) sets how many CTAs per SM the split-K factor is sized for.
-  static const int waves = []() {
-    const char* e = getenv("GDL_WGRAD_WAVES");
-    const int v = e ? atoi(e) : 1;
-    return v < 1 ? 1 : (v > 4 ? 4 : v);
-  }();
+  // overlap the first wave's epilogue, they only add a prologue, an epilogue and a set of partials each: the
+  // split-K factor is sized for one wave.
   // Split-K CTAs per job type, proportional to the type's MMA work per tile (its accumulator count): the
   // parity planes of a stride-2 convolution carry 4 / 2 / 2 / 1 taps, and with equal splits the 1-tap CTAs
-  // would idle for 3/4 of the kernel.  GDL_WGRAD_BALANCE=0 restores equal splits.
-  static const int balance = []() {
-    const char* e = getenv("GDL_WGRAD_BALANCE");
-    return e ? atoi(e) : 1;
-  }();
+  // would idle for 3/4 of the kernel.
   const int groups = w.ci_tiles * w.co_tiles;
-  int cta_budget = (waves * kNumSMs) / groups;  // CTAs of one (ci, co) tile over all types
+  int cta_budget = kNumSMs / groups;  // CTAs of one (ci, co) tile over all types
   if (cta_budget < w.ntypes) cta_budget = w.ntypes;
   int wsum = 0;
   for (int k = 0; k < w.ntypes; ++k) wsum += w.jt[k].nunits;
   int used = 0;
   for (int k = 0; k < w.ntypes; ++k) {
-    int sk = balance ? cta_budget * w.jt[k].nunits / wsum : cta_budget / w.ntypes;
+    int sk = cta_budget * w.jt[k].nunits / wsum;
     if (sk < 1) sk = 1;
     w.nsplit[k] = sk;
     used += sk;
   }
-  while (balance && used < cta_budget) {  // hand the remainder to the type with the most work per CTA
+  while (used < cta_budget) {  // hand the remainder to the type with the most work per CTA
     int best_k = 0;
     for (int k = 1; k < w.ntypes; ++k)
       if ((int64_t)w.jt[k].nunits * w.nsplit[best_k] > (int64_t)w.jt[best_k].nunits * w.nsplit[k]) best_k = k;
@@ -430,7 +419,7 @@ static int launch_wf(const WfParams& p, const WfPlan& w, cudaStream_t s) {
     attr_set = true;
   }
   dim3 grid(w.splits, w.gy);
-  launch_pdl(conv_wgrad_flat_kernel<BN, MODE>, grid, kWfThreads, w.stages * w.stage_bytes + 512 + 1024, s, p);
+  conv_wgrad_flat_kernel<BN, MODE><<<grid, kWfThreads, w.stages * w.stage_bytes + 512 + 1024, s>>>(p);
   GDL_CHECK_LAUNCH("conv_wgrad_flat_kernel");
   return GDL_OK;
 }

@@ -148,7 +148,6 @@ __global__ void bn_stats_finalize_kernel(const float* __restrict__ partial, int 
                                          const float* __restrict__ beta, float eps, float momentum,
                                          float* running_mean, float* running_var, float* mean_out,
                                          float* invstd_out, float* scale, float* shift) {
-  pdl_enter();
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (c >= C) return;
@@ -203,7 +202,6 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const bf16* __restrict__ 
                                                        bf16* __restrict__ y, int64_t nvec, int C,
                                                        const float* __restrict__ scale,
                                                        const float* __restrict__ shift, int relu, int rev) {
-  pdl_enter();
   const int groups = C / 8;
   const int64_t first = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int cg = fixed_channel_group(first, nvec, groups, rev);
@@ -250,7 +248,6 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const bf16* __restrict__ 
 __global__ void __launch_bounds__(kBnThreads) bn_bwd_reduce_kernel(
     const bf16* dy, const bf16* __restrict__ y, const bf16* __restrict__ x, bf16* dz, int64_t P, int C,
     float* __restrict__ partial, int relu, int rev) {
-  pdl_enter();
   const int groups = C / 8;
   const int lanes = kBnThreads / groups;
   const int cg = threadIdx.x % groups;
@@ -317,7 +314,6 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(
     int C, float invP, const float* __restrict__ gamma, const float* __restrict__ mean,
     const float* __restrict__ invstd, const float* __restrict__ dgamma,
     const float* __restrict__ dbeta, int rev) {
-  pdl_enter();
   // dx = a*dz + b*x + c  with  a = gamma*invstd,  b = -a*invstd*dgamma/P,
   //                            c = -a*dbeta/P - b*mean          (per channel, in registers: see fixed_channel_group)
   const int groups = C / 8;
@@ -460,7 +456,6 @@ __global__ void __launch_bounds__(256) maxpool_bwd_kernel(const bf16* __restrict
 __global__ void __launch_bounds__(kBnThreads, 3) bn_bwd_nores_reduce_kernel(
     const bf16* __restrict__ dy, const bf16* __restrict__ x, int64_t P, int C, const float* __restrict__ scale,
     const float* __restrict__ shift, float* __restrict__ partial, int rev) {
-  pdl_enter();
   const int groups = C / 8;
   const int lanes = kBnThreads / groups;
   const int cg = threadIdx.x % groups;
@@ -509,7 +504,6 @@ __global__ void __launch_bounds__(kBnThreads, 3) bn_bwd_nores_reduce_kernel(
 __global__ void bn_bwd_finalize_raw_kernel(const float* __restrict__ partial, int nblk, int C,
                                            const float* __restrict__ mean, const float* __restrict__ invstd,
                                            float* __restrict__ dgamma, float* __restrict__ dbeta) {
-  pdl_enter();
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (c >= C) return;
@@ -531,7 +525,6 @@ __global__ void __launch_bounds__(256) bn_bwd_nores_apply_kernel(
     float invP, const float* __restrict__ gamma, const float* __restrict__ mean,
     const float* __restrict__ invstd, const float* __restrict__ scale, const float* __restrict__ shift,
     const float* __restrict__ dgamma, const float* __restrict__ dbeta, int rev) {
-  pdl_enter();
   const int groups = C / 8;
   const int64_t first = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int cg = fixed_channel_group(first, nvec, groups, rev);
@@ -645,128 +638,21 @@ __global__ void __launch_bounds__(256) bn_relu_maxpool_fwd_kernel(
   }
 }
 
-// Forward on 2x2 blocks of OUTPUT pixels (8 channels per thread): the four 3x3/s2 windows of a block cover a 5x5
-// input patch, so BN+ReLU+rounding is evaluated 25 times for 4 outputs instead of 36, two channels per
-// cvt.rn.relu.bf16x2, and the running (max, first arg-max) pair is ONE unsigned max per candidate: the rounded
-// activation is a non-negative bf16, so its fp32 bit pattern orders like the value and has 16 free low bits,
-// which hold 15 - tap — equal values keep the smallest tap, the "first maximum in scan order" rule of ATen's
-// max-pool.  (The per-output kernel above spends 8 instructions per candidate and was issue-bound: 64 % SM
-// issue utilisation at 24 % of DRAM bandwidth.)  The conv output at the arg-max is re-read (an L1 hit).
+// BN+ReLU+rounding of two channels in one cvt.rn.relu.bf16x2: the rounded activation is a non-negative bf16, so its
+// fp32 bit pattern orders like the value and has 16 free low bits for an arg-max tag (the keys below).
 __device__ __forceinline__ uint32_t relu_pack_bf16x2(float hi, float lo) {
   uint32_t r;
   asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r & 0x7fff7fffu;  // -0 -> +0: the keys below compare as unsigned integers
 }
 
-__global__ void __launch_bounds__(256) bn_relu_maxpool_fwd2_kernel(
-    const bf16* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ shift,
-    bf16* __restrict__ y, uint8_t* __restrict__ amax, bf16* __restrict__ xmax, int N, int H, int W, int C, int Ho,
-    int Wo, int rev) {
-  __shared__ float s_scale[512], s_shift[512];
-  __shared__ int s_tapoff[16];  // element offset of tap (r,s) from the window's top-left pixel
-  for (int c = threadIdx.x; c < C; c += blockDim.x) {
-    s_scale[c] = scale[c];
-    s_shift[c] = shift[c];
-  }
-  if (threadIdx.x < 9) s_tapoff[threadIdx.x] = ((threadIdx.x / 3) * W + threadIdx.x % 3) * C;
-  __syncthreads();
-  const int groups = C / 8;
-  const int HB = (Ho + 1) / 2, WB = (Wo + 1) / 2;
-  // 32-bit index arithmetic: the launcher checks that every element index of x fits in an int
-  const int total = N * HB * WB * groups;
-  for (int i0 = blockIdx.x * blockDim.x + threadIdx.x; i0 < total; i0 += gridDim.x * blockDim.x) {
-    const int i = rev ? total - 1 - i0 : i0;  // gdl_set_sweep: start on the producer's tail that is still in L2
-    const int cg = i % groups;
-    int t = i / groups;
-    const int wb = t % WB;
-    t /= WB;
-    const int hb = t % HB;
-    const int n = t / HB;
-    float sc[8], sh[8];
-    uint32_t key[2][2][8];
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      sc[c] = s_scale[cg * 8 + c];
-      sh[c] = s_shift[cg * 8 + c];
-      key[0][0][c] = key[0][1][c] = key[1][0][c] = key[1][1][c] = 0u;
-    }
-    const int h0 = 4 * hb - 1, w0 = 4 * wb - 1;
-    const bf16* xn = x + (int64_t)n * H * W * C + cg * 8;
-#pragma unroll
-    for (int r = 0; r < 5; ++r) {
-      const int h = h0 + r;
-      if (h < 0 || h >= H) continue;
-#pragma unroll
-      for (int s = 0; s < 5; ++s) {
-        const int w = w0 + s;
-        if (w < 0 || w >= W) continue;
-        const uint4 u = *reinterpret_cast<const uint4*>(xn + (h * W + w) * C);
-        const uint32_t wd[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float f0 = __uint_as_float(wd[j] << 16), f1 = __uint_as_float(wd[j] & 0xffff0000u);
-          const uint32_t pk = relu_pack_bf16x2(fmaf(f1, sc[2 * j + 1], sh[2 * j + 1]), fmaf(f0, sc[2 * j], sh[2 * j]));
-          const uint32_t k0 = pk << 16, k1 = pk & 0xffff0000u;
-#pragma unroll
-          for (int oy = 0; oy < 2; ++oy) {
-            if (r < 2 * oy || r > 2 * oy + 2) continue;
-#pragma unroll
-            for (int ox = 0; ox < 2; ++ox) {
-              if (s < 2 * ox || s > 2 * ox + 2) continue;
-              const uint32_t tag = 15u - uint32_t((r - 2 * oy) * 3 + (s - 2 * ox));
-              key[oy][ox][2 * j] = max(key[oy][ox][2 * j], k0 | tag);
-              key[oy][ox][2 * j + 1] = max(key[oy][ox][2 * j + 1], k1 | tag);
-            }
-          }
-        }
-      }
-    }
-#pragma unroll
-    for (int oy = 0; oy < 2; ++oy) {
-      const int ho = 2 * hb + oy;
-      if (ho >= Ho) continue;
-#pragma unroll
-      for (int ox = 0; ox < 2; ++ox) {
-        const int wo = 2 * wb + ox;
-        if (wo >= Wo) continue;
-        const int64_t off = (int64_t)((n * Ho + ho) * Wo + wo) * C + cg * 8;
-        uint4 yv;
-        uint32_t* yw = reinterpret_cast<uint32_t*>(&yv);
-        uint32_t tap[8];
-#pragma unroll
-        for (int c = 0; c < 8; ++c) tap[c] = 15u - (key[oy][ox][c] & 15u);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) yw[j] = (key[oy][ox][2 * j] >> 16) | (key[oy][ox][2 * j + 1] & 0xffff0000u);
-        *reinterpret_cast<uint4*>(y + off) = yv;
-        uint2 packed;
-        packed.x = tap[0] | (tap[1] << 8) | (tap[2] << 16) | (tap[3] << 24);
-        packed.y = tap[4] | (tap[5] << 8) | (tap[6] << 16) | (tap[7] << 24);
-        *reinterpret_cast<uint2*>(amax + off) = packed;
-        if (xmax != nullptr) {
-          // conv output at the arg-max: re-read (L1 hit) through the tap-offset table
-          const unsigned short* xw = reinterpret_cast<const unsigned short*>(xn) + ((2 * ho - 1) * W + (2 * wo - 1)) * C;
-          uint32_t xb[8];
-#pragma unroll
-          for (int c = 0; c < 8; ++c) xb[c] = xw[s_tapoff[tap[c]] + c];
-          uint4 xv;
-          xv.x = xb[0] | (xb[1] << 16);
-          xv.y = xb[2] | (xb[3] << 16);
-          xv.z = xb[4] | (xb[5] << 16);
-          xv.w = xb[6] | (xb[7] << 16);
-          *reinterpret_cast<uint4*>(xmax + off) = xv;
-        }
-      }
-    }
-  }
-}
-
-// v3: column sweep.  One thread per (image, segment of kTailSeg output rows, output column, 8-channel group) walks
+// Column sweep.  One thread per (image, segment of kTailSeg output rows, output column, 8-channel group) walks
 // down its column: every input row is loaded and BN+ReLU-evaluated ONCE per thread (3 pixels: 1.5 evaluations per
 // output-row pixel instead of 6.25 per 2x2 block), the max is separable — horizontal max of a row with the column tag
 // (2 - s) in the key's low bits, then vertical max with the row tag 3*(2 - r) added — and the bottom row of one window
 // is the top row of the next.  Key = bf16 bits of the activation << 16 | (8 - tap): one unsigned max per candidate gives
 // the value and the FIRST arg-max in scan order (ATen's rule).  ~330 instructions per output pixel and 8 channels
-// (v2: ~640), all six loads of an iteration issued before any is consumed.
+// (~640 for one thread per 2x2 output block), all six loads of an iteration issued before any is consumed.
 constexpr int kTailSeg = 14;
 
 __device__ __forceinline__ void tail_row_keys(const uint4& u, const float (&sc)[8], const float (&sh)[8], uint32_t tag,
@@ -785,7 +671,6 @@ __global__ void __launch_bounds__(256, 3) bn_relu_maxpool_fwd3_kernel(
     const bf16* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ shift,
     bf16* __restrict__ y, uint8_t* __restrict__ amax, bf16* __restrict__ xmax, int N, int H, int W, int C, int Ho,
     int Wo, int nseg, int seglen, int rev) {
-  pdl_enter();
   __shared__ int s_tapoff[16];  // element offset of tap (r,s) from the window's top-left pixel
   if (threadIdx.x < 9) s_tapoff[threadIdx.x] = ((threadIdx.x / 3) * W + threadIdx.x % 3) * C;
   __syncthreads();
@@ -996,7 +881,6 @@ __global__ void __launch_bounds__(256, 2) bn_relu_maxpool_bwd_apply_kernel(
     const float* __restrict__ gamma, const float* __restrict__ mean, const float* __restrict__ invstd,
     const float* __restrict__ scale, const float* __restrict__ shift, const float* __restrict__ dgamma,
     const float* __restrict__ dbeta) {
-  pdl_enter();
   // per-channel coefficients in registers: the grid stride is a multiple of C/8, so a thread keeps its channel group
   // (the shared-memory tables cost 40 LDS.128 per block); block indices are 32-bit (the launcher checks the range)
   const int groups = C / 8;
@@ -1061,7 +945,6 @@ __global__ void __launch_bounds__(256, 2) bn_relu_maxpool_bwd_apply_kernel(
 // ------------------------------------------------------------------------------------------
 __global__ void gap_fwd_kernel(const bf16* __restrict__ x, float* __restrict__ out, int B, int G,
                                int C) {
-  pdl_enter();
   const int groups = C / 8;
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (int64_t)B * groups) return;
@@ -1084,7 +967,6 @@ __global__ void gap_fwd_kernel(const bf16* __restrict__ x, float* __restrict__ o
 
 __global__ void gap_bwd_kernel(const float* __restrict__ dout, bf16* __restrict__ dx, int B, int G,
                                int C) {
-  pdl_enter();
   const int groups = C / 8;
   const int64_t total = (int64_t)B * G * groups;
   const float inv = 1.f / (float)G;
@@ -1136,7 +1018,7 @@ extern "C" int gdl_bn_stats(const void* x, int64_t P, int C, float* partial, con
   int nblk = bn_blocks_cap(P, C, GDL_RESIDENT(bn_stats_kernel, kBnThreads));
   bn_stats_kernel<<<nblk, kBnThreads, 0, (cudaStream_t)s>>>((const bf16*)x, P, C, partial, g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_stats_kernel");
-  launch_pdl(bn_stats_finalize_kernel, (C * 32 + 255) / 256, 256, 0, (cudaStream_t)s, partial, nblk, P, C, gamma, beta, eps, momentum, running_mean, running_var, mean, invstd, scale, shift);
+  bn_stats_finalize_kernel<<<(C * 32 + 255) / 256, 256, 0, (cudaStream_t)s>>>(partial, nblk, P, C, gamma, beta, eps, momentum, running_mean, running_var, mean, invstd, scale, shift);
   GDL_CHECK_LAUNCH("bn_stats_finalize_kernel");
   return GDL_OK;
 }
@@ -1147,7 +1029,7 @@ extern "C" int gdl_bn_stats_finalize(const float* partial, int rows, int64_t P, 
                                      gdl_stream_t s) {
   GDL_REQUIRE(chan_ok(C) && P > 0 && rows > 0, "gdl_bn_stats_finalize: bad shape");
   GDL_REQUIRE(partial && gamma && beta && mean && invstd && scale && shift, "gdl_bn_stats_finalize: null pointer");
-  launch_pdl(bn_stats_finalize_kernel, (C * 32 + 255) / 256, 256, 0, (cudaStream_t)s, partial, rows, P, C, gamma, beta, eps, momentum, running_mean, running_var, mean, invstd, scale, shift);
+  bn_stats_finalize_kernel<<<(C * 32 + 255) / 256, 256, 0, (cudaStream_t)s>>>(partial, rows, P, C, gamma, beta, eps, momentum, running_mean, running_var, mean, invstd, scale, shift);
   GDL_CHECK_LAUNCH("bn_stats_finalize_kernel");
   return GDL_OK;
 }
@@ -1167,7 +1049,7 @@ extern "C" int gdl_bn_apply(const void* x, const void* res, void* y, int64_t P, 
   GDL_REQUIRE(chan_ok(C) && P > 0, "gdl_bn_apply: bad shape");
   GDL_REQUIRE(x && y && scale && shift, "gdl_bn_apply: null pointer");
   int64_t nvec = P * C / 8;
-  launch_pdl(bn_apply_kernel, ew_grid(nvec, 256, GDL_RESIDENT(bn_apply_kernel, 256)), 256, 0, (cudaStream_t)s, (const bf16*)x, (const bf16*)res,
+  bn_apply_kernel<<<ew_grid(nvec, 256, GDL_RESIDENT(bn_apply_kernel, 256)), 256, 0, (cudaStream_t)s>>>((const bf16*)x, (const bf16*)res,
                                                                   (bf16*)y, nvec, C, scale, shift, relu, g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_apply_kernel");
   return GDL_OK;
@@ -1181,14 +1063,14 @@ extern "C" int gdl_bn_bwd(const void* dy, const void* y, const void* x, void* dz
   GDL_REQUIRE(dy && x && dx && gamma && mean && invstd && partial && dgamma && dbeta, "gdl_bn_bwd: null pointer");
   GDL_REQUIRE(!relu || (y && dz), "gdl_bn_bwd: relu needs y and dz");
   int nblk = bn_blocks_cap(P, C, GDL_RESIDENT(bn_bwd_reduce_kernel, kBnThreads));
-  launch_pdl(bn_bwd_reduce_kernel, nblk, kBnThreads, 0, (cudaStream_t)s, (const bf16*)dy, (const bf16*)y, (const bf16*)x, (bf16*)dz, P, C, partial, relu, g_sweep_rev);
+  bn_bwd_reduce_kernel<<<nblk, kBnThreads, 0, (cudaStream_t)s>>>((const bf16*)dy, (const bf16*)y, (const bf16*)x, (bf16*)dz, P, C, partial, relu, g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_bwd_reduce_kernel");
-  launch_pdl(bn_bwd_finalize_raw_kernel, (C * 32 + 255) / 256, 256, 0, (cudaStream_t)s, partial, nblk, C, mean, invstd, dgamma,
+  bn_bwd_finalize_raw_kernel<<<(C * 32 + 255) / 256, 256, 0, (cudaStream_t)s>>>(partial, nblk, C, mean, invstd, dgamma,
                                                                                dbeta);
   GDL_CHECK_LAUNCH("bn_bwd_finalize_raw_kernel");
   int64_t nvec = P * C / 8;
   const bf16* dzp = relu ? (const bf16*)dz : (const bf16*)dy;
-  launch_pdl(bn_bwd_apply_kernel, ew_grid(nvec, 256, GDL_RESIDENT(bn_bwd_apply_kernel, 256)), 256, 0, (cudaStream_t)s, dzp, (const bf16*)x, (bf16*)dx, nvec, C, 1.f / (float)P, gamma, mean, invstd, dgamma, dbeta, !g_sweep_rev);
+  bn_bwd_apply_kernel<<<ew_grid(nvec, 256, GDL_RESIDENT(bn_bwd_apply_kernel, 256)), 256, 0, (cudaStream_t)s>>>(dzp, (const bf16*)x, (bf16*)dx, nvec, C, 1.f / (float)P, gamma, mean, invstd, dgamma, dbeta, !g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_bwd_apply_kernel");
   return GDL_OK;
 }
@@ -1200,14 +1082,14 @@ extern "C" int gdl_bn_bwd_nores(const void* dy, const void* x, void* dx, int64_t
   GDL_REQUIRE(dy && x && dx && gamma && mean && invstd && scale && shift && partial && dgamma && dbeta,
               "gdl_bn_bwd_nores: null pointer");
   int nblk = bn_blocks_cap(P, C, GDL_RESIDENT(bn_bwd_nores_reduce_kernel, kBnThreads));
-  launch_pdl(bn_bwd_nores_reduce_kernel, nblk, kBnThreads, 0, (cudaStream_t)s, (const bf16*)dy, (const bf16*)x, P, C, scale,
+  bn_bwd_nores_reduce_kernel<<<nblk, kBnThreads, 0, (cudaStream_t)s>>>((const bf16*)dy, (const bf16*)x, P, C, scale,
                                                                       shift, partial, g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_bwd_nores_reduce_kernel");
-  launch_pdl(bn_bwd_finalize_raw_kernel, (C * 32 + 255) / 256, 256, 0, (cudaStream_t)s, partial, nblk, C, mean, invstd, dgamma,
+  bn_bwd_finalize_raw_kernel<<<(C * 32 + 255) / 256, 256, 0, (cudaStream_t)s>>>(partial, nblk, C, mean, invstd, dgamma,
                                                                                dbeta);
   GDL_CHECK_LAUNCH("bn_bwd_finalize_raw_kernel");
   int64_t nvec = P * C / 8;
-  launch_pdl(bn_bwd_nores_apply_kernel, ew_grid(nvec, 256, GDL_RESIDENT(bn_bwd_nores_apply_kernel, 256)), 256, 0, (cudaStream_t)s, (const bf16*)dy, (const bf16*)x, (bf16*)dx, nvec, C, 1.f / (float)P, gamma, mean, invstd, scale, shift, dgamma,
+  bn_bwd_nores_apply_kernel<<<ew_grid(nvec, 256, GDL_RESIDENT(bn_bwd_nores_apply_kernel, 256)), 256, 0, (cudaStream_t)s>>>((const bf16*)dy, (const bf16*)x, (bf16*)dx, nvec, C, 1.f / (float)P, gamma, mean, invstd, scale, shift, dgamma,
       dbeta, !g_sweep_rev);
   GDL_CHECK_LAUNCH("bn_bwd_nores_apply_kernel");
   return GDL_OK;
@@ -1218,30 +1100,13 @@ extern "C" int gdl_bn_relu_maxpool_fwd(const void* x, const float* scale, const 
                                        gdl_stream_t s) {
   GDL_REQUIRE(x && scale && shift && y && argmax, "gdl_bn_relu_maxpool_fwd: null pointer");
   GDL_REQUIRE(chan_ok(C) && Ho == (H - 1) / 2 + 1 && Wo == (W - 1) / 2 + 1, "gdl_bn_relu_maxpool_fwd: bad shape");
-  // GDL_STEM_TAIL: 3 (default) = column sweep, 2 = one thread per 2x2 output block with packed max/arg-max keys,
-  // 1 = one thread per output
-  static const int variant = []() {
-    const char* e = getenv("GDL_STEM_TAIL");
-    return e ? atoi(e) : 3;
-  }();
-  if (variant >= 3 && (int64_t)N * H * W * C < ((int64_t)1 << 31)) {  // 32-bit indexing inside the kernel
-    static const int seglen = []() {
-      const char* e = getenv("GDL_STEM_TAIL_SEG");
-      return e && atoi(e) > 0 ? atoi(e) : kTailSeg;
-    }();
-    const int nseg = (Ho + seglen - 1) / seglen;
+  if ((int64_t)N * H * W * C < ((int64_t)1 << 31)) {  // 32-bit indexing inside the kernel
+    const int nseg = (Ho + kTailSeg - 1) / kTailSeg;
     int64_t total3 = (int64_t)N * nseg * Wo * (C / 8);
-    launch_pdl(bn_relu_maxpool_fwd3_kernel, ew_grid(total3, 256, GDL_RESIDENT(bn_relu_maxpool_fwd3_kernel, 256)), 256, 0, (cudaStream_t)s, (const bf16*)x, scale, shift, (bf16*)y, argmax, (bf16*)xmax, N, H,
-                                                     W, C, Ho, Wo, nseg, seglen, g_sweep_rev);
-    GDL_CHECK_LAUNCH("bn_relu_maxpool_fwd3_kernel");
-    return GDL_OK;
-  }
-  if (variant >= 2 && (int64_t)N * H * W * C < ((int64_t)1 << 31)) {  // the v2 kernel indexes with 32-bit integers
-    int64_t total2 = (int64_t)N * ((Ho + 1) / 2) * ((Wo + 1) / 2) * (C / 8);
-    bn_relu_maxpool_fwd2_kernel<<<ew_grid(total2, 256, GDL_RESIDENT(bn_relu_maxpool_fwd2_kernel, 256)), 256, 0,
+    bn_relu_maxpool_fwd3_kernel<<<ew_grid(total3, 256, GDL_RESIDENT(bn_relu_maxpool_fwd3_kernel, 256)), 256, 0,
                                   (cudaStream_t)s>>>((const bf16*)x, scale, shift, (bf16*)y, argmax, (bf16*)xmax, N, H,
-                                                     W, C, Ho, Wo, g_sweep_rev);
-    GDL_CHECK_LAUNCH("bn_relu_maxpool_fwd2_kernel");
+                                                     W, C, Ho, Wo, nseg, kTailSeg, g_sweep_rev);
+    GDL_CHECK_LAUNCH("bn_relu_maxpool_fwd3_kernel");
     return GDL_OK;
   }
   int64_t total = (int64_t)N * Ho * Wo * (C / 8);
@@ -1266,10 +1131,10 @@ extern "C" int gdl_bn_relu_maxpool_bwd(const void* gpool, const uint8_t* argmax,
     // whose conv output the forward saved — the no-residual BN reduce kernel on (gpool, xmax)
     const int64_t Pp = (int64_t)N * Ho * Wo;
     nblk = bn_blocks_cap(Pp, C, GDL_RESIDENT(bn_bwd_nores_reduce_kernel, kBnThreads));
-    launch_pdl(bn_bwd_nores_reduce_kernel, nblk, kBnThreads, 0, (cudaStream_t)s, (const bf16*)gpool, (const bf16*)xmax, Pp, C,
+    bn_bwd_nores_reduce_kernel<<<nblk, kBnThreads, 0, (cudaStream_t)s>>>((const bf16*)gpool, (const bf16*)xmax, Pp, C,
                                                                         scale, shift, partial, g_sweep_rev);
     GDL_CHECK_LAUNCH("bn_bwd_nores_reduce_kernel(stem tail)");
-    launch_pdl(bn_bwd_finalize_raw_kernel, (C * 32 + 255) / 256, 256, 0, (cudaStream_t)s, partial, nblk, C, mean, invstd, dgamma,
+    bn_bwd_finalize_raw_kernel<<<(C * 32 + 255) / 256, 256, 0, (cudaStream_t)s>>>(partial, nblk, C, mean, invstd, dgamma,
                                                                                  dbeta);
   } else {
     nblk = bn_blocks_cap((int64_t)N * Ho * Wo * 4, C, GDL_RESIDENT(bn_relu_maxpool_bwd_reduce_kernel, kBnThreads));
@@ -1281,7 +1146,7 @@ extern "C" int gdl_bn_relu_maxpool_bwd(const void* gpool, const uint8_t* argmax,
   GDL_CHECK_LAUNCH("bn_bwd_finalize_kernel");
   int64_t total = (int64_t)N * Ho * Wo * (C / 8);
   GDL_REQUIRE(total < ((int64_t)1 << 30), "gdl_bn_relu_maxpool_bwd: too many pooled pixels for 32-bit block indices");
-  launch_pdl(bn_relu_maxpool_bwd_apply_kernel, ew_grid(total, 256, GDL_RESIDENT(bn_relu_maxpool_bwd_apply_kernel, 256)), 256, 0, (cudaStream_t)s, (const bf16*)gpool, argmax, (const bf16*)x, (bf16*)dx, N, H, W, C, Ho, Wo, 1.f / (float)P, gamma, mean, invstd,
+  bn_relu_maxpool_bwd_apply_kernel<<<ew_grid(total, 256, GDL_RESIDENT(bn_relu_maxpool_bwd_apply_kernel, 256)), 256, 0, (cudaStream_t)s>>>((const bf16*)gpool, argmax, (const bf16*)x, (bf16*)dx, N, H, W, C, Ho, Wo, 1.f / (float)P, gamma, mean, invstd,
       scale, shift, dgamma, dbeta);
   GDL_CHECK_LAUNCH("bn_relu_maxpool_bwd_apply_kernel");
   return GDL_OK;
@@ -1312,7 +1177,7 @@ extern "C" int gdl_maxpool_bwd(const void* dy, const uint8_t* argmax, void* dx, 
 extern "C" int gdl_gap_fwd(const void* x, float* out, int B, int G, int C, gdl_stream_t s) {
   GDL_REQUIRE(x && out && B > 0 && G > 0 && C % 8 == 0, "gdl_gap_fwd: bad arguments");
   int64_t total = (int64_t)B * (C / 8);
-  launch_pdl(gap_fwd_kernel, (unsigned)ceil_div64(total, 128), 128, 0, (cudaStream_t)s, (const bf16*)x, out, B, G, C);
+  gap_fwd_kernel<<<(unsigned)ceil_div64(total, 128), 128, 0, (cudaStream_t)s>>>((const bf16*)x, out, B, G, C);
   GDL_CHECK_LAUNCH("gap_fwd_kernel");
   return GDL_OK;
 }
@@ -1320,7 +1185,7 @@ extern "C" int gdl_gap_fwd(const void* x, float* out, int B, int G, int C, gdl_s
 extern "C" int gdl_gap_bwd(const float* dout, void* dx, int B, int G, int C, gdl_stream_t s) {
   GDL_REQUIRE(dout && dx && B > 0 && G > 0 && C % 8 == 0, "gdl_gap_bwd: bad arguments");
   int64_t total = (int64_t)B * G * (C / 8);
-  launch_pdl(gap_bwd_kernel, ew_grid(total, 256), 256, 0, (cudaStream_t)s, dout, (bf16*)dx, B, G, C);
+  gap_bwd_kernel<<<ew_grid(total, 256), 256, 0, (cudaStream_t)s>>>(dout, (bf16*)dx, B, G, C);
   GDL_CHECK_LAUNCH("gap_bwd_kernel");
   return GDL_OK;
 }

@@ -85,7 +85,6 @@ __global__ void __launch_bounds__(kEvalThreads) eval_head_kernel(
     const float* __restrict__ Wo, const float* __restrict__ bo, int x_gate, const int64_t* __restrict__ labels,
     float* __restrict__ a_out, float* __restrict__ v_out, float* __restrict__ logits,
     unsigned long long* __restrict__ counts, int B, int n) {
-  pdl_enter();
   constexpr int D = kEvalD;
   __shared__ float s_a[D], s_v[D];
   __shared__ float s_m[4][D];  // pooling partials, then the gated head's h_x, h_y and its three gated vectors
@@ -183,7 +182,6 @@ __global__ void __launch_bounds__(kEvalThreads) eval_head_kernel(
 // one warp per (head, row) of logits [3][B][n]
 __global__ void eval_count_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels,
                                   unsigned long long* __restrict__ counts, int B, int n) {
-  pdl_enter();
   const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (w >= 3 * (int64_t)B) return;
   const int h = int(w / B), b = int(w - (int64_t)h * B);
@@ -196,7 +194,6 @@ __global__ void eval_count_kernel(const float* __restrict__ logits, const int64_
 __global__ void eval_confusion_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels,
                                       unsigned long long* __restrict__ conf,
                                       unsigned long long* __restrict__ out_of_range, int B, int n) {
-  pdl_enter();
   const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (w >= 3 * (int64_t)B) return;
   const int h = int(w / B), b = int(w - (int64_t)h * B);
@@ -232,7 +229,6 @@ __global__ void __launch_bounds__(kScoreThreads) eval_scores_kernel(
     const float* __restrict__ logits, const int64_t* __restrict__ labels, float* __restrict__ store,
     int* __restrict__ store_labels, const int64_t* __restrict__ cursor, unsigned long long* __restrict__ hits,
     unsigned long long* __restrict__ overflow, int64_t cap, int B, int n, int k) {
-  pdl_enter();
   __shared__ float s_max[kScoreRows], s_sum[kScoreRows];
   __shared__ unsigned s_hits;
   const int h = blockIdx.y, r0 = blockIdx.x * kScoreRows;
@@ -282,7 +278,6 @@ __global__ void __launch_bounds__(kScoreThreads) eval_scores_kernel(
 
 // after every CTA of eval_scores_kernel has read the cursor (stream order)
 __global__ void eval_scores_advance_kernel(int64_t* __restrict__ cursor, int B) {
-  pdl_enter();
   *cursor += B;
 }
 
@@ -324,7 +319,6 @@ __global__ void __launch_bounds__(kApThreads) eval_ap_kernel(const float* __rest
                                                              const int64_t* __restrict__ cursor, int64_t cap, int n,
                                                              double* __restrict__ ap, int64_t* __restrict__ support,
                                                              unsigned long long* work, int64_t work_stride) {
-  pdl_enter();
   extern __shared__ unsigned long long s_keys[];
   __shared__ int s_int[kApThreads];
   __shared__ int s_end[kApThreads], s_tp[kApThreads];
@@ -417,7 +411,6 @@ __global__ void __launch_bounds__(kApThreads) eval_ap_kernel(const float* __rest
 __global__ void eval_nonfinite_kernel(const float* __restrict__ store, const int* __restrict__ labels,
                                       const int64_t* __restrict__ cursor, int64_t cap, int n,
                                       unsigned long long* __restrict__ nonfinite) {
-  pdl_enter();
   const int64_t N = min(*cursor, cap);
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   bool bad = false;
@@ -457,7 +450,7 @@ extern "C" int gdl_eval_head(int kind, const void* fa, int Ga, const void* fv, i
                 "gdl_eval_head: bad head weights");
     GDL_REQUIRE(labels == nullptr || counts != nullptr, "gdl_eval_head: labels need counts");
   }
-  launch_pdl(eval_head_kernel, B, kEvalThreads, 0, (cudaStream_t)s, kind, (const bf16*)fa, Ga, (const bf16*)fv, Gv,
+  eval_head_kernel<<<B, kEvalThreads, 0, (cudaStream_t)s>>>(kind, (const bf16*)fa, Ga, (const bf16*)fv, Gv,
              Wx, Wy, ldw, bx, by, Wo, bo, x_gate, kind == 3 ? nullptr : labels, a_out, v_out, logits,
              (unsigned long long*)counts, B, n);
   GDL_CHECK_LAUNCH("eval_head_kernel");
@@ -468,7 +461,7 @@ extern "C" int gdl_eval_count(const float* logits, const int64_t* labels, int64_
                               gdl_stream_t s) {
   GDL_REQUIRE(logits && labels && counts && B > 0 && n > 0, "gdl_eval_count: bad arguments");
   const int64_t threads = 3 * (int64_t)B * 32;
-  launch_pdl(eval_count_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s, logits, labels,
+  eval_count_kernel<<<(unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s>>>(logits, labels,
              (unsigned long long*)counts, B, n);
   GDL_CHECK_LAUNCH("eval_count_kernel");
   return GDL_OK;
@@ -480,7 +473,7 @@ extern "C" int gdl_eval_confusion(const float* logits, const int64_t* labels, in
   GDL_REQUIRE(B > 0, "gdl_eval_confusion: B must be positive");
   GDL_REQUIRE(n > 0 && n <= kEvalMaxN, "gdl_eval_confusion: n must be in 1..512");
   const int64_t threads = 3 * (int64_t)B * 32;
-  launch_pdl(eval_confusion_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s, logits, labels,
+  eval_confusion_kernel<<<(unsigned)ceil_div64(threads, 256), 256, 0, (cudaStream_t)s>>>(logits, labels,
              (unsigned long long*)conf, (unsigned long long*)out_of_range, B, n);
   GDL_CHECK_LAUNCH("eval_confusion_kernel");
   return GDL_OK;
@@ -495,10 +488,10 @@ extern "C" int gdl_eval_scores(const float* logits, const int64_t* labels, int B
   GDL_REQUIRE(k > 0 && k <= n, "gdl_eval_scores: k must be in 1..n");
   GDL_REQUIRE(cap > 0 && cap <= kApMaxCap, "gdl_eval_scores: cap must be in 1..2^28");
   const dim3 grid((unsigned)ceil_div64(B, kScoreRows), 3);
-  launch_pdl(eval_scores_kernel, grid, kScoreThreads, 0, (cudaStream_t)s, logits, labels, store, (int*)store_labels,
+  eval_scores_kernel<<<grid, kScoreThreads, 0, (cudaStream_t)s>>>(logits, labels, store, (int*)store_labels,
              (const int64_t*)cursor, (unsigned long long*)hits, (unsigned long long*)overflow, cap, B, n, k);
   GDL_CHECK_LAUNCH("eval_scores_kernel");
-  launch_pdl(eval_scores_advance_kernel, 1, 1, 0, (cudaStream_t)s, cursor, B);
+  eval_scores_advance_kernel<<<1, 1, 0, (cudaStream_t)s>>>(cursor, B);
   GDL_CHECK_LAUNCH("eval_scores_advance_kernel");
   return GDL_OK;
 }
@@ -521,7 +514,7 @@ extern "C" int gdl_eval_ap(const float* store, const int32_t* store_labels, cons
   const cudaStream_t st = (cudaStream_t)s;
   cudaError_t e = cudaMemsetAsync(nonfinite, 0, sizeof(int64_t), st);
   if (e != cudaSuccess) return cuda_fail(e, "gdl_eval_ap: cudaMemsetAsync");
-  launch_pdl(eval_nonfinite_kernel, (unsigned)ceil_div64(cap, 256), 256, 0, st, store, (const int*)store_labels,
+  eval_nonfinite_kernel<<<(unsigned)ceil_div64(cap, 256), 256, 0, st>>>(store, (const int*)store_labels,
              cursor, cap, n, (unsigned long long*)nonfinite);
   GDL_CHECK_LAUNCH("eval_nonfinite_kernel");
   const int64_t M = ap_sort_len(cap);
@@ -529,7 +522,7 @@ extern "C" int gdl_eval_ap(const float* store, const int32_t* store_labels, cons
   e = cudaFuncSetAttribute(eval_ap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                            (int)(kApSmemKeys * sizeof(unsigned long long)));
   if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(eval_ap_kernel)");
-  launch_pdl(eval_ap_kernel, 3 * n, kApThreads, smem, st, store, (const int*)store_labels, cursor, cap, n, ap, support,
+  eval_ap_kernel<<<3 * n, kApThreads, smem, st>>>(store, (const int*)store_labels, cursor, cap, n, ap, support,
              need == 0 ? nullptr : (unsigned long long*)workspace, need == 0 ? (int64_t)0 : M);
   GDL_CHECK_LAUNCH("eval_ap_kernel");
   return GDL_OK;

@@ -100,7 +100,6 @@ __global__ void __launch_bounds__(kHeadThreads) dgl_head_sample_kernel(
     const int64_t* __restrict__ labels, float alpha, float inv_batch, float* __restrict__ logits,
     float* __restrict__ da, float* __restrict__ dv, float* __restrict__ g_out_all,
     float* __restrict__ loss_rows, int B, int D, int n) {
-  pdl_enter();
   __shared__ float s_a[kHeadMaxD], s_v[kHeadMaxD];
   __shared__ float s_z[3][kHeadMaxN];  // out, x_out, y_out
   __shared__ float s_g[3][kHeadMaxN];
@@ -165,7 +164,6 @@ __global__ void dgl_head_param_kernel(int kind, const float* __restrict__ a,
                                       float* __restrict__ dWx, float* __restrict__ dWy, int lddw,
                                       float* __restrict__ dbx, float* __restrict__ dby,
                                       float* __restrict__ losses, int B, int D, int n) {
-  pdl_enter();
   int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t nW = (int64_t)n * 2 * D;
   if (idx < nW) {
@@ -261,7 +259,6 @@ __global__ void __launch_bounds__(kHeadThreads) dgl_gated_sample_kernel(
     const int64_t* __restrict__ labels, float alpha, float inv_batch, float* __restrict__ logits, float* __restrict__ da,
     float* __restrict__ dv, float* __restrict__ m_out_all, float* __restrict__ g_out_all, float* __restrict__ loss_rows,
     int B, int n) {
-  pdl_enter();
   constexpr int D = kGatedD;
   __shared__ float s_a[D], s_v[D], s_hx[D], s_hy[D];
   __shared__ float s_m[3][D];            // m_out, m_x, m_y; later reused for dhx (row 1) and dhy (row 2)
@@ -361,7 +358,6 @@ __global__ void __launch_bounds__(kHeadThreads) dgl_gated_sample_kernel(
 __global__ void dgl_gated_param_kernel(const float* __restrict__ m_out, const float* __restrict__ g_out,
                                        const float* __restrict__ loss_rows, float inv_batch, float* __restrict__ dWo,
                                        float* __restrict__ dbo, float* __restrict__ losses, int B, int n) {
-  pdl_enter();
   constexpr int D = kGatedD;
   int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t nW = (int64_t)n * D;
@@ -429,12 +425,12 @@ extern "C" int gdl_dgl_head_linear(int kind, const float* a, const float* v, con
   GDL_REQUIRE(B > 0 && D > 0 && D <= kHeadMaxD && n > 0 && n <= kHeadMaxN, "gdl_dgl_head_linear: bad shape");
   float* g_out = scratch;
   float* loss_rows = scratch + (int64_t)B * n;
-  launch_pdl(dgl_head_sample_kernel, B, kHeadThreads, 0, (cudaStream_t)s, kind, a, v, Wx, Wy, ldw, bx, by, labels,
+  dgl_head_sample_kernel<<<B, kHeadThreads, 0, (cudaStream_t)s>>>(kind, a, v, Wx, Wy, ldw, bx, by, labels,
                                                                   alpha, inv_batch, logits, da, dv, g_out,
                                                                   loss_rows, B, D, n);
   GDL_CHECK_LAUNCH("dgl_head_sample_kernel");
   int64_t total = (int64_t)n * 2 * D + n + 3;
-  launch_pdl(dgl_head_param_kernel, (unsigned)ceil_div64(total, 256), 256, 0, (cudaStream_t)s, kind, a, v, g_out, loss_rows, inv_batch, dWx, dWy, lddw, dbx, dby, losses, B, D, n);
+  dgl_head_param_kernel<<<(unsigned)ceil_div64(total, 256), 256, 0, (cudaStream_t)s>>>(kind, a, v, g_out, loss_rows, inv_batch, dWx, dWy, lddw, dbx, dby, losses, B, D, n);
   GDL_CHECK_LAUNCH("dgl_head_param_kernel");
   return GDL_OK;
 }
@@ -480,11 +476,11 @@ extern "C" int gdl_dgl_head_gated(const float* a, const float* v, const float* W
   float* m_out = scratch;
   float* g_out = m_out + (int64_t)B * D;
   float* loss_rows = g_out + (int64_t)B * n;
-  launch_pdl(dgl_gated_sample_kernel, B, kHeadThreads, 0, (cudaStream_t)s, a, v, Wx, bx, Wy, by, Wo, bo, labels, alpha, inv_batch,
+  dgl_gated_sample_kernel<<<B, kHeadThreads, 0, (cudaStream_t)s>>>(a, v, Wx, bx, Wy, by, Wo, bo, labels, alpha, inv_batch,
                                                                    logits, da, dv, m_out, g_out, loss_rows, B, n);
   GDL_CHECK_LAUNCH("dgl_gated_sample_kernel");
   const int64_t total = (int64_t)n * D + n + 3;
-  launch_pdl(dgl_gated_param_kernel, (unsigned)ceil_div64(total, 256), 256, 0, (cudaStream_t)s, m_out, g_out, loss_rows, inv_batch,
+  dgl_gated_param_kernel<<<(unsigned)ceil_div64(total, 256), 256, 0, (cudaStream_t)s>>>(m_out, g_out, loss_rows, inv_batch,
                                                                                        dWo, dbo, losses, B, n);
   GDL_CHECK_LAUNCH("dgl_gated_param_kernel");
   return GDL_OK;

@@ -38,7 +38,6 @@ __global__ void __launch_bounds__(kOptThreads) grad_stats_kernel(
     const float* __restrict__ grad, int64_t numel, const int64_t* __restrict__ seg_end,
     const int32_t* __restrict__ seg_group, const float* __restrict__ seg_inv_numel, int nseg,
     float* __restrict__ partial) {
-  pdl_enter();
   __shared__ float red[32];
   __shared__ int s_lo, s_hi;
   const int64_t start = (int64_t)blockIdx.x * kChunk;
@@ -74,7 +73,6 @@ __global__ void __launch_bounds__(kOptThreads) grad_stats_kernel(
 
 __global__ void grad_stats_finalize_kernel(const float* __restrict__ partial, int nblk, float max_norm,
                                            float* __restrict__ stats) {
-  pdl_enter();
   // single block; fixed-order strided accumulation in double, then a fixed tree
   __shared__ double red[3][256];
   double a0 = 0, a1 = 0, a2 = 0;
@@ -113,7 +111,6 @@ __global__ void __launch_bounds__(256) sgd_momentum_kernel(float* __restrict__ p
                                                            const double* __restrict__ lr_dev, float mu,
                                                            float wd, int first,
                                                            const float* __restrict__ stats) {
-  pdl_enter();
   const float coef = stats ? stats[1] : 1.f;
   const float lr = lr_dev ? (float)*lr_dev : lr_host;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
@@ -155,7 +152,6 @@ enum { kRuleAdam = 0, kRuleAdagrad = 1 };
 
 __global__ void optim_step_prologue_kernel(int32_t* __restrict__ step_state, int rule, double lr_host,
                                            const double* __restrict__ lr_dev, double a, double b) {
-  pdl_enter();
   const double lr = lr_dev ? *lr_dev : lr_host;
   const int32_t step = step_state[0] + 1;
   step_state[0] = step;
@@ -175,7 +171,6 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, fl
                                                    int64_t n4, int64_t numel, float w1, float beta2, float w2,
                                                    float eps, float wd, const float* __restrict__ stats,
                                                    const int32_t* __restrict__ step_state) {
-  pdl_enter();
   const float coef = stats ? stats[1] : 1.f;
   const float* sc = reinterpret_cast<const float*>(step_state + 1);
   const float step_size = sc[0], bc2s = sc[1];
@@ -215,7 +210,6 @@ __global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ param,
                                                       float* __restrict__ sum, int64_t n4, int64_t numel, float eps,
                                                       float wd, const float* __restrict__ stats,
                                                       const int32_t* __restrict__ step_state) {
-  pdl_enter();
   const float coef = stats ? stats[1] : 1.f;
   const float clr = reinterpret_cast<const float*>(step_state + 1)[0];
   // s += g*g, p -= clr * g / (sqrt(s) + eps)
@@ -248,7 +242,6 @@ __global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ param,
 // dst = src or dst = dst + src: the gradient sum over replicas run one after another (DGLStep replicas > 1)
 __global__ void __launch_bounds__(256) grad_accumulate_kernel(float* __restrict__ dst, const float* __restrict__ src,
                                                               int64_t n4, int64_t numel, int accumulate) {
-  pdl_enter();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
        i += (int64_t)gridDim.x * blockDim.x) {
     float4 s = reinterpret_cast<const float4*>(src)[i];
@@ -312,10 +305,10 @@ extern "C" int gdl_grad_stats(const float* grad, int64_t numel, const int64_t* s
   GDL_REQUIRE(grad && seg_end && seg_group && seg_inv_numel && scratch && stats_out, "gdl_grad_stats: null pointer");
   GDL_REQUIRE(numel > 0 && nseg > 0, "gdl_grad_stats: bad shape");
   int nblk = (int)ceil_div64(numel, kChunk);
-  launch_pdl(grad_stats_kernel, nblk, kOptThreads, 0, (cudaStream_t)s, grad, numel, seg_end, seg_group,
+  grad_stats_kernel<<<nblk, kOptThreads, 0, (cudaStream_t)s>>>(grad, numel, seg_end, seg_group,
                                                               seg_inv_numel, nseg, scratch);
   GDL_CHECK_LAUNCH("grad_stats_kernel");
-  launch_pdl(grad_stats_finalize_kernel, 1, 256, 0, (cudaStream_t)s, scratch, nblk, max_norm, stats_out);
+  grad_stats_finalize_kernel<<<1, 256, 0, (cudaStream_t)s>>>(scratch, nblk, max_norm, stats_out);
   GDL_CHECK_LAUNCH("grad_stats_finalize_kernel");
   return GDL_OK;
 }
@@ -327,7 +320,7 @@ static int sgd_momentum_launch(float* param, float* grad, float* momentum_buf, i
   GDL_REQUIRE(param && grad && momentum_buf && numel > 0, "gdl_sgd_momentum: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)momentum_buf) & 15) == 0,
               "gdl_sgd_momentum: arenas must be 16-byte aligned");
-  launch_pdl(sgd_momentum_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, momentum_buf,
+  sgd_momentum_kernel<<<elementwise_blocks(numel), 256, 0, (cudaStream_t)s>>>(param, grad, momentum_buf,
              numel / 4, numel, lr, lr_dev, mu, wd, first_step, stats);
   GDL_CHECK_LAUNCH("sgd_momentum_kernel");
   return GDL_OK;
@@ -340,10 +333,10 @@ static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
               "gdl_adam: arenas must be 16-byte aligned");
   GDL_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0, "gdl_adam: betas must lie in [0, 1)");
-  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdam, lr, lr_dev, beta1,
+  optim_step_prologue_kernel<<<1, 1, 0, (cudaStream_t)s>>>(step_state, (int)kRuleAdam, lr, lr_dev, beta1,
              beta2);
   GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
-  launch_pdl(adam_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, exp_avg, exp_avg_sq,
+  adam_kernel<<<elementwise_blocks(numel), 256, 0, (cudaStream_t)s>>>(param, grad, exp_avg, exp_avg_sq,
              numel / 4, numel, (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)eps, (float)wd,
              stats, (const int32_t*)step_state);
   GDL_CHECK_LAUNCH("adam_kernel");
@@ -356,10 +349,10 @@ static int adagrad_launch(float* param, float* grad, float* sum, int32_t* step_s
   GDL_REQUIRE(param && grad && sum && step_state && numel > 0, "gdl_adagrad: bad arguments");
   GDL_REQUIRE((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)sum) & 15) == 0,
               "gdl_adagrad: arenas must be 16-byte aligned");
-  launch_pdl(optim_step_prologue_kernel, 1, 1, 0, (cudaStream_t)s, step_state, (int)kRuleAdagrad, lr, lr_dev,
+  optim_step_prologue_kernel<<<1, 1, 0, (cudaStream_t)s>>>(step_state, (int)kRuleAdagrad, lr, lr_dev,
              lr_decay, 0.0);
   GDL_CHECK_LAUNCH("optim_step_prologue_kernel");
-  launch_pdl(adagrad_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, param, grad, sum, numel / 4, numel,
+  adagrad_kernel<<<elementwise_blocks(numel), 256, 0, (cudaStream_t)s>>>(param, grad, sum, numel / 4, numel,
              (float)eps, (float)wd, stats, (const int32_t*)step_state);
   GDL_CHECK_LAUNCH("adagrad_kernel");
   return GDL_OK;
@@ -407,7 +400,7 @@ extern "C" int gdl_adagrad_lr_dev(float* param, float* grad, float* sum, int32_t
 extern "C" int gdl_grad_accumulate(float* dst, const float* src, int64_t numel, int accumulate, gdl_stream_t s) {
   GDL_REQUIRE(dst && src && numel > 0, "gdl_grad_accumulate: bad arguments");
   GDL_REQUIRE((((uintptr_t)dst | (uintptr_t)src) & 15) == 0, "gdl_grad_accumulate: arenas must be 16-byte aligned");
-  launch_pdl(grad_accumulate_kernel, elementwise_blocks(numel), 256, 0, (cudaStream_t)s, dst, src, numel / 4, numel,
+  grad_accumulate_kernel<<<elementwise_blocks(numel), 256, 0, (cudaStream_t)s>>>(dst, src, numel / 4, numel,
              accumulate);
   GDL_CHECK_LAUNCH("grad_accumulate_kernel");
   return GDL_OK;

@@ -11,14 +11,6 @@
 namespace gdl {
 using namespace tc05;
 
-bool pdl_enabled() {
-  static const bool on = []() {
-    const char* e = getenv("GDL_PDL");
-    return e ? atoi(e) != 0 : false;
-  }();
-  return on;
-}
-
 // ------------------------------------------------------------------------------------------
 // tensor-map cache
 // ------------------------------------------------------------------------------------------

@@ -14,26 +14,15 @@ Data layout in HBM:
                   mean / invstd / fused scale+shift saved for backward
   gradients       activations bf16 NHWC; parameters fp32 written straight into p.grad storage
 """
-import os
-
 import torch
 
 from . import ops
 
 
-# Measured on B=256: no gain (24.05 vs 23.88 ms) — the two encoder streams already keep the GPU busy and the
-# tensor-bound wgrads contend with the BN kernels for L2/HBM; kept as an option, off by default.
-USE_WGRAD_STREAM = os.environ.get("GDL_WGRAD_STREAM", "0") != "0"
-
 # Sweep directions (ops.sweep / gdl_set_sweep): every pass over a tensor larger than L2 leaves its LAST-touched
-# part in the 126 MB L2, so the next pass over the same tensor should start there, i.e. run the other way.
-#   0  every kernel ascending (the behaviour before this option)
-#   1  BatchNorm passes alternate: statistics descending after the (ascending) conv, apply ascending; backward
-#      reduce descending after the (ascending) dgrad, apply ascending
-#   2  the convolutions alternate as well (conv1 of a block descending, conv2 ascending, BN passes in between)
-SWEEP = int(os.environ.get("GDL_SWEEP", "1"))
-APPLY_SWEEP = int(os.environ.get("GDL_APPLY_SWEEP", "1"))
-STEM_STATS = int(os.environ.get("GDL_STEM_STATS", "1"))  # BatchNorm statistics of the stem from its epilogue
+# part in the 126 MB L2, so the next pass over the same tensor should start there, i.e. run the other way.  The
+# convolutions run ascending; the BatchNorm passes alternate: statistics descending after the conv, backward reduce
+# descending after the dgrad (its apply ascending).
 
 
 def note_writes(module):
@@ -79,7 +68,6 @@ class _ConvBN:
         self.conv, self.bn = conv, bn
         self.ci_real = ci_real
         self.relu = relu
-        self.cdir = 0  # sweep direction of this unit's convolution (set by the engine for SWEEP == 2)
         self.d = ops.conv_desc(N, Hi, Wi, ci_store, Co, R, S, conv.stride[0], conv.padding[0])
         self.P = N * self.d.Ho * self.d.Wo
         self.C = Co
@@ -99,11 +87,10 @@ class _ConvBN:
     def forward(self, eng, inp, res=None):
         """Training-mode unit (eval mode is EncoderEngine.forward_eval: BatchNorm folded into the conv)."""
         bn = self.bn
-        c = self.cdir
         # batch statistics come out of the conv epilogue where the kernel supports it (no extra pass over x)
-        ops.sweep(c)
+        ops.sweep(0)
         rows = ops.conv_fwd_stats(self.d, inp, self.wp, self.x, eng.bn_partial, self.ci_real)
-        ops.sweep((not c) if SWEEP else 0)
+        ops.sweep(1)
         rm, rv = eng.running(bn)
         if rows:
             ops.bn_stats_finalize(eng.bn_partial, rows, self.P, self.C, bn.weight.data, bn.bias.data, bn.eps,
@@ -113,8 +100,8 @@ class _ConvBN:
                          bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
         # with the statistics out of the conv epilogue the apply pass is the FIRST pass over x after the convolution: it
         # walks against the convolution's direction (starts on the tail that is still in L2) and leaves the head of y,
-        # where the next convolution starts, in L2.  GDL_APPLY_SWEEP=0: the round-1 order (same direction).
-        ops.sweep(((not c) if (rows and APPLY_SWEEP and SWEEP) else c))
+        # where the next convolution starts, in L2.
+        ops.sweep(1 if rows else 0)
         ops.bn_apply(self.x, res, self.y, self.P, self.C, self.scale, self.shift, self.relu)
         return self.y
 
@@ -146,16 +133,11 @@ class _StemBN(_ConvBN):
     def forward(self, eng, x16, res=None):
         bn = self.bn
         rm, rv = eng.running(bn)
-        if STEM_STATS:  # batch statistics out of the stem's epilogue: no separate pass over the largest activation
-            rows = ops.stem_fwd_stats(x16, self.wp, self.x, self.N, self.H, self.W, self.ci_real, eng.bn_partial)
-            ops.bn_stats_finalize(eng.bn_partial, rows, self.P, self.C, bn.weight.data, bn.bias.data, bn.eps,
-                                  bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
-            ops.sweep(1 if SWEEP else 0)
-        else:
-            ops.stem_fwd(x16, self.wp, self.x, self.N, self.H, self.W, self.ci_real)
-            ops.sweep(1 if SWEEP else 0)
-            ops.bn_stats(self.x, self.P, self.C, eng.bn_partial, bn.weight.data, bn.bias.data, bn.eps,
-                         bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
+        # batch statistics out of the stem's epilogue: no separate pass over the largest activation
+        rows = ops.stem_fwd_stats(x16, self.wp, self.x, self.N, self.H, self.W, self.ci_real, eng.bn_partial)
+        ops.bn_stats_finalize(eng.bn_partial, rows, self.P, self.C, bn.weight.data, bn.bias.data, bn.eps,
+                              bn.momentum, rm, rv, self.mean, self.invstd, self.scale, self.shift)
+        ops.sweep(1)
         # BN-apply + ReLU + MaxPool(3,2,1) in one pass (reference backbone.py:104-106)
         ops.bn_relu_maxpool_fwd(self.x, self.scale, self.shift, eng.pool_y, eng.pool_idx, eng.pool_xmax,
                                 self.N, self.Ho, self.Wo, 64, eng.Hp, eng.Wp)
@@ -191,21 +173,15 @@ class EncoderEngine:
                 ud = None
                 if blk.downsample is not None:
                     ud = self._unit(pre + "downsample", blk.downsample[0], blk.downsample[1], N, h, w, cin, False)
-                if SWEEP >= 2:  # the block input was written ascending (max-pool / previous bn2 apply)
-                    u1.cdir = 1
-                    if ud is not None:
-                        ud.cdir = 1
                 self.blocks.append((u1, u2, ud))
                 h, w, cin = u1.d.Ho, u1.d.Wo, u1.C
         self.Hf, self.Wf, self.Cf = h, w, cin
         self.wgrad_ws = torch.empty(max(self.max_wgrad_ws, 16) // 4, device=device, dtype=torch.float32)
         self.bn_partial = torch.empty(self.max_bn_partial, device=device, dtype=torch.float32)
-        self.wgrad_stream = torch.cuda.Stream(device) if USE_WGRAD_STREAM else None
         # running-statistics sink of a forward that must leave the modules' running buffers untouched (a replica
         # other than the first of a DGLStep with replicas > 1): the finalize kernels update this pair instead
         self.stats_sink = (torch.zeros(512, device=device), torch.zeros(512, device=device))
         self.own_stats = True
-        self._readers = {}
         self._eval_key_folded = None
         self.x_in = None  # the staged bf16 stem input (stage_input), allocated on first use
         self._plan_backward()
@@ -362,6 +338,11 @@ class EncoderEngine:
         self.bwd_plan = plan
         self.grad_buffer_bytes = pool.total_bytes
 
+    # The weight gradients run inline on the encoder's stream.  A side stream for them, overlapping the tensor-bound
+    # wgrads with the HBM-bound BatchNorm chain, measured no gain at B=256 (24.05 vs 23.88 ms on a B200) and was
+    # removed.  bench.py's roofline pass reads and restores this attribute.
+    wgrad_stream = None
+
     grad_override = None  # optional {param: tensor} destination map (autograd-compatible mode)
 
     def _grad(self, p):
@@ -383,29 +364,6 @@ class EncoderEngine:
         ops.bn_bwd(dy, u.y, u.x, dz, dx, u.P, u.C, bn.weight.data, u.mean, u.invstd, self.bn_partial,
                    self._grad(bn.weight), self._grad(bn.bias), relu)
 
-    # ------------------------------------------------------------------ weight-gradient side stream
-    # A weight gradient only needs the BN-backward output d_c and a saved forward activation, and nothing in
-    # the backward chain needs ITS result: all wgrads run on a side stream, concurrently with the dgrad -> BN
-    # chain, so the tensor-bound wgrad kernels overlap the HBM-bound BN kernels.  d_c buffers are reused by
-    # later blocks: before the chain overwrites one, it waits for the wgrad that still reads it.
-    def _wgrad(self, fn, d_c):
-        ws = self.wgrad_stream
-        if ws is None:
-            fn()
-            return
-        main = torch.cuda.current_stream()
-        ws.wait_stream(main)              # d_c is complete
-        with torch.cuda.stream(ws):
-            fn()
-            ev = torch.cuda.Event()
-            ev.record(ws)
-        self._readers[d_c.data_ptr()] = ev
-
-    def _before_write(self, buf):
-        ev = self._readers.pop(buf.data_ptr(), None)
-        if ev is not None:
-            torch.cuda.current_stream().wait_event(ev)
-
     N_LATE_BLOCKS = 4  # layer4 + layer3: 94 % of the encoder's parameters, the first gradients to be complete
 
     def late_parameters(self):
@@ -424,7 +382,6 @@ class EncoderEngine:
         part=None runs the whole backward; part=0 only layer4 + layer3 (after which the gradients of
         late_parameters() are final and their all-reduce can start), part=1 the rest (layer2, layer1, stem)."""
         x16 = self.x_in if x16 is None else x16
-        self._readers = {}
         chain = list(zip(reversed(self.blocks), self.bwd_plan, reversed(self._block_inputs())))
         if part == 0:
             chain = chain[:self.N_LATE_BLOCKS]
@@ -433,28 +390,22 @@ class EncoderEngine:
         for (u1, u2, ud), b, in_t in chain:
             g_out = b["g_out"]
             # out = relu(bn2(c2) + identity): dz = g_out * (out > 0), in place
-            self._before_write(b["d_c2"])
-            ops.sweep(1 if SWEEP else 0)      # g_out was written ascending: reduce descending, apply ascending
+            ops.sweep(1)  # g_out was written ascending: reduce descending, apply ascending
             self._bn_bwd(u2, g_out, g_out, b["d_c2"], True)
-            self._wgrad(lambda: ops.conv_wgrad(u2.d, u2.ci_real, u1.y, b["d_c2"], self._grad(u2.conv.weight),
-                                               self.wgrad_ws), b["d_c2"])
-            ops.sweep(1 if SWEEP >= 2 else 0)
+            ops.conv_wgrad(u2.d, u2.ci_real, u1.y, b["d_c2"], self._grad(u2.conv.weight), self.wgrad_ws)
+            ops.sweep(0)
             ops.conv_dgrad(u2.d, b["d_c2"], u2.wT, b["g_y1"])
-            ops.sweep(1 if SWEEP == 1 else 0)  # SWEEP 2: g_y1 was written descending -> reduce ascending
+            ops.sweep(1)
             # bn1 + relu has no residual input: mask recomputed from x, no y read / dz write
-            self._before_write(b["d_c1"])
             ops.bn_bwd_nores(b["g_y1"], u1.x, b["d_c1"], u1.P, u1.C, u1.bn.weight.data, u1.mean, u1.invstd,
                              u1.scale, u1.shift, self.bn_partial, self._grad(u1.bn.weight), self._grad(u1.bn.bias))
-            self._wgrad(lambda: ops.conv_wgrad(u1.d, u1.ci_real, in_t, b["d_c1"], self._grad(u1.conv.weight),
-                                               self.wgrad_ws), b["d_c1"])
+            ops.conv_wgrad(u1.d, u1.ci_real, in_t, b["d_c1"], self._grad(u1.conv.weight), self.wgrad_ws)
             if ud is not None:
                 # identity = bn_d(conv1x1_s2(u)), no relu: its output gradient is dz (= g_out now)
-                self._before_write(b["d_cd"])
-                ops.sweep(1 if SWEEP else 0)
+                ops.sweep(1)
                 self._bn_bwd(ud, g_out, None, b["d_cd"], False)
                 ops.sweep(0)
-                self._wgrad(lambda: ops.conv_wgrad(ud.d, ud.ci_real, in_t, b["d_cd"], self._grad(ud.conv.weight),
-                                                   self.wgrad_ws), b["d_cd"])
+                ops.conv_wgrad(ud.d, ud.ci_real, in_t, b["d_cd"], self._grad(ud.conv.weight), self.wgrad_ws)
                 # 1x1 stride-2 dgrad on the compact grid, then folded into conv1's dgrad epilogue
                 dc = ops.conv_desc(self.N, ud.d.Ho, ud.d.Wo, ud.d.Ci, ud.d.Co, 1, 1, 1, 0)
                 ops.conv_dgrad(dc, b["d_cd"], ud.wT, b["g_ds"])
@@ -464,23 +415,15 @@ class EncoderEngine:
                 ops.conv_dgrad(u1.d, b["d_c1"], u1.wT, b["g_u"], g_out, 1)
         if part == 0:
             ops.sweep(0)
-            if self.wgrad_stream is not None:
-                torch.cuda.current_stream().wait_stream(self.wgrad_stream)
-            self._readers = {}
             return
         s = self.stem
-        ops.sweep(1 if SWEEP else 0)  # g_pool was written ascending by the last dgrad
+        ops.sweep(1)  # g_pool was written ascending by the last dgrad
         # max-pool scatter + ReLU mask + BN backward in one pair of passes over the stem conv output
-        self._before_write(self.d_c0)
         ops.bn_relu_maxpool_bwd(self.g_pool, self.pool_idx, self.pool_xmax, s.x, self.d_c0, self.N, s.d.Ho, s.d.Wo,
                                 64, self.Hp, self.Wp, s.bn.weight.data, s.mean, s.invstd, s.scale, s.shift, self.bn_partial,
                                 self._grad(s.bn.weight), self._grad(s.bn.bias))
-        self._wgrad(lambda: ops.stem_wgrad(x16, self.d_c0, self._grad(s.conv.weight), s.ci_real, self.N, self.H,
-                                           self.W, self.wgrad_ws), self.d_c0)
+        ops.stem_wgrad(x16, self.d_c0, self._grad(s.conv.weight), s.ci_real, self.N, self.H, self.W, self.wgrad_ws)
         ops.sweep(0)
-        if self.wgrad_stream is not None:
-            torch.cuda.current_stream().wait_stream(self.wgrad_stream)  # join: every gradient is complete
-        self._readers = {}
 
     def _block_inputs(self):
         ins = [self.pool_y]

@@ -10,7 +10,7 @@ so that the three big contractions are the library's two flat-window GEMMs (csrc
     G  [262144, 2B]  = W1t * [dH_a; dH_v]^T         gemm_nt   (unimodal only: Lf saw detached features)
 
 `FilmHead` is the fused-step path (step.DGLStep).  It never holds the 262144-row operands whole: the reduction
-index f = i*512 + j is walked in CHUNKS of `CHUNK_I` values of i (default 128: 65536 features; GDL_FILM_CHUNK_I).
+index f = i*512 + j is walked in CHUNKS of `CHUNK_I` = 128 values of i (65536 features).
 Per chunk the outer products (100 MB at B = 256), the unimodal gradient G (67 MB) and the weight-gradient tile
 (67 MB) live in three rolling buffers, instead of 403 + 268 + 268 MB held for the whole step; H accumulates over the
 chunks (gemm_tn_f32 / gemm_tn_f32_acc), dW1 is written window by window, da / dv accumulate (film_contract_chunk).
@@ -20,16 +20,13 @@ operands is the second evaluation of the outer products in the backward loop (0.
 `FilmFn` is the autograd bridge the drop-in module uses so the reference's own two-backward loop runs unmodified
 (one outer product per call, whole operands).
 """
-import os
-
 import torch
 
 from . import ops
 
 D = 512
 F2 = D * D
-CHUNK_I = int(os.environ.get("GDL_FILM_CHUNK_I", "128"))  # values of the first outer-product index per chunk
-assert CHUNK_I in (32, 64, 128, 256, 512)
+CHUNK_I = 128  # values of the first outer-product index per chunk
 FC = CHUNK_I * D        # features per chunk
 
 

@@ -172,7 +172,7 @@ def sweep(reverse):
 
 def set_fused_stats_min_k(k):
     """Enable the conv-epilogue BN statistics for convolutions with R*S*Ci >= k (k < 0: library default = every
-    flat-window convolution, or GDL_FUSED_STATS_MIN_K).  Returns the previous setting."""
+    flat-window convolution).  Returns the previous setting."""
     return int(_lib.load().gdl_set_fused_stats_min_k(int(k)))
 
 

@@ -339,11 +339,11 @@ class DGLStep:
         self._bn_counters = [m.num_batches_tracked for m in model.modules()
                              if isinstance(m, torch.nn.BatchNorm2d)]
         self.head = fusion_head(model.fusion_module, B, self.n, dev)
-        # GDL_STREAM_PRIO: 0 = equal priorities, 1 = the visual encoder's stream (the long chain: 3x the audio work) is
-        # high priority so its kernels' CTAs are placed first and the audio kernels fill the gaps, 2 = the reverse
-        prio = int(os.environ.get("GDL_STREAM_PRIO", "1"))  # measured: 20.40 / 20.09 ms vs 20.48 / 20.40 ms per step, e2e +1.7 %
-        self.stream_a = torch.cuda.Stream(dev, priority=-1 if prio == 2 else 0)
-        self.stream_v = torch.cuda.Stream(dev, priority=-1 if prio == 1 else 0)
+        # the visual encoder's stream (the long chain: 3x the audio work) is high priority so its kernels' CTAs are placed
+        # first and the audio kernels fill the gaps (measured: 20.40 / 20.09 ms vs 20.48 / 20.40 ms per step with equal
+        # priorities, e2e +1.7 %)
+        self.stream_a = torch.cuda.Stream(dev, priority=0)
+        self.stream_v = torch.cuda.Stream(dev, priority=-1)
         self.steps_done = 0
         self.momentum_loaded = False  # set by train.adopt_momentum when a checkpoint's buffers were copied in
         self.graphs = GraphCache()  # the device runs of the schedule, captured once

@@ -99,9 +99,9 @@ int gdl_conv_fwd_bias_act(const gdl_conv_desc* d, const void* x, const void* w_p
  * a path without the fused statistics (call gdl_bn_stats on y instead).  bn_partial: gdl_bn_partial_floats(). */
 int gdl_conv_fwd_stats(const gdl_conv_desc* d, const void* x, const void* w_packed, void* y,
                        float* bn_partial, int* bn_partial_rows, gdl_stream_t s);
-/* Fused statistics are used for convolutions with R*S*Ci >= k.  Default (k < 0): the environment variable
- * GDL_FUSED_STATS_MIN_K, else 0 = every convolution the flat-window kernels run (the per-warp shared-memory
- * transpose costs less than the separate statistics pass on every layer of the bench geometry).  Thread-local.
+/* Fused statistics are used for convolutions with R*S*Ci >= k.  Default (k < 0): 0 = every convolution the
+ * flat-window kernels run (the per-warp shared-memory transpose costs less than the separate statistics pass on
+ * every layer of the bench geometry).  Thread-local.
  * Returns the old value (negative: the default was in force). */
 int gdl_set_fused_stats_min_k(int k);
 /* Scheduling hint for the calling thread (no reference counterpart: the reference's kernels are cuDNN's):

@@ -1,8 +1,8 @@
 """Per-layer convolution timing at the bench geometry (B=256 CREMA-D shape): fwd / dgrad / wgrad of every
 distinct conv of both encoders, CUDA-event timed, L2 flushed between repetitions.
     python tools/conv_bench.py [--out gpurun_out/conv_bench.json] [--tag name] [--ops fwd,dgrad,wgrad]
-Kernel selection follows the library's env switches (GDL_FLAT, GDL_FLAT_MT, GDL_CONV_IMPL ...), which are
-read once per process: run it once per configuration and compare the JSON files."""
+GDL_FLAT=0 / GDL_WFLAT=0 select the generic gather kernels instead of the flat-window ones; the library reads them
+once per process: run it once per setting and compare the JSON files."""
 import argparse
 import json
 import os
